@@ -8,7 +8,8 @@ A "step" is one forward pass (poly encoder + Q-Former + LoRA-Llama + LTSF fusion
 batch of synthetic highD-shaped scenes.  N=1 workload = BASELINE.json configs[1]: the GPT-2-small-class Llama
 backbone (H=768, 12 layers, LoRA r=8), bf16, 1024 scenes per step.  With N>1 every rank runs its own 1024-scene
 shard (scene-parallel, weak scaling) and the step ends with one all-reduce of (sum ADE, sum FDE, n).
-Prints ONE JSON line on rank 0.
+Prints ONE JSON line on rank 0.  `--dump-outputs DIR` also writes what the last timed step returned, for an output-for-output
+comparison of two builds.
 """
 import argparse
 import json
@@ -39,6 +40,29 @@ def emit(obj):
     out = _JSON_OUT or sys.stdout
     out.write(json.dumps(obj) + "\n")
     out.flush()
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays, scenes):
+    """Writes the tensors the timed path returned in its last step as <path>/<name>.npy (float64 stays float64, every other dtype
+    becomes float32), so that two builds can be compared output for output on the same seeded inputs.  Above 64 MB in all, the
+    per-scene arrays (leading dimension `scenes`) keep one seeded sample of scenes, the same rows in each; the others stay whole."""
+    import numpy as np
+    arrs = {k: v.detach().to("cpu", torch.float64 if v.dtype == torch.float64 else torch.float32) for k, v in arrays.items()}
+    total = sum(a.numel() * a.element_size() for a in arrs.values())
+    budget = DUMP_LIMIT_BYTES - 4096 * len(arrs)        # room for the .npy headers
+    per_scene = [k for k, a in arrs.items() if a.dim() and a.shape[0] == scenes]
+    if total > budget and per_scene:
+        fixed = total - sum(arrs[k].numel() * arrs[k].element_size() for k in per_scene)
+        n = max(1, scenes * (budget - fixed) // (total - fixed))
+        rows = torch.randperm(scenes, generator=torch.Generator().manual_seed(0))[:n].sort().values
+        for k in per_scene:
+            arrs[k] = arrs[k][rows]
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrs.items():
+        np.save(os.path.join(path, k + ".npy"), a.numpy())
 
 
 METRIC = "predicted scenes/sec (forward + ADE/FDE)"
@@ -244,8 +268,9 @@ def _roofline(prof, pk, ms_step, steps_profiled, extra=None, top=10):
     return r, dom
 
 
-def measure_infer(ctx, workload, steps, warmup, e2e=True, scenes=0, merge_lora=False):
-    """One inference workload: device-resident `value` leg (clean timed region), separate profiling pass, optional host-buffer e2e leg."""
+def measure_infer(ctx, workload, steps, warmup, e2e=True, scenes=0, merge_lora=False, dump=None):
+    """One inference workload: device-resident `value` leg (clean timed region), separate profiling pass, optional host-buffer e2e leg.
+    `dump`: directory for what the last timed step returned (rank 0)."""
     import tcavp_b200 as T
     from tcavp_b200 import ops
     dist, rank, world, dev = ctx.dist, ctx.rank, ctx.world, ctx.dev
@@ -299,6 +324,8 @@ def measure_infer(ctx, workload, steps, warmup, e2e=True, scenes=0, merge_lora=F
     launches = ops.launch_count() - launches0
     clocks = sampler.stop() if sampler else None
     ms = ctx.max_over_ranks(e0.elapsed_time(e1))
+    if dump and rank == 0:          # before the passes below: with a CUDA graph, `o` holds the graph's static output buffers
+        dump_outputs(dump, {k: v for k, v in o.items() if torch.is_tensor(v)}, B)
     value = world * B * steps / (ms / 1e3)
     ade, fde = float(o["sum_ade"]) / B, float(o["sum_fde"]) / B
     # ---- profiling pass (untimed): the same steps again with CUDA events around every launch ---------------
@@ -419,9 +446,10 @@ TRAIN_WORKLOADS = {
 }
 
 
-def measure_train(ctx, workload, steps, warmup, scenes=0, dropout=None):
+def measure_train(ctx, workload, steps, warmup, scenes=0, dropout=None, dump=None):
     """One fine-tune step = forward + hand-written backward + ONE all-reduce of the trainable gradients + fused AdamW
-    (tcavp_b200.FineTuner).  Metric: LoRA fine-tune tokens/sec (tokens = scenes x (16 image + L_text))."""
+    (tcavp_b200.FineTuner).  Metric: LoRA fine-tune tokens/sec (tokens = scenes x (16 image + L_text)).
+    `dump`: directory for the (loss, decoded) of the last timed step (rank 0)."""
     import warnings
 
     import tcavp_b200 as T
@@ -455,13 +483,15 @@ def measure_train(ctx, workload, steps, warmup, scenes=0, dropout=None):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(steps):
-        loss, _ = step()
+        loss, decoded = step()
     e1.record()
     ctx.barrier()
     # forward + backward are replayed from a CUDA graph: the library's launch counter only sees the capture
     launches = (ops.launch_count() - launches0) + (ft.launches_per_step * steps if ft.use_cuda_graph else 0)
     clocks = sampler.stop() if sampler else None
     ms = ctx.max_over_ranks(e0.elapsed_time(e1))
+    if dump and rank == 0:
+        dump_outputs(dump, {"loss": loss, "decoded": decoded}, B)
     # the collective alone (same buffer, same communicator), outside the timed region
     ar_ms = ar_exposed_ms = None
     ar_ab = {"overlapped": [], "serial": []}
@@ -535,7 +565,7 @@ def measure_train(ctx, workload, steps, warmup, scenes=0, dropout=None):
     return out
 
 
-def measure_stage1(ctx, steps, warmup, scenes=0):
+def measure_stage1(ctx, steps, warmup, scenes=0, dump=None):
     """Stage-1 (CausalLM) training step of the reference's scripts/check_generation.py loop at the 768-class shape: model.stage1_forward(...)
     -> outputs.loss.backward() -> AdamW on the mllm.* tensors.  Metric: tokens/sec through the model (scenes x (16 image + L_text));
     the labelled half of every sequence (64 answer tokens per scene) goes through lm_head (vocabulary 32000) in row chunks."""
@@ -583,6 +613,8 @@ def measure_stage1(ctx, steps, warmup, scenes=0):
     launches = ops.launch_count() - n0
     clocks = sampler.stop() if sampler else None
     ms = ctx.max_over_ranks(e0.elapsed_time(e1))
+    if dump and rank == 0:
+        dump_outputs(dump, {"loss": loss}, B)
     losses.append(float(loss))
     prof = ops.LaunchProfiler()
     with prof:
@@ -622,7 +654,8 @@ def _free():
 
 def run_ours(args):
     ctx = _Ctx(args)
-    out, keep = measure_infer(ctx, args.workload, args.steps, args.warmup, e2e=True, scenes=args.scenes, merge_lora=args.merge_lora)
+    out, keep = measure_infer(ctx, args.workload, args.steps, args.warmup, e2e=True, scenes=args.scenes, merge_lora=args.merge_lora,
+                              dump=args.dump_outputs)
     if ctx.world == 1 and ctx.rank == 0 and not args.no_cpu_baseline:
         out["cpu_baseline"] = cpu_baseline(keep["model"], keep["cfg"], keep["lc"], keep["l_text"], sample=args.cpu_sample, repeats=2,
                                            frozen=keep["frozen"])
@@ -656,7 +689,7 @@ def run_ours(args):
 def run_train(args):
     """--mode train: the LoRA fine-tune step as the only workload of the run."""
     ctx = _Ctx(args)
-    out = measure_train(ctx, args.workload, args.steps, args.warmup, scenes=args.scenes, dropout=args.dropout)
+    out = measure_train(ctx, args.workload, args.steps, args.warmup, scenes=args.scenes, dropout=args.dropout, dump=args.dump_outputs)
     if ctx.rank == 0:
         emit(out)
     ctx.close()
@@ -762,7 +795,13 @@ if __name__ == "__main__":
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--merge-lora", action="store_true", help="serve-time option: fold LoRA into the base weights at pack time (not the default "
                     "benchmark configuration: the reference runs the unmerged peft form)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="CUDA path: write what the last timed step of the headline workload returned as DIR/<name>.npy (float32 / float64, at most 64 MB)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.impl == "reference" and a.dump_outputs:
+        ap.error("--dump-outputs applies to the CUDA path only (not to --impl reference)")
     _claim_stdout()
     if a.impl == "reference":
         run_reference(a)
@@ -770,7 +809,7 @@ if __name__ == "__main__":
         run_train(a)
     elif a.mode == "stage1":
         _ctx = _Ctx(a)
-        _out = measure_stage1(_ctx, a.steps, a.warmup, scenes=a.scenes)
+        _out = measure_stage1(_ctx, a.steps, a.warmup, scenes=a.scenes, dump=a.dump_outputs)
         if _ctx.rank == 0:
             emit(_out)
         _ctx.close()

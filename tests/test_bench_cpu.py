@@ -39,3 +39,38 @@ def test_cuda_arm_fails_loudly_without_a_device():
     r = _run("--steps", "1")
     assert r.returncode != 0
     assert not any(l.lstrip().startswith("{") for l in r.stdout.splitlines()), "no bench line may be printed without a GPU"
+
+
+
+def test_dump_outputs_is_rejected_on_the_reference_arm(tmp_path):
+    r = _run("--impl", "reference", "--steps", "1", "--warmup", "0", "--cpu-sample", "2", "--dump-outputs", str(tmp_path / "d"))
+    assert r.returncode != 0 and "--dump-outputs" in r.stderr and r.stdout.strip() == ""
+    assert not (tmp_path / "d").exists()
+
+
+def test_dump_outputs_writes_float_arrays_and_samples_scenes_above_64_mb(tmp_path):
+    import numpy as np
+    import bench
+    small = {"decoded": torch.randn(5, 2, 7).to(torch.bfloat16), "metrics": torch.arange(8, dtype=torch.float64), "loss": torch.tensor(3.5)}
+    bench.dump_outputs(str(tmp_path / "small"), small, 5)
+    for k, v in small.items():
+        a = np.load(tmp_path / "small" / f"{k}.npy")
+        assert a.dtype == (np.float64 if v.dtype == torch.float64 else np.float32) and a.shape == tuple(v.shape), k
+        assert np.array_equal(a, v.double().numpy()), k
+    # 80 MB of per-scene rows numbered by their scene: one seeded sample of scenes, the same in every per-scene array and on every
+    # call, 64 MB at most in all; arrays that are not per scene (metrics, here also of leading length > 1) stay whole
+    scenes = 163840
+    big = {"decoded": torch.arange(scenes, dtype=torch.float32)[:, None].repeat(1, 128),
+           "per_scene": torch.arange(scenes, dtype=torch.float32)[:, None].repeat(1, 2),
+           "metrics": torch.arange(8, dtype=torch.float32), "loss": torch.tensor(1.0)}
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), big, scenes)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["decoded.npy", "loss.npy", "metrics.npy", "per_scene.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= bench.DUMP_LIMIT_BYTES
+    dec, per = np.load(tmp_path / "a" / "decoded.npy"), np.load(tmp_path / "a" / "per_scene.npy")
+    assert 0.5 * scenes < dec.shape[0] < scenes and dec.shape[1] == 128
+    assert (dec == dec[:, :1]).all() and np.array_equal(dec[:, 0], per[:, 0]) and (np.diff(dec[:, 0]) > 0).all()
+    assert np.array_equal(np.load(tmp_path / "a" / "metrics.npy"), np.arange(8, dtype=np.float32))
+    for f in files:
+        assert np.array_equal(np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)), f

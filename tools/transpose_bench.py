@@ -1,5 +1,5 @@
-import sys, torch
-sys.path.insert(0, '/root/repo')
+import os, sys, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from tcavp_b200 import ops
 for (M, N, dt) in [(73728, 768, torch.bfloat16), (73728, 1536, torch.bfloat16), (73728, 768, torch.float32)]:
     x = torch.randn(M, N, device='cuda').to(dt)
