@@ -14,7 +14,8 @@
  *   - Every call is asynchronous on `stream` (a cudaStream_t passed as void*), never synchronises,
  *     returns 0 on success or a negative TCAVP_ERR_* code; tcavp_last_error() gives the thread-local text.
  *   - dtype codes: TCAVP_F32 (fp32 storage, exact fp32 SIMT math, no TF32) / TCAVP_BF16 (bf16 storage,
- *     fp32 accumulate; dense contractions on tcgen05 tensor cores).
+ *     fp32 accumulate; dense contractions on tcgen05 tensor cores) / TCAVP_E4M3 (one-byte OCP e4m3fn GEMM operands
+ *     with per-row / per-column fp32 scales: the opt-in fp8 serving mode of the decoder stack).
  *   - Matrices are row-major; "ld*" are leading dimensions in ELEMENTS.  Weights keep nn.Linear's
  *     [out_features, in_features] layout so state_dict tensors are consumed without transposition.
  *   - There is no CPU fallback anywhere: without an sm_100 device every compute entry point fails.
@@ -31,7 +32,7 @@ extern "C" {
 
 typedef void* tcavp_stream_t; /* cudaStream_t */
 
-enum { TCAVP_F32 = 0, TCAVP_BF16 = 1 };
+enum { TCAVP_F32 = 0, TCAVP_BF16 = 1, TCAVP_E4M3 = 2 };
 enum { TCAVP_OK = 0, TCAVP_ERR_ARG = -1, TCAVP_ERR_CUDA = -2, TCAVP_ERR_UNSUPPORTED = -3 };
 enum { TCAVP_ACT_NONE = 0, TCAVP_ACT_RELU = 1, TCAVP_ACT_SWIGLU = 2, TCAVP_ACT_SWIGLU_BWD = 3,
        TCAVP_ACT_GELU_TANH = 4 /* HF "gelu_new" (GPT-2 mlp.c_fc): 0.5 x (1 + tanh(sqrt(2/pi) (x + 0.044715 x^3))) */ };
@@ -70,6 +71,9 @@ int tcavp_gemm_tile_order(int tiles_m, int tiles_n, int panel_w, int* mg, int* n
  *   in_dtype   TCAVP_BF16: A and W are bf16 -> TMA-fed tcgen05.mma, fp32 accumulators in TMEM.
  *              Requires K % 8 == 0, lda % 8 == 0, ldw % 8 == 0 and 16-byte aligned A / W.
  *              TCAVP_F32 : A and W are fp32 -> SIMT FFMA kernel (exact fp32 accumulate).
+ *              TCAVP_E4M3: A and W are e4m3fn bytes -> tcgen05.mma.kind::f8f6f4, fp32 accumulators in TMEM.  Requires
+ *              col_scale, K % 16 == 0, lda % 16 == 0, ldw % 16 == 0 and 16-byte aligned A / W; output and residual stay
+ *              bf16 / fp32.  row_sumsq, sumsq_out, aux_out and SWIGLU_BWD are bf16-only (TCAVP_ERR_ARG).
  *   LoRA       is NOT an epilogue term: the caller appends T = x.A^T (rank r, from a skinny call of
  *              this same function) as extra K columns of A and (alpha/r).B as extra K columns of W,
  *              so the rank-r update accumulates in the same TMEM tile as the base product.
@@ -116,6 +120,10 @@ typedef struct tcavp_gemm_args {
                                   columns are d(mid) and the epilogue writes the 2N interleaved columns (d gate, d up) to `out`
                                   (bf16, ldo >= 2N): d gate = d u s (1 + g (1 - s)), d up = d g s, s = sigmoid(g) — the backward of
                                   HF LlamaMLP's act_fn(gate) * up (HF:190) fused into the down_proj^T GEMM. */
+  const float* col_scale;      /* e4m3 operands only (required there, 16-byte aligned, N floats): accumulator column n is multiplied by
+                                  col_scale[n] (the weight row's dequantisation factor) before the row factor, RoPE and SwiGLU — for
+                                  SwiGLU n indexes the interleaved accumulator rows of W.  With row_scale = the activation rows'
+                                  factors: out = act(acc * row_scale[m] * col_scale[n] + bias) + residual.  NULL for bf16 / fp32. */
 } tcavp_gemm_args;
 
 int tcavp_gemm(const tcavp_gemm_args* args, tcavp_stream_t stream);
@@ -175,6 +183,13 @@ int tcavp_rmsnorm(const void* x, int ldi, const float* w, void* out, int rows, i
                   int out_dtype, tcavp_stream_t stream);
 /* out[r] = rsqrt(mean(x[r, 0:cols]^2) + eps)  — the per-row factor of LlamaRMSNorm, consumed by tcavp_gemm's row_scale. */
 int tcavp_row_rstd(const void* x, int ldx, int rows, int cols, float eps, int dtype, float* out, tcavp_stream_t stream);
+/* Per-row e4m3 quantisation of bf16 rows (the activation operand of the fp8 decoder projections, HF:182-196 / 251-289):
+ *   s = 448 / amax(|x[r, :]|) (fp32, correctly rounded), q[r, c] = e4m3_rn_satfinite(x[r, c] * s), f[r] = amax / 448;
+ *   an all-zero row gives q = 0, f = 0.  rms != 0 folds LlamaRMSNorm (HF:53-70; its weight is folded into the e4m3 weight) into the
+ *   factor: f[r] = rsqrt(mean(x[r, :]^2) + eps) * amax / 448, so one read of x gives the QKV / gate-up operand and its row_scale.
+ * x bf16 [rows, ldi], q e4m3 [rows, ldo] (bytes), f fp32 [rows].  cols % 16 == 0, 16 <= cols <= 14336, ldi % 8 == 0, ldo % 16 == 0, 16-byte
+ * aligned x / q.  Rows stream through shared memory by the bulk-copy engine; every row is quantised independently of its batch. */
+int tcavp_quant_e4m3_rows(const void* x, int ldi, void* q, int ldo, float* f, int rows, int cols, int rms, float eps, tcavp_stream_t stream);
 
 /* ---- rotary embedding (HF:146-170 apply_rotary_pos_emb, default rope HF:73-136) ----------------
  * In place on the q and k head blocks of a packed [rows, ld] qkv buffer (q heads first, then k heads);

@@ -84,6 +84,7 @@ struct EpilogueParams {
   unsigned long long* sumsq_out;                       // += sum of squares of the final output row, Q44.20 fixed point (order-independent)
   const unsigned long long* row_sumsq; float ss_inv, ss_eps;   // row factor rsqrt(row_sumsq[m] * 2^-20 * ss_inv + ss_eps) (alternative to row_scale)
   __nv_bfloat16* aux; int ld_aux;                      // SwiGLU only: raw (row-scaled) gate/up accumulators for the backward pass
+  const float* col_scale;                              // e4m3 operands: per-accumulator-column factor applied to the raw accumulators
 };
 
 __device__ __forceinline__ int remap_row(int gi, int go, int off, int m) {

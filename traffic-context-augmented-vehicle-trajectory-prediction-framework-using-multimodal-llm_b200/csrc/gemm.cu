@@ -28,6 +28,14 @@ constexpr int UMMA_K = 16;
 constexpr int NUM_EPI_WARPS = 16;  // four warps per TMEM lane quarter, each draining every fourth 32-column chunk
 constexpr int NUM_THREADS = 64 + 32 * NUM_EPI_WARPS;  // warp 0: TMA producer, warp 1: MMA issuer + TMEM owner, warps 2..: epilogue
 constexpr int A_STAGE_BYTES = BLOCK_M * BLOCK_K * 2;
+// Operand geometry per element type.  e4m3 (kind::f8f6f4) keeps the byte geometry of bf16: a k-block is one 128-byte swizzle row
+// (128 elements) and one MMA covers 32 bytes of K (32 elements), so stage sizes, descriptor advances and TMEM budgets are shared.
+template <bool F8>
+struct Op {
+  static constexpr int KB = F8 ? 128 : BLOCK_K;   // elements per k-block
+  static constexpr int UK = F8 ? 32 : UMMA_K;     // elements per MMA
+  static constexpr int ESZ = F8 ? 1 : 2;          // bytes per element
+};
 
 template <int BLOCK_N>
 struct Cfg {
@@ -107,6 +115,18 @@ __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint6
       "{\n\t.reg .pred p;\n\t"
       "setp.ne.b32 p, %4, 0;\n\t"
       "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
+      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+// kind::f8f6f4 instruction descriptor: D fp32, A/B E4M3 (format code 0 in bits 7-9 / 10-12), both K-major, M x N tile.
+__host__ __device__ constexpr uint32_t umma_idesc_e4m3(int M, int N) {
+  return (1u << 4) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
+}
+__device__ __forceinline__ void umma_e4m3(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
       "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
@@ -197,6 +217,25 @@ constexpr int PANEL_SHIFT = 16;   // flags >> PANEL_SHIFT = panel width in n-til
 enum { EPI_VEC_OUT = 1, EPI_VEC_RES = 2, EPI_VEC_BIAS = 4, EPI_TMA_OUT = 8,    // EPI_TMA_OUT: bf16 output staged in shared memory, stored by TMA
        DBG_NO_TMA = 16, DBG_NO_MMA = 32, DBG_NO_EPI = 64, DBG_NO_STORE = 128,   // TCAVP_GEMM_DEBUG: ablation switches for profiling (results are garbage)
        L2_W_LAST = 256, L2_A_FIRST = 512, L2_OUT_FIRST = 1024 };      // L2 eviction priorities of a panelled problem (TCAVP_GEMM_L2HINT)
+
+// e4m3 operands: accumulator column n carries the dequantisation factor col_scale[n] of its weight row.  Applied to the raw accumulators
+// (before the row factor, RoPE and SwiGLU, which mix or pair columns with different scales); columns past Nacc get 0.
+__device__ __forceinline__ void scale_cols(uint32_t (&r)[32], const float* __restrict__ cs, int nacc0, int nacc) {
+  if (nacc0 + 32 <= nacc) {
+    const float4* p = reinterpret_cast<const float4*>(cs + nacc0);
+#pragma unroll
+    for (int q = 0; q < 8; ++q) {
+      const float4 s = __ldg(p + q);
+      r[4 * q] = __float_as_uint(__uint_as_float(r[4 * q]) * s.x);
+      r[4 * q + 1] = __float_as_uint(__uint_as_float(r[4 * q + 1]) * s.y);
+      r[4 * q + 2] = __float_as_uint(__uint_as_float(r[4 * q + 2]) * s.z);
+      r[4 * q + 3] = __float_as_uint(__uint_as_float(r[4 * q + 3]) * s.w);
+    }
+  } else {
+#pragma unroll
+    for (int j = 0; j < 32; ++j) r[j] = __float_as_uint(__uint_as_float(r[j]) * (nacc0 + j < nacc ? __ldg(cs + nacc0 + j) : 0.f));
+  }
+}
 
 // Epilogue of 32 accumulator columns [nacc0, nacc0+32) of row m for one thread.  The interior-tile path (full chunk,
 // 16-byte aligned rows) is branch-light and fully vectorised; ragged edges take the scalar path.
@@ -402,7 +441,7 @@ __device__ __forceinline__ void epilogue_chunk(const EpilogueParams& p, int m, i
 // CM = CTAs per cluster along M.  With CM = 2 the two CTAs of a cluster work on vertically adjacent output tiles that
 // share the W tile: each CTA fetches half of it and TMA-multicasts that half into both shared memories, which cuts
 // the L2 -> SM operand traffic per CTA from A + W to A + W/2 (the binding resource for K <= 1024 GEMMs).
-template <int BLOCK_N, int CM>
+template <int BLOCK_N, int CM, bool F8 = false>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b, EpilogueParams ep,
                int M, int Nacc, int K, int flags) {
@@ -428,7 +467,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
   // work unit = CM vertically adjacent tiles; unit u -> (m group u / tiles_n, n tile u % tiles_n); a cluster strides over units
   const int num_units = ((tiles_m + CM - 1) / CM) * tiles_n;
   const int unit0 = blockIdx.x / CM, unit_stride = gridDim.x / CM;
-  const int num_kb = (K + BLOCK_K - 1) / BLOCK_K;
+  using O = Op<F8>;
+  const int num_kb = (K + O::KB - 1) / O::KB;
   const int pw = (flags >> PANEL_SHIFT) > 0 ? (flags >> PANEL_SHIFT) : tiles_n;   // n-tiles per L2-resident panel of W
 
   if (warp == 0 && lane == 0) {
@@ -467,9 +507,9 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
         for (int kb = 0; kb < num_kb; ++kb) {
           mbar_wait(empty_bar + 8 * stage, phase ^ 1);
           mbar_expect_tx(full_bar + 8 * stage, C::STAGE_BYTES);
-          tma_load_2d(smem_a + stage * A_STAGE_BYTES, &tma_a, full_bar + 8 * stage, kb * BLOCK_K, m0);
+          tma_load_2d(smem_a + stage * A_STAGE_BYTES, &tma_a, full_bar + 8 * stage, kb * O::KB, m0);
           if (CM == 1) {
-            tma_load_2d(smem_b + stage * C::B_STAGE_BYTES, &tma_b, full_bar + 8 * stage, kb * BLOCK_K, n0);
+            tma_load_2d(smem_b + stage * C::B_STAGE_BYTES, &tma_b, full_bar + 8 * stage, kb * O::KB, n0);
           } else {   // my 1/CM slice of the W tile goes to every CTA of the cluster
             constexpr int SLICE = BLOCK_N / CM;
             tma_load_2d_mc(smem_b + stage * C::B_STAGE_BYTES + cta_rank * (SLICE * BLOCK_K * 2), &tma_b, full_bar + 8 * stage,
@@ -482,7 +522,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
   } else if (warp == 1) {
     // ===================== MMA issuer =====================
     if (lane == 0) {
-      constexpr uint32_t idesc = umma_idesc(BLOCK_M, BLOCK_N);
+      constexpr uint32_t idesc = F8 ? umma_idesc_e4m3(BLOCK_M, BLOCK_N) : umma_idesc(BLOCK_M, BLOCK_N);
       int stage = 0;
       uint32_t phase = 0;
       int it = 0;
@@ -494,13 +534,14 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
         for (int kb = 0; kb < num_kb; ++kb) {
           mbar_wait(full_bar + 8 * stage, phase);
           tc_fence_after();
-          const int k_left = K - kb * BLOCK_K;
-          const int ksteps = k_left >= BLOCK_K ? BLOCK_K / UMMA_K : (k_left + UMMA_K - 1) / UMMA_K;
+          const int k_left = K - kb * O::KB;
+          const int ksteps = k_left >= O::KB ? O::KB / O::UK : (k_left + O::UK - 1) / O::UK;
           const uint32_t a_addr = smem_a + stage * A_STAGE_BYTES;
           const uint32_t b_addr = smem_b + stage * C::B_STAGE_BYTES;
           for (int k = 0; k < ksteps; ++k) {
-            umma_bf16(tmem_d, umma_smem_desc(a_addr + k * UMMA_K * 2), umma_smem_desc(b_addr + k * UMMA_K * 2), idesc,
-                      (kb | k) != 0 ? 1u : 0u);
+            const uint64_t ad = umma_smem_desc(a_addr + k * O::UK * O::ESZ), bd = umma_smem_desc(b_addr + k * O::UK * O::ESZ);
+            if constexpr (F8) umma_e4m3(tmem_d, ad, bd, idesc, (kb | k) != 0 ? 1u : 0u);
+            else umma_bf16(tmem_d, ad, bd, idesc, (kb | k) != 0 ? 1u : 0u);
           }
           // frees the smem slot (in every CTA whose multicast writes into it) once the MMAs above retire
           if (CM == 1) umma_commit(empty_bar + 8 * stage);
@@ -536,6 +577,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
         if (n0 + c * 32 >= Nacc) break;   // warp-uniform
         uint32_t r[32];
         tmem_ld32(tmem_base + ((uint32_t)(quarter * 32) << 16) + acc * BLOCK_N + c * 32, r);
+        if constexpr (F8) scale_cols(r, ep.col_scale, n0 + c * 32, Nacc);
         epilogue_chunk(ep, m, pos, n0 + c * 32, r, rs, flags, ssq);
       }
       if (ep.sumsq_out && m < M) sumsq_add(ep.sumsq_out + remap_row(ep.remap_gi, ep.remap_go, ep.remap_off, m), ssq);
@@ -597,6 +639,14 @@ __device__ __forceinline__ void umma_bf16_pair(uint32_t tmem_d, uint64_t adesc, 
       "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+__device__ __forceinline__ void umma_e4m3_pair(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
+      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 __device__ __forceinline__ void umma_commit_pair(uint32_t bar) {   // arrives on the same barrier offset in both CTAs
   asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
                "h"((uint16_t)3)
@@ -627,7 +677,7 @@ __device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, uint32_t sr
 // the tile, writes its bf16 results into a private 4 KB swizzled staging tile and lets one lane issue a cp.async.bulk.tensor store
 // (the copy engine writes full 128-byte lines and clips the tensor edges); the staging tile is reused once the previous store has
 // read it (cp.async.bulk.wait_group.read).  One operand stage is given up for the staging tiles.
-template <int BLOCK_N, bool TMA_OUT = false>
+template <int BLOCK_N, bool TMA_OUT = false, bool F8 = false>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b, const __grid_constant__ CUtensorMap tma_o,
                     EpilogueParams ep, int M, int Nacc, int K, int flags) {
@@ -654,7 +704,8 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_cons
   const int tiles_m = (M + PAIR_M - 1) / PAIR_M;
   const int num_units = tiles_m * tiles_n;
   const int unit0 = blockIdx.x >> 1, unit_stride = gridDim.x >> 1;
-  const int num_kb = (K + BLOCK_K - 1) / BLOCK_K;
+  using O = Op<F8>;
+  const int num_kb = (K + O::KB - 1) / O::KB;
   const int pw = (flags >> PANEL_SHIFT) > 0 ? (flags >> PANEL_SHIFT) : tiles_n;   // n-tiles per L2-resident panel of W
 
   if (warp == 0 && lane == 0) {
@@ -700,11 +751,11 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_cons
           } else {
             if (leader) mbar_expect_tx(full_bar + 8 * stage, 2 * C::STAGE_BYTES);
             if (hinted) {
-              tma_load_2d_pair_hint(smem_a + stage * A_STAGE_BYTES, &tma_a, leader_full + 8 * stage, kb * BLOCK_K, m0, pol_a);
-              tma_load_2d_pair_hint(smem_b + stage * C::B_STAGE_BYTES, &tma_b, leader_full + 8 * stage, kb * BLOCK_K, n0, pol_w);
+              tma_load_2d_pair_hint(smem_a + stage * A_STAGE_BYTES, &tma_a, leader_full + 8 * stage, kb * O::KB, m0, pol_a);
+              tma_load_2d_pair_hint(smem_b + stage * C::B_STAGE_BYTES, &tma_b, leader_full + 8 * stage, kb * O::KB, n0, pol_w);
             } else {
-              tma_load_2d_pair(smem_a + stage * A_STAGE_BYTES, &tma_a, leader_full + 8 * stage, kb * BLOCK_K, m0);
-              tma_load_2d_pair(smem_b + stage * C::B_STAGE_BYTES, &tma_b, leader_full + 8 * stage, kb * BLOCK_K, n0);
+              tma_load_2d_pair(smem_a + stage * A_STAGE_BYTES, &tma_a, leader_full + 8 * stage, kb * O::KB, m0);
+              tma_load_2d_pair(smem_b + stage * C::B_STAGE_BYTES, &tma_b, leader_full + 8 * stage, kb * O::KB, n0);
             }
           }
           if (++stage == C::STAGES) { stage = 0; phase ^= 1; }
@@ -714,7 +765,7 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_cons
   } else if (warp == 1) {
     // ===================== MMA issuer (leader CTA only) =====================
     if (leader && lane == 0) {
-      constexpr uint32_t idesc = umma_idesc(PAIR_M, BLOCK_N);
+      constexpr uint32_t idesc = F8 ? umma_idesc_e4m3(PAIR_M, BLOCK_N) : umma_idesc(PAIR_M, BLOCK_N);
       int stage = 0;
       uint32_t phase = 0;
       int it = 0;
@@ -726,8 +777,8 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_cons
         for (int kb = 0; kb < num_kb; ++kb) {
           mbar_wait(full_bar + 8 * stage, phase);
           tc_fence_after();
-          const int k_left = K - kb * BLOCK_K;
-          const int ksteps = k_left >= BLOCK_K ? BLOCK_K / UMMA_K : (k_left + UMMA_K - 1) / UMMA_K;
+          const int k_left = K - kb * O::KB;
+          const int ksteps = k_left >= O::KB ? O::KB / O::UK : (k_left + O::UK - 1) / O::UK;
           const uint32_t a_addr = smem_a + stage * A_STAGE_BYTES;
           const uint32_t b_addr = smem_b + stage * C::B_STAGE_BYTES;
           if (flags & DBG_NO_MMA) {
@@ -739,8 +790,9 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_cons
             }
           } else {
             for (int k = 0; k < ksteps; ++k) {
-              umma_bf16_pair(tmem_d, umma_smem_desc(a_addr + k * UMMA_K * 2), umma_smem_desc(b_addr + k * UMMA_K * 2), idesc,
-                             (kb | k) != 0 ? 1u : 0u);
+              const uint64_t ad = umma_smem_desc(a_addr + k * O::UK * O::ESZ), bd = umma_smem_desc(b_addr + k * O::UK * O::ESZ);
+              if constexpr (F8) umma_e4m3_pair(tmem_d, ad, bd, idesc, (kb | k) != 0 ? 1u : 0u);
+              else umma_bf16_pair(tmem_d, ad, bd, idesc, (kb | k) != 0 ? 1u : 0u);
             }
             umma_commit_pair(empty_bar + 8 * stage);
             if (kb == num_kb - 1) umma_commit_pair(tmem_full_bar + 8 * acc);
@@ -787,6 +839,7 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_cons
               if (n0 + c * 32 >= Nacc) break;
               uint32_t r[32];
               tmem_ld32(tmem_base + ((uint32_t)(quarter * 32) << 16) + acc * BLOCK_N + c * 32, r);
+              if constexpr (F8) scale_cols(r, ep.col_scale, n0 + c * 32, Nacc);
               epilogue_chunk(ep, m, pos, n0 + c * 32, r, rs, flags, ssq, stage_row, hh, lane);
             }
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
@@ -803,6 +856,7 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_cons
             if (n0 + c * 32 >= Nacc) break;   // warp-uniform
             uint32_t r[32];
             tmem_ld32(tmem_base + ((uint32_t)(quarter * 32) << 16) + acc * BLOCK_N + c * 32, r);
+            if constexpr (F8) scale_cols(r, ep.col_scale, n0 + c * 32, Nacc);
             epilogue_chunk(ep, m, pos, n0 + c * 32, r, rs, flags, ssq);
           }
         }
@@ -1209,18 +1263,18 @@ static EncodeTiledFn get_encode() {
   return fn;
 }
 
-// rows x cols bf16 matrix with leading dimension ld; box = box_rows x 64 columns, 128-byte swizzle.
-static int make_map(CUtensorMap* map, const void* base, int rows, int cols, int ld, int box_rows) {
+// rows x cols bf16 (f8: e4m3) matrix with leading dimension ld; box = box_rows x one 128-byte row (64 bf16 / 128 e4m3), 128-byte swizzle.
+static int make_map(CUtensorMap* map, const void* base, int rows, int cols, int ld, int box_rows, bool f8 = false) {
   EncodeTiledFn enc = get_encode();
   if (!enc) {
     set_error("cuTensorMapEncodeTiled is unavailable (no CUDA driver?)");
     return TCAVP_ERR_CUDA;
   }
   cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)ld * 2};
-  cuuint32_t box[2] = {(cuuint32_t)BLOCK_K, (cuuint32_t)box_rows};
+  cuuint64_t strides[1] = {(cuuint64_t)ld * (f8 ? 1 : 2)};
+  cuuint32_t box[2] = {(cuuint32_t)(f8 ? Op<true>::KB : BLOCK_K), (cuuint32_t)box_rows};
   cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
+  CUresult r = enc(map, f8 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
@@ -1288,15 +1342,21 @@ static int panel_flags(long long M, long long N, long long K, int unit_m, int ti
   return ((int)pw << PANEL_SHIFT) | hint_flags;
 }
 
-template <int BLOCK_N, int CM>
+// tcavp_last_kernel() names of the e4m3 forms (the bf16 launches keep their plain kernel names)
+template <int BLOCK_N> constexpr const char* e4m3_name() {
+  return BLOCK_N == 32 ? "gemm_tc_kernel<32,e4m3>" : BLOCK_N == 64 ? "gemm_tc_kernel<64,e4m3>" : BLOCK_N == 128 ? "gemm_tc_kernel<128,e4m3>"
+                                                                                                             : "gemm_tc_kernel<256,e4m3>";
+}
+
+template <int BLOCK_N, int CM, bool F8 = false>
 static int launch_tc(const tcavp_gemm_args& a, const EpilogueParams& ep, cudaStream_t stream) {
   using C = Cfg<BLOCK_N>;
   CUtensorMap ma, mb;
-  int rc = make_map(&ma, a.A, a.M, a.K, a.lda, BLOCK_M);
+  int rc = make_map(&ma, a.A, a.M, a.K, a.lda, BLOCK_M, F8);
   if (rc) return rc;
-  rc = make_map(&mb, a.W, a.N, a.K, a.ldw, BLOCK_N / CM);
+  rc = make_map(&mb, a.W, a.N, a.K, a.ldw, BLOCK_N / CM, F8);
   if (rc) return rc;
-  TCAVP_CUDA(cudaFuncSetAttribute(gemm_tc_kernel<BLOCK_N, CM>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
+  TCAVP_CUDA(cudaFuncSetAttribute(gemm_tc_kernel<BLOCK_N, CM, F8>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
   const int tiles_m = (a.M + BLOCK_M - 1) / BLOCK_M, tiles_n = (a.N + BLOCK_N - 1) / BLOCK_N;
   const int units = ((tiles_m + CM - 1) / CM) * tiles_n;
   const int max_clusters = sm_count() / CM;
@@ -1315,8 +1375,8 @@ static int launch_tc(const tcavp_gemm_args& a, const EpilogueParams& ep, cudaStr
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   flags |= panel_flags(a.M, a.N, a.K, BLOCK_M * CM, BLOCK_N, max_clusters, false);
-  TCAVP_CUDA(cudaLaunchKernelEx(&cfg, gemm_tc_kernel<BLOCK_N, CM>, ma, mb, ep, a.M, a.N, a.K, flags));
-  return check_launch("gemm_tc_kernel");
+  TCAVP_CUDA(cudaLaunchKernelEx(&cfg, gemm_tc_kernel<BLOCK_N, CM, F8>, ma, mb, ep, a.M, a.N, a.K, flags));
+  return check_launch(F8 ? e4m3_name<BLOCK_N>() : "gemm_tc_kernel");
 }
 
 // TCAVP_GEMM_TMASTORE: 1 (default) = bf16 outputs leave through shared memory + TMA stores (pair kernel), 0 = 256-bit global stores.
@@ -1352,15 +1412,15 @@ static int make_out_map(CUtensorMap* map, void* base, int rows, int cols, int ld
   return TCAVP_OK;
 }
 
-template <int BLOCK_N>
+template <int BLOCK_N, bool F8 = false>
 static int launch_tc_pair(const tcavp_gemm_args& a, const EpilogueParams& ep, cudaStream_t stream) {
   // TMA-store epilogue: bf16 output rows in place (no row remap), 16-byte aligned rows, not the SwiGLU-backward form
   const bool tma_out = tma_store_pref() && ep.out_dtype == TCAVP_BF16 && ep.remap_gi == 0 && ep.act != TCAVP_ACT_SWIGLU_BWD &&
                        (ep.ldo % 8) == 0 && reinterpret_cast<uintptr_t>(ep.out) % 16 == 0;
   CUtensorMap ma, mb, mo;
-  int rc = make_map(&ma, a.A, a.M, a.K, a.lda, BLOCK_M);
+  int rc = make_map(&ma, a.A, a.M, a.K, a.lda, BLOCK_M, F8);
   if (rc) return rc;
-  rc = make_map(&mb, a.W, a.N, a.K, a.ldw, BLOCK_N / 2);
+  rc = make_map(&mb, a.W, a.N, a.K, a.ldw, BLOCK_N / 2, F8);
   if (rc) return rc;
   if (tma_out) {
     rc = make_out_map(&mo, ep.out, ep.M, ep.N, ep.ldo, ep.act == TCAVP_ACT_SWIGLU ? 32 : 64);
@@ -1369,8 +1429,8 @@ static int launch_tc_pair(const tcavp_gemm_args& a, const EpilogueParams& ep, cu
     mo = ma;      // unused by the kernel
   }
   const int smem_bytes = tma_out ? PairCfg<BLOCK_N, true>::SMEM_BYTES : PairCfg<BLOCK_N, false>::SMEM_BYTES;
-  if (tma_out) TCAVP_CUDA(cudaFuncSetAttribute(gemm_tc_pair_kernel<BLOCK_N, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
-  else TCAVP_CUDA(cudaFuncSetAttribute(gemm_tc_pair_kernel<BLOCK_N, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
+  if (tma_out) TCAVP_CUDA(cudaFuncSetAttribute(gemm_tc_pair_kernel<BLOCK_N, true, F8>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
+  else TCAVP_CUDA(cudaFuncSetAttribute(gemm_tc_pair_kernel<BLOCK_N, false, F8>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
   const int tiles_m = (a.M + 2 * BLOCK_M - 1) / (2 * BLOCK_M), tiles_n = (a.N + BLOCK_N - 1) / BLOCK_N;
   const int units = tiles_m * tiles_n;
   const int max_pairs = sm_count() / 2;
@@ -1391,9 +1451,9 @@ static int launch_tc_pair(const tcavp_gemm_args& a, const EpilogueParams& ep, cu
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   flags |= panel_flags(a.M, a.N, a.K, 2 * BLOCK_M, BLOCK_N, max_pairs, true);
-  if (tma_out) TCAVP_CUDA(cudaLaunchKernelEx(&cfg, gemm_tc_pair_kernel<BLOCK_N, true>, ma, mb, mo, ep, a.M, a.N, a.K, flags));
-  else TCAVP_CUDA(cudaLaunchKernelEx(&cfg, gemm_tc_pair_kernel<BLOCK_N, false>, ma, mb, mo, ep, a.M, a.N, a.K, flags));
-  return check_launch("gemm_tc_pair_kernel");
+  if (tma_out) TCAVP_CUDA(cudaLaunchKernelEx(&cfg, gemm_tc_pair_kernel<BLOCK_N, true, F8>, ma, mb, mo, ep, a.M, a.N, a.K, flags));
+  else TCAVP_CUDA(cudaLaunchKernelEx(&cfg, gemm_tc_pair_kernel<BLOCK_N, false, F8>, ma, mb, mo, ep, a.M, a.N, a.K, flags));
+  return check_launch(F8 ? "gemm_tc_pair_kernel<256,e4m3>" : "gemm_tc_pair_kernel");
 }
 
 template <int BLOCK_N>
@@ -1698,6 +1758,8 @@ extern "C" int tcavp_gemm(const tcavp_gemm_args* a, tcavp_stream_t stream_) {
   TCAVP_REQUIRE((!a->sumsq_out && !a->row_sumsq) || a->in_dtype == TCAVP_BF16, "tcavp_gemm: sumsq_out / row_sumsq need bf16 operands");
   TCAVP_REQUIRE(!a->sumsq_out || a->act != TCAVP_ACT_SWIGLU, "tcavp_gemm: sumsq_out is not defined for the SwiGLU epilogue");
   ep.aux = reinterpret_cast<__nv_bfloat16*>(a->aux_out); ep.ld_aux = a->ld_aux;
+  ep.col_scale = a->col_scale;
+  TCAVP_REQUIRE(!a->col_scale || a->in_dtype == TCAVP_E4M3, "tcavp_gemm: col_scale needs e4m3 operands");
   if (ep.aux && a->act != TCAVP_ACT_SWIGLU_BWD) {
     TCAVP_REQUIRE(a->act == TCAVP_ACT_SWIGLU && a->in_dtype == TCAVP_BF16, "tcavp_gemm: aux_out needs act SWIGLU and bf16 operands");
     TCAVP_REQUIRE(a->N % 32 == 0 && a->ld_aux >= a->N && a->ld_aux % 16 == 0 && reinterpret_cast<uintptr_t>(a->aux_out) % 32 == 0,
@@ -1726,6 +1788,19 @@ extern "C" int tcavp_gemm(const tcavp_gemm_args* a, tcavp_stream_t stream_) {
     if (tc::cluster_pref() >= 3 && a->M >= 16 * tc::BLOCK_M) return tc::launch_tc_pair<256>(*a, ep, stream);
     if (tc::cluster_pref() == 2 && a->M >= 16 * tc::BLOCK_M) return tc::launch_tc<256, 2>(*a, ep, stream);
     return tc::launch_tc<256, 1>(*a, ep, stream);
+  }
+  if (a->in_dtype == TCAVP_E4M3) {
+    TCAVP_REQUIRE(a->col_scale && reinterpret_cast<uintptr_t>(a->col_scale) % 16 == 0, "tcavp_gemm(e4m3): needs a 16-byte aligned col_scale");
+    TCAVP_REQUIRE(a->K % 16 == 0 && a->lda % 16 == 0 && a->ldw % 16 == 0, "tcavp_gemm(e4m3): K, lda, ldw must be multiples of 16 (K=%d lda=%d ldw=%d)",
+                  a->K, a->lda, a->ldw);
+    TCAVP_REQUIRE(reinterpret_cast<uintptr_t>(a->A) % 16 == 0 && reinterpret_cast<uintptr_t>(a->W) % 16 == 0, "tcavp_gemm(e4m3): A and W must be 16-byte aligned");
+    TCAVP_REQUIRE(!a->row_sumsq && !a->sumsq_out && !a->aux_out && a->act != TCAVP_ACT_SWIGLU_BWD,
+                  "tcavp_gemm(e4m3): row_sumsq, sumsq_out, aux_out and SWIGLU_BWD are bf16-only epilogues");
+    if (a->N <= 32) return tc::launch_tc<32, 1, true>(*a, ep, stream);
+    if (a->N <= 64) return tc::launch_tc<64, 1, true>(*a, ep, stream);
+    if (a->N <= 128) return tc::launch_tc<128, 1, true>(*a, ep, stream);
+    if (tc::cluster_pref() >= 3 && a->M >= 16 * tc::BLOCK_M) return tc::launch_tc_pair<256, true>(*a, ep, stream);
+    return tc::launch_tc<256, 1, true>(*a, ep, stream);
   }
   if (a->in_dtype == TCAVP_F32) {
     const long long t64 = (long long)((a->N + 63) / 64) * ((a->M + 63) / 64);

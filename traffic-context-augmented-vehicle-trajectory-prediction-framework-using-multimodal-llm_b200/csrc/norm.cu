@@ -318,6 +318,100 @@ __global__ void __launch_bounds__(lnp::WARPS * 32, 2) layernorm_pipe_kernel(cons
   }
 }
 
+// Per-row e4m3 quantisation (tcavp_quant_e4m3_rows) on the same bulk-copy row ring: each warp owns `stages` row buffers filled by
+// cp.async.bulk.  The whole row stays in shared memory while the warp finds its amax (and sum of squares), then is read a second time to
+// quantise it, so rows of any width up to the ring size take the same path (768-class rows: eight per warp in flight, 7B-class MLP
+// rows of 11 008 columns: one).
+namespace q8 {
+__device__ __forceinline__ uint32_t e4m3x4(float a, float b, float c, float d) {     // a lands in the lowest byte
+  uint16_t lo, hi;
+  asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(lo) : "f"(b), "f"(a));
+  asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(hi) : "f"(d), "f"(c));
+  return (uint32_t)lo | ((uint32_t)hi << 16);
+}
+__device__ __forceinline__ void lds8(uint32_t addr, float (&v)[8]) {
+  uint4 u;
+  asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(u.x), "=r"(u.y), "=r"(u.z), "=r"(u.w) : "r"(addr));
+  const uint32_t q[4] = {u.x, u.y, u.z, u.w};
+#pragma unroll
+  for (int e = 0; e < 4; ++e) {
+    v[2 * e] = __uint_as_float(q[e] << 16);
+    v[2 * e + 1] = __uint_as_float(q[e] & 0xffff0000u);
+  }
+}
+constexpr int RING_BYTES = 96 << 10;     // per block (lnp::WARPS warps); two blocks per SM at 768-class rows
+__host__ __device__ inline int stages_for(int cols) {
+  const int s = RING_BYTES / (lnp::WARPS * (cols * 2 + 8));
+  return s < 1 ? 1 : (s > lnp::MAX_STAGES ? lnp::MAX_STAGES : s);
+}
+}  // namespace q8
+
+__global__ void __launch_bounds__(lnp::WARPS * 32) quant_e4m3_kernel(const __nv_bfloat16* __restrict__ x, int ldi, uint8_t* __restrict__ q, int ldo,
+                                                                    float* __restrict__ f, int rows, int cols, int rms, float eps) {
+  using namespace lnp;
+  extern __shared__ __align__(128) uint8_t ln_smem[];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const uint32_t row_bytes = (uint32_t)cols * 2u;
+  const int stages = q8::stages_for(cols);
+  const uint32_t ring = smem_u32(ln_smem) + (uint32_t)warp * stages * row_bytes;
+  const uint32_t bars = smem_u32(ln_smem) + (uint32_t)WARPS * stages * row_bytes + (uint32_t)warp * stages * 8u;
+  const int wstride = gridDim.x * WARPS;
+  const int row0 = blockIdx.x * WARPS + warp;
+  if (lane == 0) {
+    for (int s = 0; s < stages; ++s) mbar_init(bars + 8 * s, 1);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  __syncwarp();
+  if (lane == 0) {
+    for (int s = 0; s < stages; ++s) {
+      const long long r = (long long)row0 + (long long)s * wstride;
+      if (r < rows) {
+        mbar_expect_tx(bars + 8 * s, row_bytes);
+        bulk_load(ring + s * row_bytes, x + (size_t)r * ldi, row_bytes, bars + 8 * s);
+      }
+    }
+  }
+  int stage = 0;
+  uint32_t phase = 0;
+  for (long long row = row0; row < rows; row += wstride) {
+    mbar_wait(bars + 8 * stage, phase);
+    const uint32_t buf = ring + stage * row_bytes;
+    float amax = 0.f, ss = 0.f;
+    for (int c = lane * 8; c < cols; c += 256) {
+      float v[8];
+      q8::lds8(buf + c * 2, v);
+      float p = 0.f;
+#pragma unroll
+      for (int e = 0; e < 8; ++e) {
+        amax = fmaxf(amax, fabsf(v[e]));
+        p = fmaf(v[e], v[e], p);
+      }
+      ss += p;      // per-8-element partials keep the rounding error of long rows (11 008 columns) near 1e-7
+    }
+    amax = warp_max(amax);
+    const float s = amax > 0.f ? __fdiv_rn(448.f, amax) : 0.f;
+    uint8_t* qrow = q + (size_t)row * ldo;
+    for (int c = lane * 8; c < cols; c += 256) {
+      float v[8];
+      q8::lds8(buf + c * 2, v);
+      const uint32_t lo = q8::e4m3x4(v[0] * s, v[1] * s, v[2] * s, v[3] * s), hi = q8::e4m3x4(v[4] * s, v[5] * s, v[6] * s, v[7] * s);
+      asm volatile("st.global.v2.b32 [%0], {%1, %2};" ::"l"(qrow + c), "r"(lo), "r"(hi) : "memory");
+    }
+    float fr = __fdiv_rn(amax, 448.f);
+    if (rms) fr *= rsqrtf(warp_sum(ss) / cols + eps);
+    __syncwarp();     // every lane has read the row: the buffer goes back to the copy engine
+    if (lane == 0) {
+      f[row] = fr;
+      const long long nxt = row + (long long)stages * wstride;
+      if (nxt < rows) {
+        mbar_expect_tx(bars + 8 * stage, row_bytes);
+        bulk_load(buf, x + (size_t)nxt * ldi, row_bytes, bars + 8 * stage);
+      }
+    }
+    if (++stage == stages) { stage = 0; phase ^= 1; }
+  }
+}
+
 // Row-strided LayerNorm for shapes outside the bulk-copy kernel (narrow / unaligned rows, fp32): warp per row, element-wise.
 __global__ void __launch_bounds__(256) layernorm_strided_kernel(const void* __restrict__ x, int ldx, const float* __restrict__ w,
                                                                 const float* __restrict__ b, void* __restrict__ out, int ldo, int rows, int cols,
@@ -576,4 +670,24 @@ extern "C" int tcavp_rmsnorm(const void* x, int ldi, const float* w, void* out, 
   else
     rmsnorm_kernel<false><<<grid, wpb * 32, 0, stream>>>(x, w, out, rows, cols, ldi, ldo, eps, in_dtype, out_dtype);
   return check_launch("rmsnorm_kernel");
+}
+
+extern "C" int tcavp_quant_e4m3_rows(const void* x, int ldi, void* q, int ldo, float* f, int rows, int cols, int rms, float eps, tcavp_stream_t stream_) {
+  using namespace tcavp;
+  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+  TCAVP_REQUIRE(rows >= 0 && cols >= 16 && cols <= 14336 && cols % 16 == 0 && ldi >= cols && ldo >= cols,
+                "tcavp_quant_e4m3_rows: bad shape rows=%d cols=%d ldi=%d ldo=%d (cols %% 16 == 0, 16 <= cols <= 14336)", rows, cols, ldi, ldo);
+  if (rows == 0) return TCAVP_OK;
+  TCAVP_REQUIRE(x && q && f, "tcavp_quant_e4m3_rows: null pointer");
+  TCAVP_REQUIRE(ldi % 8 == 0 && ldo % 16 == 0 && reinterpret_cast<uintptr_t>(x) % 16 == 0 && reinterpret_cast<uintptr_t>(q) % 16 == 0,
+                "tcavp_quant_e4m3_rows: needs ldi %% 8 == 0, ldo %% 16 == 0 and 16-byte aligned x / q (ldi=%d ldo=%d)", ldi, ldo);
+  const size_t smem = (size_t)lnp::WARPS * q8::stages_for(cols) * ((size_t)cols * 2 + 8);
+  int bps = (int)((200u << 10) / smem);
+  bps = bps < 1 ? 1 : (bps > 4 ? 4 : bps);
+  int grid = sm_count() * bps;
+  if (grid > (rows + lnp::WARPS - 1) / lnp::WARPS) grid = (rows + lnp::WARPS - 1) / lnp::WARPS;
+  TCAVP_CUDA(cudaFuncSetAttribute(quant_e4m3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  quant_e4m3_kernel<<<grid, lnp::WARPS * 32, smem, stream>>>(reinterpret_cast<const __nv_bfloat16*>(x), ldi, reinterpret_cast<uint8_t*>(q), ldo, f,
+                                                             rows, cols, rms, eps);
+  return check_launch("quant_e4m3_kernel");
 }

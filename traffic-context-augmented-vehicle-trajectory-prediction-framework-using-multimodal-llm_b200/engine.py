@@ -30,9 +30,17 @@ class _Lin:
 class Engine:
     # fp32 ("small") layers of the temporal path run on the tensor cores through a bf16 hi/lo split in bf16 compute mode
     SPLIT_SMALL = True
+    # fp8 serving mode (fp8=True): the Llama decoder projections that run on e4m3 operands.  A projection is listed where its e4m3 GEMM
+    # plus the quantisation pass in front of it measured faster than its bf16 GEMM at both the cfg2 and the cfg3 shape on B200 (DESIGN §5,
+    # profiles/fp8_cfg*_r01_all4.json).  o_proj is not: at cfg2 its quantisation pass costs more than the e4m3 GEMM saves
+    # (2.34 + 0.91 ms against 2.61 ms per step), so it keeps its bf16 weight.
+    FP8_PROJ = ("wqkv", "wgu", "wdown")
 
-    def __init__(self, model, compute_dtype="bf16", merge_lora=False):
+    def __init__(self, model, compute_dtype="bf16", merge_lora=False, fp8=False):
         p0 = next(model.ltsf.parameters())
+        if fp8 and compute_dtype != "bf16":
+            raise ValueError(f"the fp8 serving mode runs on the bf16 engine (compute_dtype={compute_dtype!r})")
+        self.fp8 = bool(fp8)
         self.merge_lora = merge_lora
         self.dev = dev = p0.device   # packing works anywhere (host-side tests); forward() requires CUDA
         self.act = act = _ACT[compute_dtype]
@@ -219,13 +227,15 @@ class Engine:
         wrap = mllm.llama_wrapper
         c = wrap.config
         if c.get("arch") == "gpt2":
+            if self.fp8:
+                raise NotImplementedError("the fp8 serving mode covers Llama-arch backbones (GPT-2's LayerNorm mean and bias need another fold)")
             return self._pack_gpt2(mllm)
         lm = wrap.causal_lm()
         self._lm_head_param, self._embed_param = lm.lm_head.weight, lm.model.embed_tokens.weight
         act, dev = self.act, self.dev
         H, nh, nkv, dh, I = c["hidden_size"], c["num_attention_heads"], c["num_key_value_heads"], c["head_dim"], c["intermediate_size"]
-        # serve-time option (SURVEY.md §8f.3): W' = W + (alpha/r) B A merged at pack time — no side path, K stays H
-        merge = bool(wrap.use_lora and getattr(self, "merge_lora", False))
+        # serve-time option (SURVEY.md §8f.3): W' = W + (alpha/r) B A merged at pack time — no side path, K stays H (always so in fp8 mode)
+        merge = bool(wrap.use_lora and (getattr(self, "merge_lora", False) or self.fp8))
         lora_targets = tuple(wrap.llama_model.targets) if wrap.use_lora else ()
         targets = () if merge else lora_targets
         r = self.model_hp["lora_r"] if (wrap.use_lora and not merge) else 0
@@ -276,6 +286,50 @@ class Engine:
             self.llm["layers"].append(dict(
                 wqkv=wqkv, a_cat=a_cat, ln1=ln1, wo=sa.o_proj.weight.detach().to(dev, act).contiguous(), wgu=gu,
                 wdown=layer.mlp.down_proj.weight.detach().to(dev, act).contiguous()))
+            if self.fp8:
+                self._pack_fp8(self.llm["layers"][-1], layer, lora_targets, qk_perm if self.llm["fuse_rope"] else None, ln1, ln2)
+
+    def _pack_fp8(self, ly, layer, lora_targets, qk_perm, ln1, ln2):
+        """Replaces the bf16 weights of the FP8_PROJ projections of one packed layer by e4m3 weights with per-output-channel scales:
+        s_w[n] = amax(W'[n, :]) / 448, Wq = e4m3(W' / s_w) (zero rows: s_w = 0, Wq = 0).  W' is the fp32 weight the bf16 pack rounds
+        once: LoRA merged, RMSNorm weight folded into the columns, q / k rows RoPE-permuted, gate / up interleaved — here rounded once,
+        from fp32 straight to e4m3."""
+        dev = self.dev
+        sa, mlp = layer.self_attn, layer.mlp
+
+        def w32(mod, name):
+            if name in lora_targets:
+                A, B = mod.lora_A["default"].weight.detach().to(dev).float(), mod.lora_B["default"].weight.detach().to(dev).float()
+                return mod.base_layer.weight.detach().to(dev).float() + mod.scaling * (B @ A)
+            return mod.weight.detach().to(dev).float()
+        full = {}
+        if "wqkv" in self.FP8_PROJ:
+            w = torch.cat([w32(sa.q_proj, "q_proj"), w32(sa.k_proj, "k_proj"), w32(sa.v_proj, "v_proj")])
+            full["wqkv"] = (w if qk_perm is None else w[qk_perm]) * ln1[None, :]
+        if "wo" in self.FP8_PROJ:
+            full["wo"] = w32(sa.o_proj, "o_proj")
+        if "wgu" in self.FP8_PROJ:
+            g, u = mlp.gate_proj.weight.detach().to(dev).float() * ln2[None, :], mlp.up_proj.weight.detach().to(dev).float() * ln2[None, :]
+            full["wgu"] = torch.stack([g, u], dim=1).reshape(2 * g.shape[0], g.shape[1])
+        if "wdown" in self.FP8_PROJ:
+            full["wdown"] = mlp.down_proj.weight.detach().to(dev).float()
+        for name, w in full.items():
+            s = w.abs().amax(dim=1) / 448.0
+            q = torch.where(s[:, None] > 0, w / torch.where(s > 0, s, 1.0)[:, None], 0.0)
+            ly[name], ly["s_" + name] = q.to(torch.float8_e4m3fn).contiguous(), s.contiguous()
+
+    def _proj(self, ly, name, a, out, *, rms=False, **kw):
+        """One Llama decoder projection of the fp8 engine.  An e4m3 weight takes a per-row quantised copy of `a` (tcavp_quant_e4m3_rows,
+        with LlamaRMSNorm's factor folded into the row factor when `rms`); a projection left in bf16 takes `a` itself with the RMSNorm
+        factor from tcavp_row_rstd."""
+        w, rows, cols, eps = ly[name], a.shape[0], a.shape[1], self.llm["eps"]
+        if w.dtype == torch.float8_e4m3fn:
+            aq, f = ops.quant_e4m3_rows(a, self._new(rows, cols, dtype=torch.float8_e4m3fn), self._new(rows, dtype=torch.float32),
+                                        rms_eps=eps if rms else None)
+            return ops.gemm(aq, w, out, row_scale=f, col_scale=ly["s_" + name], **kw)
+        if rms:
+            kw["row_scale"] = ops.row_rstd(a, self._new(rows, dtype=torch.float32), rows=rows, cols=cols, ldx=a.stride(0), eps=eps)
+        return ops.gemm(a, w, out, **kw)
 
     def _pack_ltsf(self, lt):
         act, dev, small = self.act, self.dev, self.small
@@ -467,17 +521,20 @@ class Engine:
         # turns it into rstd in its epilogue, so the only separate
         # pass over the residual stream is the one before the first layer (bf16 tensor-core path; fp32 keeps tcavp_row_rstd).
         nl = len(m["layers"])
-        fuse_ss = self.act == torch.bfloat16 and not os.environ.get("TCAVP_NO_FUSE_RSTD")
+        fuse_ss = self.act == torch.bfloat16 and not self.fp8 and not os.environ.get("TCAVP_NO_FUSE_RSTD")
         ss = torch.zeros(2 * nl, M, dtype=torch.int64, device=self.dev) if fuse_ss else None
         for li, ly in enumerate(m["layers"]):
-            if fuse_ss and li > 0:
-                norm1 = dict(row_sumsq=(ss[2 * li - 1], H, m["eps"]))
+            if self.fp8:            # LoRA merged: kx == 0, x == xs
+                self._proj(ly, "wqkv", x, qkv, rms=True, rope=rope)
             else:
-                ops.row_rstd(xs, rstd, rows=M, cols=H, ldx=Kx, eps=m["eps"])
-                norm1 = dict(row_scale=rstd)
-            if kx:
-                ops.gemm(xs, ly["a_cat"], xs[:, H:], M=M, N=m["n_lora"], K=H, lda=Kx, ldo=Kx)
-            ops.gemm(xs, ly["wqkv"], qkv, M=M, N=nqkv, K=Kx, lda=Kx, rope=rope, **norm1)
+                if fuse_ss and li > 0:
+                    norm1 = dict(row_sumsq=(ss[2 * li - 1], H, m["eps"]))
+                else:
+                    ops.row_rstd(xs, rstd, rows=M, cols=H, ldx=Kx, eps=m["eps"])
+                    norm1 = dict(row_scale=rstd)
+                if kx:
+                    ops.gemm(xs, ly["a_cat"], xs[:, H:], M=M, N=m["n_lora"], K=H, lda=Kx, ldo=Kx)
+                ops.gemm(xs, ly["wqkv"], qkv, M=M, N=nqkv, K=Kx, lda=Kx, rope=rope, **norm1)
             if rope is None:
                 ops.rope_(qkv, rows=M, L=L, ld=nqkv, n_q_heads=nh, n_k_heads=nkv, dh=dh, table=table)
             if kv_out is not None:
@@ -487,7 +544,11 @@ class Engine:
             ops.attention(qkv, qkv[:, nh * dh:], qkv[:, (nh + nkv) * dh:], attn, B=B, H=nh, Hkv=nkv, Tq=L, Tk=L, dh=dh,
                           q_strides=(L * nqkv, nqkv), k_strides=(L * nqkv, nqkv), v_strides=(L * nqkv, nqkv),
                           o_strides=(L * nh * dh, nh * dh), scale=dh ** -0.5, causal=True, key_mask=mask)
-            if fuse_ss:
+            if self.fp8:
+                self._proj(ly, "wo", attn, x, residual=x)
+                self._proj(ly, "wgu", x, mid, rms=True, act=ops.ACT_SWIGLU)
+                self._proj(ly, "wdown", mid, x, residual=x)
+            elif fuse_ss:
                 ops.gemm(attn, ly["wo"], x, ldo=Kx, residual=x, ldr=Kx, sumsq_out=ss[2 * li])
                 ops.gemm(xs, ly["wgu"], mid, M=M, K=H, lda=Kx, act=ops.ACT_SWIGLU, row_sumsq=(ss[2 * li], H, m["eps"]))
                 ops.gemm(mid, ly["wdown"], x, ldo=Kx, residual=x, ldr=Kx, sumsq_out=ss[2 * li + 1] if li + 1 < nl else None)
@@ -527,15 +588,23 @@ class Engine:
         qkv, attn, mid = self._new(B, nqkv), self._new(B, nq), self._new(B, I)
         rope = (table, 1, dh, nq + nk) if m["fuse_rope"] else None
         for ly, cache in zip(m["layers"], caches):
-            ops.row_rstd(xs, rstd, rows=B, cols=H, ldx=Kx, eps=m["eps"])
-            if kx:
-                ops.gemm(xs, ly["a_cat"], xs[:, H:], M=B, N=m["n_lora"], K=H, lda=Kx, ldo=Kx)
-            ops.gemm(xs, ly["wqkv"], qkv, M=B, N=nqkv, K=Kx, lda=Kx, rope=rope, row_scale=rstd)
+            if self.fp8:            # LoRA merged: kx == 0, x == xs
+                self._proj(ly, "wqkv", x, qkv, rms=True, rope=rope)
+            else:
+                ops.row_rstd(xs, rstd, rows=B, cols=H, ldx=Kx, eps=m["eps"])
+                if kx:
+                    ops.gemm(xs, ly["a_cat"], xs[:, H:], M=B, N=m["n_lora"], K=H, lda=Kx, ldo=Kx)
+                ops.gemm(xs, ly["wqkv"], qkv, M=B, N=nqkv, K=Kx, lda=Kx, rope=rope, row_scale=rstd)
             if rope is None:
                 ops.rope_(qkv, rows=B, L=1, ld=nqkv, n_q_heads=nh, n_k_heads=nkv, dh=dh, table=table)
             cache[:, t].copy_(qkv[:, nq:])
             ops.attention(qkv, cache, cache[:, :, nk:], attn, B=B, H=nh, Hkv=nkv, Tq=1, Tk=t + 1, dh=dh, q_strides=(nqkv, nqkv),
                           k_strides=(cap * 2 * nk, 2 * nk), v_strides=(cap * 2 * nk, 2 * nk), o_strides=(nq, nq), scale=dh ** -0.5)
+            if self.fp8:
+                self._proj(ly, "wo", attn, x, residual=x)
+                self._proj(ly, "wgu", x, mid, rms=True, act=ops.ACT_SWIGLU)
+                self._proj(ly, "wdown", mid, x, residual=x)
+                continue
             ops.gemm(attn, ly["wo"], x, ldo=Kx, residual=x, ldr=Kx)
             ops.row_rstd(xs, rstd, rows=B, cols=H, ldx=Kx, eps=m["eps"])
             ops.gemm(xs, ly["wgu"], mid, M=B, K=H, lda=Kx, act=ops.ACT_SWIGLU, row_scale=rstd)

@@ -573,7 +573,7 @@ class MultiModalTrajectoryModel(nn.Module):
     def engine(self):
         sig = self._signature()
         if self._engine is None or sig != self._engine_sig:
-            self._engine = Engine(self, self.compute_dtype, merge_lora=getattr(self, "_merge_lora", False))
+            self._engine = Engine(self, self.compute_dtype, merge_lora=getattr(self, "_merge_lora", False), fp8=getattr(self, "_fp8", False))
             self._engine_sig = sig
         return self._engine
 
@@ -599,6 +599,21 @@ class MultiModalTrajectoryModel(nn.Module):
         parameters (and state_dict()) are untouched; training always uses the unmerged form."""
         if bool(enabled) != getattr(self, "_merge_lora", False):
             self._merge_lora = bool(enabled)
+            self._engine = None
+        return self
+
+    def fp8_backbone_for_inference(self, enabled=True):
+        """Serve-time option: the inference engine runs the Llama decoder projections on e4m3 operands (tcgen05 kind::f8f6f4) — weights
+        quantised once per output channel at pack time (LoRA merged), activations per row at run time, fp32 accumulation, the scales applied
+        in the GEMM epilogue.  Everything that runs through engine() follows it (forward, predict_with_metrics, evaluate, CUDA-graph replay,
+        generate_batch); train-mode passes, best_of_k, the fine-tune step and stage1_forward stay bf16.  The module's own parameters (and
+        state_dict()) are untouched.  Needs compute_dtype "bf16" and a Llama-arch backbone."""
+        if enabled and self.compute_dtype != "bf16":
+            raise ValueError(f"the fp8 serving mode needs compute_dtype 'bf16' (model has {self.compute_dtype!r})")
+        if enabled and self.mllm.llama_wrapper.config.get("arch") == "gpt2":
+            raise NotImplementedError("the fp8 serving mode covers Llama-arch backbones only")
+        if bool(enabled) != getattr(self, "_fp8", False):
+            self._fp8 = bool(enabled)
             self._engine = None
         return self
 

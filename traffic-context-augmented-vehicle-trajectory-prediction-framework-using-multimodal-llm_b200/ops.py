@@ -10,9 +10,9 @@ import torch
 
 from . import lib as _lib
 
-F32, BF16 = 0, 1
+F32, BF16, E4M3 = 0, 1, 2
 ACT_NONE, ACT_RELU, ACT_SWIGLU, ACT_SWIGLU_BWD, ACT_GELU_TANH = 0, 1, 2, 3, 4
-_DT = {torch.float32: F32, torch.bfloat16: BF16}
+_DT = {torch.float32: F32, torch.bfloat16: BF16, torch.float8_e4m3fn: E4M3}
 
 
 class GemmArgs(Structure):
@@ -28,7 +28,8 @@ class GemmArgs(Structure):
                 ("rope_cos_sin", c_void_p), ("rope_L", c_int), ("rope_dh", c_int), ("rope_cols", c_int),
                 ("row_scale", c_void_p),
                 ("sumsq_out", c_void_p), ("row_sumsq", c_void_p), ("sumsq_inv_cols", c_float), ("sumsq_eps", c_float),
-                ("aux_out", c_void_p), ("ld_aux", c_int)]
+                ("aux_out", c_void_p), ("ld_aux", c_int),
+                ("col_scale", c_void_p)]
 
 
 class AttnArgs(Structure):
@@ -216,9 +217,11 @@ def autotune_gemm_route(budget_ms=120.0):
 
 
 def gemm(a, w, out, *, M=None, N=None, K=None, lda=None, ldw=None, ldo=None, bias=None, residual=None, ldr=None,
-         act=ACT_NONE, remap=(0, 0, 0), rope=None, row_scale=None, aux_out=None, sumsq_out=None, row_sumsq=None):
-    """out = act(a @ w.T + bias) + residual.  a: [M, >=K] row-major (lda = a.stride(0)), w: [N, >=K]."""
-    _need_cuda(a, w, out, bias, residual)
+         act=ACT_NONE, remap=(0, 0, 0), rope=None, row_scale=None, aux_out=None, sumsq_out=None, row_sumsq=None, col_scale=None):
+    """out = act(a @ w.T + bias) + residual.  a: [M, >=K] row-major (lda = a.stride(0)), w: [N, >=K].
+    float8_e4m3fn operands need `col_scale` (fp32 [N], the weight rows' dequantisation factors) and usually `row_scale` (the activation
+    rows' factors from quant_e4m3_rows): out = act(acc * row_scale[m] * col_scale[n] + bias) + residual."""
+    _need_cuda(a, w, out, bias, residual, col_scale)
     g = GemmArgs()
     g.M = a.shape[0] if M is None else M
     g.N = w.shape[0] if N is None else N
@@ -255,7 +258,16 @@ def gemm(a, w, out, *, M=None, N=None, K=None, lda=None, ldw=None, ldo=None, bia
         g.aux_out, g.ld_aux = aux_out.data_ptr(), aux_out.stride(0)
     if rope is not None:     # (table, L, dh, cols)
         g.rope_cos_sin, g.rope_L, g.rope_dh, g.rope_cols = rope[0].data_ptr(), rope[1], rope[2], rope[3]
-    if g.in_dtype == BF16:
+    if col_scale is not None:
+        if col_scale.dtype != torch.float32:
+            raise TypeError("gemm: col_scale must be fp32")
+        g.col_scale = col_scale.data_ptr()
+    if g.in_dtype == E4M3:   # mirrors tcavp_gemm's e4m3 dispatch (no wide / quad forms)
+        if g.N > 128 and g.M >= 2048:
+            kern = "gemm_tc_pair_kernel<256,e4m3>[%sN%d,K%d]" % ("M%d," % g.M if g.M < 32768 else "", g.N, g.K)
+        else:
+            kern = "gemm_tc_kernel<%d,e4m3>[N%d,K%d]" % (32 if g.N <= 32 else 64 if g.N <= 64 else 128 if g.N <= 128 else 256, g.N, g.K)
+    elif g.in_dtype == BF16:
         long_k = g.N > 128 and g.K >= 2048 and g.M >= 8192 and ((g.M + 511) // 512) * ((g.N + 255) // 256) >= 4 * 74
         if long_k and _ROUTE["wide_k"] is None:
             autotune_gemm_route()
@@ -548,6 +560,21 @@ def ce_loss(logits, targets, loss_sum, grad=None, *, scale=1.0):
                                              c_longlong(grad.stride(0) if grad is not None else 0), dt(grad) if grad is not None else 0,
                                              c_longlong(rows), V, c_float(scale), _stream()), "tcavp_ce_loss")
     return loss_sum
+
+
+def quant_e4m3_rows(x, q, f, *, rows=None, cols=None, ldi=None, ldo=None, rms_eps=None):
+    """q = e4m3(x * 448 / amax(row)) (float8_e4m3fn [rows, >=cols]), f = amax / 448 per row (fp32 [rows]); with `rms_eps` the row's
+    LlamaRMSNorm factor rsqrt(mean(x^2) + eps) is folded into f.  x: bf16 [rows, >=cols]."""
+    _need_cuda(x, q, f)
+    if x.dtype != torch.bfloat16 or q.dtype != torch.float8_e4m3fn or f.dtype != torch.float32:
+        raise TypeError(f"quant_e4m3_rows: x bf16, q float8_e4m3fn, f fp32 (got {x.dtype}, {q.dtype}, {f.dtype})")
+    rows = x.shape[0] if rows is None else rows
+    cols = x.shape[1] if cols is None else cols
+    with _Timed("quant_e4m3_kernel[%d]" % cols, 0.0, float(rows * (cols * 3 + 4))):
+        _lib.check(_lib.load().tcavp_quant_e4m3_rows(_p(x), c_int(x.stride(0) if ldi is None else ldi), _p(q), c_int(q.stride(0) if ldo is None else ldo),
+                                                     _p(f), c_int(rows), c_int(cols), c_int(0 if rms_eps is None else 1),
+                                                     c_float(0.0 if rms_eps is None else rms_eps), _stream()), "tcavp_quant_e4m3_rows")
+    return q, f
 
 
 def launch_count():
