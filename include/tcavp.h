@@ -381,6 +381,31 @@ int tcavp_ce_loss(const float* logits, long long ld, const long long* targets, f
 int tcavp_adamw(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, long long n, float lr, float beta1, float beta2,
                 float eps, float weight_decay, int step, float grad_scale, tcavp_stream_t stream);
 
+/* ---- gradient-norm clipping and non-finite step skipping, decided on the device (reference modify_scripts/modify_train.py:1190-1196:
+ * a step whose loss is NaN is skipped, the gradient norm is clipped; scripts/modify_im_kim_train.py: clip_grad_norm_(…, 1.0) before
+ * optimizer.step()) ------------------------------------------------------------------------------------------------------------------ */
+typedef struct {
+  float total_norm; /* L2 norm of grad_scale * grad before clipping: the value torch.nn.utils.clip_grad_norm_ returns */
+  float clip_coef;  /* min(1, max_norm / (total_norm + 1e-6)) evaluated as torch does (NaN norm -> NaN); 1 when max_norm <= 0 */
+  int skip;         /* skip_nonfinite && (total_norm or *loss is not finite) */
+  int reserved;
+} tcavp_clip_record;
+#define TCAVP_CLIP_WORKSPACE_BYTES 9472 /* 1184 fp64 block partials, 8-byte aligned */
+/* Writes *record for the flat fp32 gradient buffer grad[n].  The norm is accumulated deterministically (fixed partition, fp64 block
+ * partials in `workspace`, fixed-order combine), so repeated calls and graph replays give the same bits.  Reads grad once.
+ * max_norm <= 0: no clipping (clip_coef = 1).  loss (one fp32 device value) may be NULL. */
+int tcavp_clip_prologue(const float* grad, long long n, float grad_scale, float max_norm, const float* loss, int skip_nonfinite,
+                        void* workspace, long long workspace_bytes, tcavp_clip_record* record, tcavp_stream_t stream);
+/* tcavp_adamw driven by a record of tcavp_clip_prologue and a device step counter.  record->skip set: param, exp_avg, exp_avg_sq and
+ * *step are left untouched and *skipped (may be NULL) is incremented.  Otherwise the gradient is multiplied by
+ * grad_scale * record->clip_coef, the bias corrections are those of tcavp_adamw for step = *step + 1, and *step is incremented. */
+int tcavp_adamw_clipped(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, long long n, float lr, float beta1, float beta2,
+                        float eps, float weight_decay, float grad_scale, const tcavp_clip_record* record, int* step, int* skipped,
+                        tcavp_stream_t stream);
+/* *dst = NaN when *loss is not finite.  Run on a gradient element before its all-reduce, it makes the global norm of every rank
+ * non-finite, so every rank skips the step a non-finite loss on one rank asks to skip. */
+int tcavp_mark_nonfinite(const float* loss, float* dst, tcavp_stream_t stream);
+
 /* ---- dropout (train mode: lora_dropout train.py:432-440 -> peft lora.Linear; nn.Dropout of train.py:664-671, 745-750; the
  * dropout / dropout1 / dropout2 / dropout3 of torch's nn.TransformerEncoderLayer / DecoderLayer, train.py:358, 402-405) --------------
  * Counter-based mask, a pure function of (seed, site, element index) — nothing is stored, the backward pass regenerates it:

@@ -1035,8 +1035,9 @@ int attention_bwd_tc_launch(const tcavp_attn_args& a, const void* dout, long lon
 // AdamW (torch.optim.AdamW semantics, reference scripts/im_kim_train_GRN.py:1008): decoupled weight decay,
 // bias-corrected moments.  One flat fp32 buffer per state.
 // ------------------------------------------------------------------------------------------------
-__global__ void adamw_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v, long long n,
-                             float lr, float b1, float b2, float eps, float wd, float bc1, float bc2_sqrt, float gscale) {
+__device__ __forceinline__ void adamw_update(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
+                                             long long n, float lr, float b1, float b2, float eps, float wd, float bc1, float bc2_sqrt,
+                                             float gscale) {
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
     const float gi = g[i] * gscale;
     float pi = p[i] * (1.f - lr * wd);
@@ -1048,6 +1049,115 @@ __global__ void adamw_kernel(float* __restrict__ p, const float* __restrict__ g,
     pi -= (lr / bc1) * (mi / denom);
     p[i] = pi;
   }
+}
+
+__global__ void adamw_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v, long long n,
+                             float lr, float b1, float b2, float eps, float wd, float bc1, float bc2_sqrt, float gscale) {
+  adamw_update(p, g, m, v, n, lr, b1, b2, eps, wd, bc1, bc2_sqrt, gscale);
+}
+
+// ------------------------------------------------------------------------------------------------
+// Gradient-norm clipping and non-finite step skipping (reference modify_scripts/modify_train.py:1190-1196: skip a step whose loss
+// is NaN, clip_grad_norm_; scripts/modify_im_kim_train.py: clip_grad_norm_(…, 1.0) before optimizer.step()).
+// The norm is a two-launch deterministic reduction: a fixed partition of the buffer over at most CLIP_BLOCKS blocks, one fp64
+// partial per block, then one block combines the partials in a fixed order.  No atomics and no counters to reset, so repeated
+// calls and graph replays give the same bits.
+// ------------------------------------------------------------------------------------------------
+constexpr int CLIP_BLOCKS = TCAVP_CLIP_WORKSPACE_BYTES / 8;   // 1184 = 8 resident blocks on each of the 148 SMs of a B200
+constexpr int CLIP_THREADS = 256;
+constexpr int CLIP_UNROLL = 4;                                // float4 loads in flight per thread
+
+__device__ __forceinline__ double block_sum_f64(double v, double* red) {
+  for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
+  __syncthreads();
+  double s = 0.0;
+  if (threadIdx.x == 0)
+    for (int w = 0; w < CLIP_THREADS / 32; ++w) s += red[w];
+  return s;   // valid in thread 0
+}
+
+// Squares of four elements summed in fp32 (at most 4 roundings, < 2.4e-7 relative), accumulated across the buffer in fp64.
+__device__ __forceinline__ double sumsq4(float4 x) {
+  return (double)fmaf(x.w, x.w, fmaf(x.z, x.z, fmaf(x.y, x.y, x.x * x.x)));
+}
+
+// Block b reduces g[b * chunk, min(n, (b + 1) * chunk)); chunk is a multiple of 4, so with VEC every block's float4 run is aligned.
+template <bool VEC>
+__global__ void __launch_bounds__(CLIP_THREADS, CLIP_BLOCKS / 148) clip_norm_partial_kernel(const float* __restrict__ g, long long n, long long chunk,
+                                                                         double* __restrict__ partial) {
+  __shared__ double red[CLIP_THREADS / 32];
+  const long long lo = blockIdx.x * chunk;
+  const long long hi = min(n, lo + chunk);
+  double acc = 0.0;
+  long long tail = lo;
+  if (VEC) {
+    const float4* v = reinterpret_cast<const float4*>(g + lo);
+    const long long nv = (hi - lo) >> 2;
+    long long i = threadIdx.x;
+#pragma unroll 1
+    for (; i + (CLIP_UNROLL - 1) * CLIP_THREADS < nv; i += CLIP_UNROLL * CLIP_THREADS) {
+      float4 x[CLIP_UNROLL];
+#pragma unroll
+      for (int u = 0; u < CLIP_UNROLL; ++u) x[u] = __ldcs(v + i + u * CLIP_THREADS);
+#pragma unroll
+      for (int u = 0; u < CLIP_UNROLL; ++u) acc += sumsq4(x[u]);
+    }
+#pragma unroll 1
+    for (; i < nv; i += CLIP_THREADS) acc += sumsq4(__ldcs(v + i));
+    tail = lo + (nv << 2);
+  }
+#pragma unroll 1
+  for (long long i = tail + threadIdx.x; i < hi; i += CLIP_THREADS) {
+    const float x = g[i];
+    acc += (double)(x * x);
+  }
+  const double s = block_sum_f64(acc, red);
+  if (threadIdx.x == 0) partial[blockIdx.x] = s;
+}
+
+__global__ void __launch_bounds__(CLIP_THREADS) clip_finish_kernel(const double* __restrict__ partial, int nparts, float grad_scale,
+                                                                   float max_norm, const float* __restrict__ loss, int skip_nonfinite,
+                                                                   tcavp_clip_record* __restrict__ rec) {
+  __shared__ double red[CLIP_THREADS / 32];
+  double s = 0.0;
+  for (int i = threadIdx.x; i < nparts; i += CLIP_THREADS) s += partial[i];
+  s = block_sum_f64(s, red);
+  if (threadIdx.x != 0) return;
+  const float norm = (float)(sqrt(s) * fabs((double)grad_scale));
+  float coef = 1.f;
+  if (max_norm > 0.f) {
+    // torch.nn.utils.clip_grad_norm_: max_norm / (total_norm + 1e-6) on an fp32 tensor is reciprocal() * max_norm, then
+    // clamp(max=1), which keeps a NaN (fminf would return 1 and let a NaN gradient through unclipped)
+    coef = __frcp_rn(norm + 1e-6f) * max_norm;
+    coef = coef > 1.f ? 1.f : coef;
+  }
+  rec->total_norm = norm;
+  rec->clip_coef = coef;
+  rec->skip = skip_nonfinite && (!isfinite(norm) || (loss != nullptr && !isfinite(*loss)));
+  rec->reserved = 0;
+}
+
+// tcavp_adamw with the gradient factor, the skip and the step number read from the device: the bias corrections are the host
+// expressions of tcavp_adamw evaluated for step = *step + 1.  The counter itself moves in adamw_count_kernel, after every block
+// has read it.
+__global__ void adamw_clipped_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v,
+                                     long long n, float lr, float b1, float b2, float eps, float wd, float gscale,
+                                     const tcavp_clip_record* __restrict__ clip, const int* __restrict__ step) {
+  if (clip->skip) return;
+  const float t = (float)(*step + 1);
+  adamw_update(p, g, m, v, n, lr, b1, b2, eps, wd, 1.f - powf(b1, t), sqrtf(1.f - powf(b2, t)), gscale * clip->clip_coef);
+}
+
+__global__ void adamw_count_kernel(const tcavp_clip_record* __restrict__ clip, int* __restrict__ step, int* __restrict__ skipped) {
+  if (!clip->skip)
+    ++*step;
+  else if (skipped != nullptr)
+    ++*skipped;
+}
+
+__global__ void mark_nonfinite_kernel(const float* __restrict__ loss, float* __restrict__ dst) {
+  if (!isfinite(*loss)) *dst = __int_as_float(0x7fc00000);
 }
 
 }  // namespace tcavp
@@ -1419,4 +1529,52 @@ extern "C" int tcavp_adamw(float* param, const float* grad, float* exp_avg, floa
   adamw_kernel<<<grid_cap((n + 255) / 256, 16), 256, 0, STREAM(stream)>>>(param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, weight_decay,
                                                                         bc1, bc2, grad_scale);
   return check_launch("adamw_kernel");
+}
+
+extern "C" int tcavp_clip_prologue(const float* grad, long long n, float grad_scale, float max_norm, const float* loss, int skip_nonfinite,
+                                   void* workspace, long long workspace_bytes, tcavp_clip_record* record, tcavp_stream_t stream) {
+  TCAVP_REQUIRE(n >= 0, "tcavp_clip_prologue: bad n");
+  TCAVP_REQUIRE(record && (n == 0 || (grad && workspace)), "tcavp_clip_prologue: null pointer");
+  TCAVP_REQUIRE(n == 0 || workspace_bytes >= TCAVP_CLIP_WORKSPACE_BYTES, "tcavp_clip_prologue: workspace below TCAVP_CLIP_WORKSPACE_BYTES");
+  TCAVP_REQUIRE(reinterpret_cast<uintptr_t>(workspace) % 8 == 0, "tcavp_clip_prologue: workspace not 8-byte aligned");
+  int parts = 0;
+  if (n > 0) {
+    // equal 4-aligned chunks, at most CLIP_BLOCKS of them and at least one unrolled block sweep (4096 elements) each
+    const long long sweep = (long long)CLIP_THREADS * CLIP_UNROLL * 4;
+    const long long want = (n + sweep - 1) / sweep;
+    const long long blocks = want < CLIP_BLOCKS ? want : CLIP_BLOCKS;
+    const long long chunk = ((n + blocks - 1) / blocks + 3) / 4 * 4;
+    parts = (int)((n + chunk - 1) / chunk);
+    double* partial = static_cast<double*>(workspace);
+    if (reinterpret_cast<uintptr_t>(grad) % 16 == 0)
+      clip_norm_partial_kernel<true><<<parts, CLIP_THREADS, 0, STREAM(stream)>>>(grad, n, chunk, partial);
+    else
+      clip_norm_partial_kernel<false><<<parts, CLIP_THREADS, 0, STREAM(stream)>>>(grad, n, chunk, partial);
+    int rc = check_launch("clip_norm_partial_kernel");
+    if (rc) return rc;
+  }
+  clip_finish_kernel<<<1, CLIP_THREADS, 0, STREAM(stream)>>>(static_cast<const double*>(workspace), parts, grad_scale, max_norm, loss,
+                                                             skip_nonfinite != 0, record);
+  return check_launch("clip_finish_kernel");
+}
+
+extern "C" int tcavp_adamw_clipped(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, long long n, float lr, float beta1,
+                                   float beta2, float eps, float weight_decay, float grad_scale, const tcavp_clip_record* clip, int* step,
+                                   int* skipped, tcavp_stream_t stream) {
+  TCAVP_REQUIRE(n >= 0, "tcavp_adamw_clipped: bad n");
+  TCAVP_REQUIRE(clip && step && (n == 0 || (param && grad && exp_avg && exp_avg_sq)), "tcavp_adamw_clipped: null pointer");
+  if (n > 0) {
+    adamw_clipped_kernel<<<grid_cap((n + 255) / 256, 16), 256, 0, STREAM(stream)>>>(param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps,
+                                                                                  weight_decay, grad_scale, clip, step);
+    int rc = check_launch("adamw_clipped_kernel");
+    if (rc) return rc;
+  }
+  adamw_count_kernel<<<1, 1, 0, STREAM(stream)>>>(clip, step, skipped);
+  return check_launch("adamw_count_kernel");
+}
+
+extern "C" int tcavp_mark_nonfinite(const float* loss, float* dst, tcavp_stream_t stream) {
+  TCAVP_REQUIRE(loss && dst, "tcavp_mark_nonfinite: null pointer");
+  mark_nonfinite_kernel<<<1, 1, 0, STREAM(stream)>>>(loss, dst);
+  return check_launch("mark_nonfinite_kernel");
 }

@@ -11,7 +11,13 @@ stack: everything outside `mllm.*` (regression head, cross-attention fusion — 
 shape —, temporal and lane-polygon encoders) has its final gradient by then, so that slice of the flat buffer is all-reduced on
 NCCL's stream WHILE the second graph (LoRA-Llama + Q-Former backward, the bulk of the step) runs; only the `mllm.*` slice is
 exchanged after it.  DistributedDataParallel gets the same overlap from its gradient buckets (train.py:1127-1132).  The reference's own loop (torch.optim.AdamW + DDP
-+ loss.backward()) also works unchanged on the same model — this class is the faster equivalent."""
++ loss.backward()) also works unchanged on the same model — this class is the faster equivalent.
+
+`max_grad_norm` / `skip_nonfinite` add the reference's two training safeguards (modify_scripts/modify_train.py:1190-1196: skip a step
+whose loss is NaN, clip_grad_norm_; scripts/modify_im_kim_train.py: clip_grad_norm_(…, 1.0)).  Both are decided on the device, after the
+all-reduce, so the step still needs no host synchronisation: tcavp_clip_prologue reads the reduced gradient once and writes the norm, the
+clip coefficient and the skip flag, and tcavp_adamw_clipped applies them with the optimiser step count kept on the device."""
+import math
 import os
 
 import torch
@@ -23,7 +29,17 @@ from .distributed import FlatGradBucket
 
 class FineTuner:
     def __init__(self, model, lr=5e-4, weight_decay=1e-4, betas=(0.9, 0.999), eps=1e-8, group=None, use_cuda_graph=True, max_graphs=8,
-                 overlap_allreduce=None):
+                 overlap_allreduce=None, max_grad_norm=None, skip_nonfinite=False):
+        """max_grad_norm: clip the global L2 norm of the averaged gradient to this value before AdamW, as
+        torch.nn.utils.clip_grad_norm_(params, max_grad_norm) after DDP's averaging does.  skip_nonfinite: leave the parameters, the
+        moments and the step count untouched when the loss of any rank or the gradient norm is not finite (the reference's
+        `if not torch.isfinite(loss): continue`).  A skipped step has still drawn its dropout masks: the mask counter advances inside
+        the captured forward, as the reference's RNG advances in its forward."""
+        if max_grad_norm is not None:
+            max_grad_norm = float(max_grad_norm)
+            if not (math.isfinite(max_grad_norm) and max_grad_norm > 0):
+                raise ValueError(f"max_grad_norm must be finite and > 0, got {max_grad_norm}")
+        self.max_grad_norm, self.skip_nonfinite = max_grad_norm, bool(skip_nonfinite)
         self.model, self.group = model, group
         self.lr, self.wd, self.betas, self.eps = lr, weight_decay, betas, eps
         named = model.trainable_named_parameters()
@@ -62,7 +78,15 @@ class FineTuner:
         self.targets = dict(zip(self.names, self.bucket.views))
         self.exp_avg = torch.zeros_like(self.flat_p)
         self.exp_avg_sq = torch.zeros_like(self.flat_p)
-        self.steps = 0
+        self.steps = 0                # step() calls
+        # clip / skip state: the tcavp_clip_record of the last step, the prologue's workspace, the optimiser step count and the number of
+        # skipped steps (device int32 each: a skip decided on the device cannot tell the host which step number comes next)
+        self._clip_rec = self._clip_ws = self.step_counter = self.skipped_steps = None
+        if self.max_grad_norm is not None or self.skip_nonfinite:
+            self._clip_rec = ops.clip_record(dev)
+            self._clip_ws = torch.empty(ops.CLIP_WORKSPACE_BYTES // 8, dtype=torch.float64, device=dev)
+            self.step_counter = torch.zeros((), dtype=torch.int32, device=dev)
+            self.skipped_steps = torch.zeros((), dtype=torch.int32, device=dev)
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
         self.use_cuda_graph = use_cuda_graph
         # one captured graph (+ its static input buffers and output tensors) per input-shape signature: the reference collate pads the
@@ -78,6 +102,12 @@ class FineTuner:
         if self.dropout_active:
             rank = dist.get_rank(group) if dist.is_initialized() else 0
             model.set_dropout_seed((torch.initial_seed() + 7919 * rank) & 0x7FFFFFFF, 0)
+
+    @property
+    def grad_norm(self):
+        """Device fp32 scalar: the global gradient norm of the last step before clipping (what clip_grad_norm_ returns); None when
+        neither option is set.  The next step overwrites it."""
+        return None if self._clip_rec is None else self._clip_rec[0]
 
     @property
     def payload_bytes(self):
@@ -201,20 +231,34 @@ class FineTuner:
         flat = self.bucket.flat
         works = []
         reduce = self.world > 1 and not skip_allreduce
+        # a non-finite loss on this rank turns one gradient element NaN before that element's all-reduce: the reduced norm is then
+        # NaN on every rank, and every rank skips
+        mark = reduce and self.skip_nonfinite
         if reduce and self.overlap and self.n_late < flat.numel():
             # gradients behind n_late are final: their exchange runs on NCCL's stream under the decoder-stack backward
+            if mark:
+                ops.mark_nonfinite_(loss, flat[self.n_late:])
             works.append(dist.all_reduce(flat[self.n_late:], op=dist.ReduceOp.SUM, group=self.group, async_op=True))
             second()
             if self.n_late:
                 works.append(dist.all_reduce(flat[:self.n_late], op=dist.ReduceOp.SUM, group=self.group, async_op=True))
         else:
             second()
+            if mark:
+                ops.mark_nonfinite_(loss, flat)
             if reduce:
                 works.append(dist.all_reduce(flat, op=dist.ReduceOp.SUM, group=self.group, async_op=True))
         for w in works:
             w.wait()                     # the current stream waits for the collective (no host block with NCCL)
         self.steps += 1
-        ops.adamw_(self.flat_p, flat, self.exp_avg, self.exp_avg_sq, lr=self.lr, betas=self.betas, eps=self.eps,
-                   weight_decay=self.wd, step=self.steps, grad_scale=1.0 / self.world)
+        if self._clip_rec is None:
+            ops.adamw_(self.flat_p, flat, self.exp_avg, self.exp_avg_sq, lr=self.lr, betas=self.betas, eps=self.eps,
+                       weight_decay=self.wd, step=self.steps, grad_scale=1.0 / self.world)
+        else:
+            ops.clip_prologue(flat, self._clip_rec, self._clip_ws, grad_scale=1.0 / self.world, max_norm=self.max_grad_norm, loss=loss,
+                              skip_nonfinite=self.skip_nonfinite)
+            ops.adamw_clipped_(self.flat_p, flat, self.exp_avg, self.exp_avg_sq, record=self._clip_rec, step=self.step_counter,
+                               skipped=self.skipped_steps, lr=self.lr, betas=self.betas, eps=self.eps, weight_decay=self.wd,
+                               grad_scale=1.0 / self.world)
         self.model._engine = None        # parameters changed behind torch's version counters: drop the inference packing
         return loss.detach(), decoded

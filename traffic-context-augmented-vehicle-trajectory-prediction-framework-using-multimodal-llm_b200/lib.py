@@ -26,6 +26,8 @@ EXPORTS = [
     "tcavp_rmsnorm_bwd", "tcavp_rope_adjacent", "tcavp_copy_rows", "tcavp_masked_mean_bwd", "tcavp_nlinear_bwd", "tcavp_head_assemble",
     "tcavp_traj_loss_bwd", "tcavp_skinny_dw", "tcavp_dw", "tcavp_attention_bwd", "tcavp_attention_bwd_owned", "tcavp_adamw",
     "tcavp_lora_a_drop", "tcavp_lora_dx_drop", "tcavp_lora_da_drop", "tcavp_ce_loss", "tcavp_gelu_tanh", "tcavp_gelu_tanh_bwd", "tcavp_layernorm_bwd_dx", "tcavp_layernorm_strided",
+    # gradient clipping / non-finite step skipping
+    "tcavp_clip_prologue", "tcavp_adamw_clipped", "tcavp_mark_nonfinite",
     # fp8 serving mode
     "tcavp_quant_e4m3_rows",
 ]

@@ -821,3 +821,54 @@ def adamw_(param, grad, exp_avg, exp_avg_sq, *, lr, betas=(0.9, 0.999), eps=1e-8
     _call("tcavp_adamw", "adamw_kernel", _p(param), _p(grad), _p(exp_avg), _p(exp_avg_sq), _ll(param.numel()), c_float(lr), c_float(betas[0]),
           c_float(betas[1]), c_float(eps), c_float(weight_decay), int(step), c_float(grad_scale))
     return param
+
+
+CLIP_WORKSPACE_BYTES = 9472       # include/tcavp.h: TCAVP_CLIP_WORKSPACE_BYTES
+
+
+def _flat_f32(name, *ts):
+    for t in ts:
+        if t is not None and (t.dtype != torch.float32 or not t.is_contiguous()):
+            raise TypeError(f"{name}: flat contiguous fp32 buffers required")
+
+
+def clip_record(device):
+    """A zeroed tcavp_clip_record on `device`: fp32 [total_norm, clip_coef, skip (int32 bits), reserved]."""
+    return torch.zeros(4, dtype=torch.float32, device=device)
+
+
+def clip_prologue(grad, record, workspace, *, grad_scale=1.0, max_norm=None, loss=None, skip_nonfinite=False):
+    """record <- {total_norm = ||grad_scale * grad||_2, clip_coef (torch.nn.utils.clip_grad_norm_'s, 1 when max_norm is None),
+    skip = skip_nonfinite and (total_norm or loss not finite)}.  workspace: >= CLIP_WORKSPACE_BYTES of device memory."""
+    _need_cuda(grad, record, workspace, loss)
+    _flat_f32("clip_prologue", grad, record, loss)
+    if record.numel() != 4 or (loss is not None and loss.numel() != 1):
+        raise ValueError("clip_prologue: record is fp32[4] (clip_record()), loss one fp32 value")
+    _call("tcavp_clip_prologue", "clip_norm_kernel", _p(grad), _ll(grad.numel()), c_float(grad_scale), c_float(max_norm or 0.0), _p(loss),
+          int(bool(skip_nonfinite)), _p(workspace), _ll(workspace.numel() * workspace.element_size()), _p(record), nbytes=_nb(grad))
+    return record
+
+
+def adamw_clipped_(param, grad, exp_avg, exp_avg_sq, *, record, step, skipped=None, lr, betas=(0.9, 0.999), eps=1e-8, weight_decay=1e-2,
+                   grad_scale=1.0):
+    """adamw_ with the clip coefficient and the skip decision of a clip_prologue record and the step number in the device int32
+    counter `step` (incremented unless the step is skipped; `skipped` counts the skipped steps)."""
+    _need_cuda(param, grad, exp_avg, exp_avg_sq, record, step, skipped)
+    _flat_f32("adamw_clipped_", param, grad, exp_avg, exp_avg_sq, record)
+    for t in (step, skipped):
+        if t is not None and (t.dtype != torch.int32 or t.numel() != 1):
+            raise TypeError("adamw_clipped_: step / skipped are one device int32 each")
+    _call("tcavp_adamw_clipped", "adamw_clipped_kernel", _p(param), _p(grad), _p(exp_avg), _p(exp_avg_sq), _ll(param.numel()), c_float(lr),
+          c_float(betas[0]), c_float(betas[1]), c_float(eps), c_float(weight_decay), c_float(grad_scale), _p(record), _p(step), _p(skipped),
+          nbytes=_nb(param, grad, exp_avg, exp_avg_sq) + _nb(param, exp_avg, exp_avg_sq))
+    return param
+
+
+def mark_nonfinite_(loss, dst):
+    """dst[0] = NaN when the device scalar `loss` is not finite."""
+    _need_cuda(loss, dst)
+    _flat_f32("mark_nonfinite_", loss, dst)
+    if loss.numel() != 1 or dst.numel() == 0:
+        raise ValueError("mark_nonfinite_: loss is one value, dst not empty")
+    _call("tcavp_mark_nonfinite", "mark_nonfinite_kernel", _p(loss), _p(dst))
+    return dst
