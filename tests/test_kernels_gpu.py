@@ -585,16 +585,16 @@ def test_gemm_large_fused_rope_and_lora_extension(ops):
     torch.testing.assert_close(out.float().cpu(), want, rtol=2e-2, atol=2e-2)
 
 
-@pytest.mark.parametrize("wide", [True, False])
-def test_gemm_wide_kernel_sampled_rows(ops, wide):
+@pytest.mark.parametrize("wide_k,kernel", [(2048, "gemm_tc_wide_kernel"), (0, "gemm_tc_pair_kernel<256>")], ids=["wide", "pair"])
+def test_gemm_wide_kernel_sampled_rows(ops, wide_k, kernel):
     """The 512 x 256 pair tile (K >= 2048 and >= 4 waves of tiles) at a 7B-like shape; the CPU check samples rows (incl. the first / last
     row of several 128-row halves) instead of forming the whole product.  Which kernel serves long contractions is tuned per board
-    (ops.autotune_gemm_route), so both are pinned here in turn (`wide` False: the 256 x 256 pair tile on the same problem)."""
+    (ops.autotune_gemm_route), so both are pinned here in turn (`pair`: the 256 x 256 pair tile on the same problem)."""
     import tcavp_b200.lib as L
     ops.autotune_gemm_route()                         # whatever the process decided is restored below
-    old = L.load().tcavp_gemm_wide_min_k(2048 if wide else 0)
+    old = L.load().tcavp_gemm_wide_min_k(wide_k)
     try:
-        _wide_kernel_case(ops, "gemm_tc_wide_kernel" if wide else "gemm_tc_pair_kernel")
+        _wide_kernel_case(ops, kernel)
     finally:
         L.load().tcavp_gemm_wide_min_k(old)
 
@@ -626,6 +626,64 @@ def _wide_kernel_case(ops, kernel):
     sw = ops.gemm(a, w, torch.empty(M, N // 2, dtype=torch.bfloat16, device=DEV), act=ops.ACT_SWIGLU)
     y = a[rows].float() @ w.float().t()
     torch.testing.assert_close(sw[rows].float(), torch.nn.functional.silu(y[:, 0::2]) * y[:, 1::2], rtol=3e-2, atol=2e-2)
+
+
+def test_profiler_labels_name_the_launched_kernel(ops):
+    """LaunchProfiler labels of ops.gemm / ops.attention: the kernel tcavp_gemm / tcavp_attention launched (tcavp_last_kernel) plus
+    the problem shape, for one shape per route; the long-K route is pinned both ways.  An empty GEMM launches nothing and is not recorded."""
+    import tcavp_b200.lib as L
+
+    def gemm(M, N, K, dtype=torch.bfloat16):
+        a, w = torch.randn(M, K, device=DEV), torch.randn(N, K, device=DEV) * K ** -0.5
+        out = torch.empty(M, N, device=DEV, dtype=torch.float32 if dtype == torch.float32 else torch.bfloat16)
+        if dtype == torch.float8_e4m3fn:
+            ops.gemm(a.to(dtype), w.to(dtype), out, col_scale=torch.ones(N, device=DEV))
+        else:
+            ops.gemm(a.to(dtype), w.to(dtype), out)
+
+    def attention(B, H, Hkv, Tq, Tk, dh, causal=False, dtype=torch.bfloat16, shared_kv=False):
+        q = torch.randn(B, Tq, H, dh, device=DEV).to(dtype)
+        k = torch.randn(B, Tk, Hkv, dh, device=DEV).to(dtype)
+        v = k if shared_kv else torch.randn(B, Tk, Hkv, dh, device=DEV).to(dtype)
+        ops.attention(q, k, v, torch.empty_like(q), B=B, H=H, Hkv=Hkv, Tq=Tq, Tk=Tk, dh=dh, q_strides=(Tq * H * dh, H * dh),
+                      k_strides=(Tk * Hkv * dh, Hkv * dh), v_strides=(Tk * Hkv * dh, Hkv * dh), o_strides=(Tq * H * dh, H * dh),
+                      scale=dh ** -0.5, causal=causal)
+
+    ops.autotune_gemm_route()                         # before the pins below; whatever the process decided is restored at the end
+    old = L.load().tcavp_gemm_wide_min_k(-1)
+    try:
+        with ops.LaunchProfiler() as prof:
+            gemm(300, 32, 64)
+            gemm(300, 64, 64)
+            gemm(300, 100, 64)
+            gemm(300, 200, 64)
+            gemm(4100, 520, 64)
+            gemm(32768, 256, 64)
+            gemm(0, 256, 64)
+            gemm(100, 24, 72, torch.float32)
+            gemm(300, 200, 128, torch.float8_e4m3fn)
+            gemm(4100, 520, 128, torch.float8_e4m3fn)
+            L.load().tcavp_gemm_wide_min_k(2048)
+            gemm(16384, 2560, 2048)
+            L.load().tcavp_gemm_wide_min_k(0)
+            gemm(16384, 2560, 2048)
+            attention(2, 4, 4, 144, 144, 64, causal=True)
+            attention(2, 2, 1, 25, 144, 256, shared_kv=True)
+            attention(2, 2, 2, 25, 144, 384)
+            attention(2, 8, 8, 15, 15, 96)
+            attention(3, 2, 2, 15, 15, 32, dtype=torch.float32)
+            attention(2, 8, 8, 15, 15, 96, dtype=torch.float32)
+    finally:
+        L.load().tcavp_gemm_wide_min_k(old)
+    assert [r[0] for r in prof.rec] == [
+        "gemm_tc_kernel<32>[N32,K64]", "gemm_tc_kernel<64>[N64,K64]", "gemm_tc_kernel<128>[N100,K64]", "gemm_tc_kernel<256>[N200,K64]",
+        "gemm_tc_pair_kernel<256>[M4100,N520,K64]", "gemm_tc_pair_kernel<256>[N256,K64]", "gemm_simt_kernel",
+        "gemm_tc_kernel<256,e4m3>[N200,K128]", "gemm_tc_pair_kernel<256,e4m3>[M4100,N520,K128]",
+        "gemm_tc_wide_kernel[N2560,K2048]", "gemm_tc_pair_kernel<256>[M16384,N2560,K2048]",
+        "attn_tm_kernel[dh64,L144]", "attn_xt_kernel[dh256,q25,k144]", "attn_x_kernel", "attn_flash_kernel[dh96,q15,k15]",
+        "attn_row_kernel[dh32,q15,k15]", "attn_warp_kernel[dh96,q15,k15]"]
+    # algorithmic bytes: the shared K = V head of attn_xt_kernel is read once, the K and V heads of attn_x_kernel once each
+    assert prof.rec[12][2] == 2 * 2 * 256 * (2 * 2 * 25 + 1 * 144) and prof.rec[13][2] == 2 * 2 * 384 * (2 * 2 * 25 + 2 * 2 * 144)
 
 
 @pytest.mark.parametrize("pw", [1, 3, 5])

@@ -1,5 +1,5 @@
 """Times tcavp_gemm for ~1.5 s per shape with SM clock / power sampled through NVML, and reports per-clock tensor-pipe
-utilisation (TF/s / (148 SM x 8192 FLOP/clk x clk)).  TCAVP_GEMM_DEBUG bits (pair kernel only): 16 no TMA, 32 no MMA, 64 no epilogue."""
+utilisation (TF/s / (148 SM x 8192 FLOP/clk x clk))."""
 import os, sys, time, threading, statistics, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import tcavp_b200.lib as L
@@ -40,4 +40,4 @@ for (M, N, K) in shapes:
     ms = e0.elapsed_time(e1) / n
     tf = 2.0 * M * N * K / ms / 1e9
     c = statistics.median(clk[len(clk) // 2:]); p = statistics.median(pw[len(pw) // 2:])
-    print(f"mode={os.environ.get('TCAVP_GEMM_CLUSTER','3')} dbg={os.environ.get('TCAVP_GEMM_DEBUG','0')} M{M} N{N} K{K}: {ms*1e3:.1f} us {tf:.0f} TF/s  clk {c:.0f} MHz  {p:.0f} W  util/clk {tf*1e12/(148*8192*c*1e6):.3f}  probe clk {float(probe[0])/max(float(probe[1]),1)*1e3:.0f} MHz -> util {tf*1e12/(148*8192*max(float(probe[0]),1)/max(float(probe[1]),1)*1e9):.3f}", flush=True)
+    print(f"M{M} N{N} K{K}: {ms*1e3:.1f} us {tf:.0f} TF/s  clk {c:.0f} MHz  {p:.0f} W  util/clk {tf*1e12/(148*8192*c*1e6):.3f}  probe clk {float(probe[0])/max(float(probe[1]),1)*1e3:.0f} MHz -> util {tf*1e12/(148*8192*max(float(probe[0]),1)/max(float(probe[1]),1)*1e9):.3f}", flush=True)

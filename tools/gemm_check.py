@@ -1,5 +1,5 @@
 """GPU-box check of tcavp_gemm (bf16 tcgen05 paths) against torch matmul + CUDA-event timings per shape.
-    TCAVP_GEMM_CLUSTER={1,2,3} python tools/gemm_check.py [--time]
+    python tools/gemm_check.py [--time] [--big]
 Run under `timeout` — a barrier mistake in a new kernel variant hangs instead of failing."""
 import os
 import sys
@@ -19,7 +19,7 @@ SHAPES = [  # (M, N, K)  incl. ragged M / N / K tails
     (147456, 768, 3072), (2048 + 130, 320, 200), (36864, 12288, 4096), (36864, 4096, 4096), (36864, 22016, 4096), (36864, 4096, 11008),
     (36864 + 300, 11008 + 64, 4096),
 ]
-if "--big" in sys.argv:      # the 7B-class shapes only (W larger than the L2 panel budget: TCAVP_GEMM_PANEL_MB A/B)
+if "--big" in sys.argv:      # the 7B-class shapes only (W larger than the 40 MB L2 panel budget)
     SHAPES = [s for s in SHAPES if s[2] >= 4096]
 timing = "--time" in sys.argv
 for (M, N, K) in SHAPES:

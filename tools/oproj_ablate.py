@@ -1,7 +1,7 @@
 """Where does the o_proj-shaped GEMM (M = 147 456, N = K = 768: the slowest K = 768 group of the cfg2 step) lose its time?
 Times tcavp_gemm on that shape with the epilogue terms switched on one at a time (device events, ~0.3 s per variant, A-B-A order so a
 clock drift shows up as a difference between the two passes of the same variant), next to the QKV / gate-up shapes of the same step.
-    python tools/oproj_ablate.py                 # TCAVP_GEMM_DEBUG=64 (no epilogue) / 128 (no stores) for the kernel-side ablation"""
+    python tools/oproj_ablate.py"""
 import os
 import sys
 
@@ -57,7 +57,6 @@ rows = {name: [] for name, _ in VARIANTS}
 for rnd in range(2):
     for name, fn in VARIANTS:
         rows[name].append(timed(fn, 400 if "shape" not in name else 150))
-print(f"TCAVP_GEMM_DEBUG={os.environ.get('TCAVP_GEMM_DEBUG', '0')}")
 for name, _ in VARIANTS:
     N, K = (2304, Kx) if "QKV" in name else (6144, H) if "gate" in name else (H, H)
     fl = 2.0 * M * N * K

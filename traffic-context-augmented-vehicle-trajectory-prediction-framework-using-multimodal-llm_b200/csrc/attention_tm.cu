@@ -140,74 +140,58 @@ __device__ __forceinline__ uint32_t unit_bits(const uint32_t* s_mask, int u, int
   return key16 & c16;
 }
 
-// Softmax of one score row per thread (TMEM lane = row): two sweeps over the row's scores (row max, then exp2 / row sum / P), each in
-// batches of UB x 16 columns (UB x16 loads in flight, one wait; larger batches cost more in instruction-cache misses than they hide).  The bf16 probabilities overwrite the score columns (P aliases S).  A
+// Softmax of one score row per thread (TMEM lane = row): two sweeps over the row's scores (row max, then exp2 / row sum / P), each one
+// 16-column unit (one x16 load, one wait) at a time: batches of two units in flight cost more in instruction-cache misses than they hid
+// (211 us against 202 us on the 768-class shape).  The bf16 probabilities overwrite the score columns (P aliases S).  A
 // 16-column unit whose keys are all attendable for every row of the warp (the common case left of the causal diagonal) takes a
 // select-free path.  `q`: query index of the row, `ncols`: key columns of the tile, `warp_kmax`: largest key any row of the warp sees.
 // Returns the row sum.
 // (__noinline__: tile A and tile B share one copy — ten warps in different places of a 60 KB kernel thrash the instruction caches)
-template <int UB>
 __device__ __noinline__ float softmax_rows(const Geo& g, uint32_t srow, int q, int ncols, int warp_kmax, const uint32_t* s_mask) {
   const int nu = min(ncols, (warp_kmax + 16) & ~15) >> 4;
   const int nu_all = ncols >> 4;
-  const int nbatch = (nu + UB - 1) / UB;
   float m = -INFINITY;
-  for (int bt = 0; bt < nbatch; ++bt) {
-    uint32_t r[UB][16];
-#pragma unroll
-    for (int i = 0; i < UB; ++i) tmem_ld16_issue(srow + (bt * UB + i) * 16, r[i]);   // unconditional: columns past `nu` stay inside the 512 and are skipped below
+  for (int u = 0; u < nu; ++u) {
+    uint32_t r[16];
+    tmem_ld16_issue(srow + u * 16, r);
     tmem_ld_wait();
+    tmem_ld_fence(r);
+    const uint32_t vb = unit_bits(s_mask, u, q);
+    if (__all_sync(0xffffffffu, vb == 0xFFFFu)) {
 #pragma unroll
-    for (int i = 0; i < UB; ++i) {
-      const int u = bt * UB + i;
-      if (u < nu) {
-        tmem_ld_fence(r[i]);
-        const uint32_t vb = unit_bits(s_mask, u, q);
-        if (__all_sync(0xffffffffu, vb == 0xFFFFu)) {
+      for (int c = 0; c < 16; ++c) m = fmaxf(m, __uint_as_float(r[c]));
+    } else {
 #pragma unroll
-          for (int c = 0; c < 16; ++c) m = fmaxf(m, __uint_as_float(r[i][c]));
-        } else {
-#pragma unroll
-          for (int c = 0; c < 16; ++c) m = fmaxf(m, ((vb >> c) & 1u) ? __uint_as_float(r[i][c]) : -INFINITY);
-        }
-      }
+      for (int c = 0; c < 16; ++c) m = fmaxf(m, ((vb >> c) & 1u) ? __uint_as_float(r[c]) : -INFINITY);
     }
   }
   const float mref = m == -INFINITY ? 0.f : m * g.sl2;
   float l = 0.f;
-  for (int bt = 0; bt < nbatch; ++bt) {
-    uint32_t r[UB][16];
-#pragma unroll
-    for (int i = 0; i < UB; ++i) tmem_ld16_issue(srow + (bt * UB + i) * 16, r[i]);
+  for (int u = 0; u < nu; ++u) {
+    uint32_t r[16];
+    tmem_ld16_issue(srow + u * 16, r);
     tmem_ld_wait();
-    // every score column of this batch is in registers: the bf16 probabilities may now overwrite score columns (8u + 8 <= 16u + 16,
-    // and the batch's own columns have been read)
+    // the unit's score columns are in registers: its bf16 probabilities may now overwrite score columns (8u + 8 <= 16u + 16)
+    tmem_ld_fence(r);
+    uint32_t pk[8];
+    const uint32_t vb = unit_bits(s_mask, u, q);
+    if (__all_sync(0xffffffffu, vb == 0xFFFFu)) {
 #pragma unroll
-    for (int i = 0; i < UB; ++i) {
-      const int u = bt * UB + i;
-      if (u < nu) {
-        tmem_ld_fence(r[i]);
-        uint32_t pk[8];
-        const uint32_t vb = unit_bits(s_mask, u, q);
-        if (__all_sync(0xffffffffu, vb == 0xFFFFu)) {
+      for (int c = 0; c < 16; c += 2) {
+        const float p0 = ex2(fmaf(__uint_as_float(r[c]), g.sl2, -mref)), p1 = ex2(fmaf(__uint_as_float(r[c + 1]), g.sl2, -mref));
+        l += p0 + p1;
+        pk[c >> 1] = pack2(p0, p1);
+      }
+    } else {
 #pragma unroll
-          for (int c = 0; c < 16; c += 2) {
-            const float p0 = ex2(fmaf(__uint_as_float(r[i][c]), g.sl2, -mref)), p1 = ex2(fmaf(__uint_as_float(r[i][c + 1]), g.sl2, -mref));
-            l += p0 + p1;
-            pk[c >> 1] = pack2(p0, p1);
-          }
-        } else {
-#pragma unroll
-          for (int c = 0; c < 16; c += 2) {
-            const float p0 = ((vb >> c) & 1u) ? ex2(fmaf(__uint_as_float(r[i][c]), g.sl2, -mref)) : 0.f;
-            const float p1 = ((vb >> (c + 1)) & 1u) ? ex2(fmaf(__uint_as_float(r[i][c + 1]), g.sl2, -mref)) : 0.f;
-            l += p0 + p1;
-            pk[c >> 1] = pack2(p0, p1);
-          }
-        }
-        tmem_st8(srow + u * 8, pk);
+      for (int c = 0; c < 16; c += 2) {
+        const float p0 = ((vb >> c) & 1u) ? ex2(fmaf(__uint_as_float(r[c]), g.sl2, -mref)) : 0.f;
+        const float p1 = ((vb >> (c + 1)) & 1u) ? ex2(fmaf(__uint_as_float(r[c + 1]), g.sl2, -mref)) : 0.f;
+        l += p0 + p1;
+        pk[c >> 1] = pack2(p0, p1);
       }
     }
+    tmem_st8(srow + u * 8, pk);
   }
   {
     const uint32_t z[8] = {0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u};
@@ -249,7 +233,7 @@ constexpr uint32_t BAR_FULL = 0, BAR_EMPTY = 8 * MAX_STAGES, BAR_MASK = 16 * MAX
 constexpr uint32_t SL_SFULL = 0, SL_PB = 8, SL_PA = 16, SL_OBFULL = 24, SL_OBDRAINED = 32, SL_OAFULL = 40, SL_OFREE = 48, SL_BYTES = 56;
 constexpr uint32_t BAR_BYTES = BAR_SLOT + MAX_SLOTS * SL_BYTES + 8;     // + the TMEM base address slot
 
-template <int DH, int UB>
+template <int DH>
 __global__ void __launch_bounds__(THREADS, 1)
 attn_tm_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constant__ CUtensorMap tma_k, const __grid_constant__ CUtensorMap tma_v, Geo g) {
   constexpr int NBOX = DH / BOXC;      // 64-column boxes per operand
@@ -416,12 +400,12 @@ attn_tm_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constant_
       const int qb = wq * 32 + lane;                    // tile B row = query index
       if (has_b) {
         // rows >= NB of tile B are not part of the problem: their query index is pushed past L so nothing is stored for them
-        l_b = softmax_rows<UB>(g, lane_base + g.sb_col, qb < g.NB ? qb : g.L + qb, g.NB, min(wq * 32 + 31, g.NB - 1), s_mask[st]);
+        l_b = softmax_rows(g, lane_base + g.sb_col, qb < g.NB ? qb : g.L + qb, g.NB, min(wq * 32 + 31, g.NB - 1), s_mask[st]);
         __syncwarp();
         if (lane == 0) mbar_arrive(sbar + SL_PB);
       }
       const int qa = qa0 + wq * 32 + lane;
-      const float l_a = softmax_rows<UB>(g, lane_base, qa, g.L16, qa0 + wq * 32 + 31, s_mask[st]);
+      const float l_a = softmax_rows(g, lane_base, qa, g.L16, qa0 + wq * 32 + 31, s_mask[st]);
       __syncwarp();
       if (lane == 0) mbar_arrive(sbar + SL_PA);
       if (has_b) {
@@ -510,15 +494,9 @@ int attention_tm_launch(const tcavp_attn_args& a, cudaStream_t stream) {
   g.o_col = (uint32_t)((L16 + NB + 31) / 32 * 32);
   g.slot_cols = g.o_col + (uint32_t)a.dh;
   if (g.slot_cols > 512u) return 1;
-  static int max_slots = -1;
-  if (max_slots < 0) {
-    const char* e = getenv("TCAVP_ATTN_SLOTS");       // 1: one item in flight per CTA (A/B runs)
-    max_slots = e ? atoi(e) : MAX_SLOTS;
-    if (max_slots < 1 || max_slots > MAX_SLOTS) max_slots = MAX_SLOTS;
-  }
   const int fit = (int)((225u * 1024u - 2048u) / g.stage_bytes);     // stages that fit in shared memory
   if (fit < 1) return 1;
-  g.slots = (2u * g.slot_cols <= 512u && fit >= 2 && max_slots >= 2) ? 2 : 1;
+  g.slots = (2u * g.slot_cols <= 512u && fit >= 2) ? MAX_SLOTS : 1;
   g.stages = fit >= 2 * g.slots ? 2 * g.slots : (fit >= g.slots ? (fit / g.slots) * g.slots : 1);
   if (g.stages > MAX_STAGES) g.stages = MAX_STAGES;
   if (g.stages < g.slots) g.slots = 1;
@@ -535,23 +513,13 @@ int attention_tm_launch(const tcavp_attn_args& a, cudaStream_t stream) {
   if (smem < 118 * 1024) smem = 118 * 1024;
   const int items = a.B * a.H;
   const int grid = items < sm_count() ? items : sm_count();
-  static int ub = -1;
-  if (ub < 0) {
-    const char* e = getenv("TCAVP_ATTN_UB");           // score columns per tcgen05.ld batch / 16 (A/B runs)
-    ub = e ? atoi(e) : 1;
-  }
-#define TCAVP_TM(DH_, UB_)                                                                                              \
-  do {                                                                                                                  \
-    TCAVP_CUDA(cudaFuncSetAttribute(attn_tm_kernel<DH_, UB_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    attn_tm_kernel<DH_, UB_><<<grid, THREADS, smem, stream>>>(mq, mk, mv, g);                                           \
-  } while (0)
-  // one 16-column unit per batch is the fastest (smallest loop bodies: 202 us against 211 us with two units on the 768-class shape)
   if (a.dh == 64) {
-    if (ub == 2) TCAVP_TM(64, 2); else TCAVP_TM(64, 1);
+    TCAVP_CUDA(cudaFuncSetAttribute(attn_tm_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    attn_tm_kernel<64><<<grid, THREADS, smem, stream>>>(mq, mk, mv, g);
   } else {
-    if (ub == 2) TCAVP_TM(128, 2); else TCAVP_TM(128, 1);
+    TCAVP_CUDA(cudaFuncSetAttribute(attn_tm_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    attn_tm_kernel<128><<<grid, THREADS, smem, stream>>>(mq, mk, mv, g);
   }
-#undef TCAVP_TM
   return check_launch("attn_tm_kernel");
 }
 

@@ -5,11 +5,11 @@
 //          128-byte swizzle) into a multi-stage shared-memory ring; warp 1: one elected thread issues tcgen05.mma (bf16 -> fp32)
 //          into TMEM; 16 epilogue warps drain TMEM with tcgen05.ld, apply the fused epilogue and store 32 bytes per lane.
 //          Variants, picked by tcavp_gemm from the problem shape:
-//            gemm_tc_kernel<BN, CM>   one CTA per 128 x BN tile (BN 32..256), double-buffered accumulators; CM = 2 multicasts W
+//            gemm_tc_kernel<BN>       one CTA per 128 x BN tile (BN 32..256), double-buffered accumulators
 //            gemm_tc_pair_kernel<256> CTA pair (cta_group::2) on a 256 x 256 tile, double-buffered accumulators (the default for
 //                                     large problems: the epilogue of tile i overlaps the MMAs of tile i+1)
 //            gemm_tc_wide_kernel      CTA pair on a 512 x 256 tile, all 512 TMEM columns, for long contractions (K >= 2048)
-//            gemm_tc_quad_kernel<256> two pairs per 4-CTA cluster sharing W by multicast (A/B option only)
+//   e4m3 : the gemm_tc_kernel and gemm_tc_pair_kernel pipelines with tcgen05.mma.kind::f8f6f4 and per-column dequantisation.
 //   fp32 : SIMT FFMA kernel with exact fp32 accumulation (the rtol 1e-4 parity mode; no TF32).
 //
 // LoRA (peft lora.Linear, reference scripts/train.py:432-440) is expressed by the caller as extra K columns
@@ -77,13 +77,6 @@ __device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map
       : "memory");
 }
 
-// Same load, delivered to the same shared-memory offset (and signalling the same barrier offset) in every CTA of `mask`.
-__device__ __forceinline__ void tma_load_2d_mc(uint32_t dst, const CUtensorMap* map, uint32_t bar, int c0, int c1, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;" ::"r"(dst),
-      "l"(reinterpret_cast<uint64_t>(map)), "r"(bar), "r"(c0), "r"(c1), "h"(mask)
-      : "memory");
-}
 __device__ __forceinline__ uint32_t cluster_ctarank() {
   uint32_t r;
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
@@ -132,10 +125,6 @@ __device__ __forceinline__ void umma_e4m3(uint32_t tmem_d, uint64_t adesc, uint6
 }
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void umma_commit_mc(uint32_t bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar), "h"(mask)
-               : "memory");
 }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
@@ -215,8 +204,7 @@ __host__ __device__ __forceinline__ void unit_to_tile(int u, int tiles_mg, int t
 constexpr int PANEL_SHIFT = 16;   // flags >> PANEL_SHIFT = panel width in n-tiles (0: no panels)
 
 enum { EPI_VEC_OUT = 1, EPI_VEC_RES = 2, EPI_VEC_BIAS = 4, EPI_TMA_OUT = 8,    // EPI_TMA_OUT: bf16 output staged in shared memory, stored by TMA
-       DBG_NO_TMA = 16, DBG_NO_MMA = 32, DBG_NO_EPI = 64, DBG_NO_STORE = 128,   // TCAVP_GEMM_DEBUG: ablation switches for profiling (results are garbage)
-       L2_W_LAST = 256, L2_A_FIRST = 512, L2_OUT_FIRST = 1024 };      // L2 eviction priorities of a panelled problem (TCAVP_GEMM_L2HINT)
+       L2_W_LAST = 256, L2_OUT_FIRST = 1024 };      // L2 eviction priorities of a panelled problem (see panel_flags)
 
 // e4m3 operands: accumulator column n carries the dequantisation factor col_scale[n] of its weight row.  Applied to the raw accumulators
 // (before the row factor, RoPE and SwiGLU, which mix or pair columns with different scales); columns past Nacc get 0.
@@ -377,14 +365,6 @@ __device__ __forceinline__ void epilogue_chunk(const EpilogueParams& p, int m, i
     for (int j = 0; j < 32; ++j)
       if (j < cnt && (full || n0 + j < p.N)) ssq = fmaf(o[j], o[j], ssq);
   }
-  if (flags & DBG_NO_STORE) {      // profiling ablation: everything but the global stores (keeps the math alive through ssq)
-    float t = 0.f;
-#pragma unroll
-    for (int j = 0; j < 32; ++j)
-      if (j < cnt) t += o[j];
-    ssq += t;
-    return;
-  }
   if (flags & EPI_TMA_OUT) {
     // bf16 rows of the warp's 32 x 64 (SwiGLU: 32 x 32) output tile in the swizzled layout the TMA store expects: 16-byte chunk j of
     // row r sits at chunk j ^ (r & 7) of a 128-byte row (SWIZZLE_128B) / j ^ ((r >> 1) & 3) of a 64-byte row (SWIZZLE_64B).
@@ -438,16 +418,11 @@ __device__ __forceinline__ void epilogue_chunk(const EpilogueParams& p, int m, i
   }
 }
 
-// CM = CTAs per cluster along M.  With CM = 2 the two CTAs of a cluster work on vertically adjacent output tiles that
-// share the W tile: each CTA fetches half of it and TMA-multicasts that half into both shared memories, which cuts
-// the L2 -> SM operand traffic per CTA from A + W to A + W/2 (the binding resource for K <= 1024 GEMMs).
-template <int BLOCK_N, int CM, bool F8 = false>
+template <int BLOCK_N, bool F8 = false>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b, EpilogueParams ep,
                int M, int Nacc, int K, int flags) {
   using C = Cfg<BLOCK_N>;
-  const uint32_t cta_rank = CM > 1 ? cluster_ctarank() : 0u;
-  constexpr uint16_t MC_MASK = (uint16_t)((1u << CM) - 1);
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   const uint32_t smem_a = smem_base;
@@ -464,9 +439,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
   const int lane = threadIdx.x & 31;
   const int tiles_n = (Nacc + BLOCK_N - 1) / BLOCK_N;
   const int tiles_m = (M + BLOCK_M - 1) / BLOCK_M;
-  // work unit = CM vertically adjacent tiles; unit u -> (m group u / tiles_n, n tile u % tiles_n); a cluster strides over units
-  const int num_units = ((tiles_m + CM - 1) / CM) * tiles_n;
-  const int unit0 = blockIdx.x / CM, unit_stride = gridDim.x / CM;
+  const int num_units = tiles_m * tiles_n;
+  const int unit0 = blockIdx.x, unit_stride = gridDim.x;
   using O = Op<F8>;
   const int num_kb = (K + O::KB - 1) / O::KB;
   const int pw = (flags >> PANEL_SHIFT) > 0 ? (flags >> PANEL_SHIFT) : tiles_n;   // n-tiles per L2-resident panel of W
@@ -476,7 +450,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tma_b)) : "memory");
     for (int s = 0; s < C::STAGES; ++s) {
       mbar_init(full_bar + 8 * s, 1);
-      mbar_init(empty_bar + 8 * s, CM);      // one tcgen05.commit arrival from every CTA that reads the stage
+      mbar_init(empty_bar + 8 * s, 1);
     }
     for (int s = 0; s < 2; ++s) {
       mbar_init(tmem_full_bar + 8 * s, 1);
@@ -490,7 +464,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
   }
   tc_fence_before();
   __syncthreads();
-  if (CM > 1) cluster_sync_all();   // peers' barriers must be initialised before any multicast lands
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot_ptr;
 
@@ -501,20 +474,14 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
       uint32_t phase = 0;
       for (int unit = unit0; unit < num_units; unit += unit_stride) {
         int mg, nt;
-        unit_to_tile(unit, num_units / tiles_n, tiles_n, pw, mg, nt);
-        const int m0 = (mg * CM + (int)cta_rank) * BLOCK_M;
+        unit_to_tile(unit, tiles_m, tiles_n, pw, mg, nt);
+        const int m0 = mg * BLOCK_M;
         const int n0 = nt * BLOCK_N;
         for (int kb = 0; kb < num_kb; ++kb) {
           mbar_wait(empty_bar + 8 * stage, phase ^ 1);
           mbar_expect_tx(full_bar + 8 * stage, C::STAGE_BYTES);
           tma_load_2d(smem_a + stage * A_STAGE_BYTES, &tma_a, full_bar + 8 * stage, kb * O::KB, m0);
-          if (CM == 1) {
-            tma_load_2d(smem_b + stage * C::B_STAGE_BYTES, &tma_b, full_bar + 8 * stage, kb * O::KB, n0);
-          } else {   // my 1/CM slice of the W tile goes to every CTA of the cluster
-            constexpr int SLICE = BLOCK_N / CM;
-            tma_load_2d_mc(smem_b + stage * C::B_STAGE_BYTES + cta_rank * (SLICE * BLOCK_K * 2), &tma_b, full_bar + 8 * stage,
-                           kb * BLOCK_K, n0 + (int)cta_rank * SLICE, MC_MASK);
-          }
+          tma_load_2d(smem_b + stage * C::B_STAGE_BYTES, &tma_b, full_bar + 8 * stage, kb * O::KB, n0);
           if (++stage == C::STAGES) { stage = 0; phase ^= 1; }
         }
       }
@@ -543,9 +510,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
             if constexpr (F8) umma_e4m3(tmem_d, ad, bd, idesc, (kb | k) != 0 ? 1u : 0u);
             else umma_bf16(tmem_d, ad, bd, idesc, (kb | k) != 0 ? 1u : 0u);
           }
-          // frees the smem slot (in every CTA whose multicast writes into it) once the MMAs above retire
-          if (CM == 1) umma_commit(empty_bar + 8 * stage);
-          else umma_commit_mc(empty_bar + 8 * stage, MC_MASK);
+          umma_commit(empty_bar + 8 * stage);   // frees the smem slot once the MMAs above retire
           if (kb == num_kb - 1) umma_commit(tmem_full_bar + 8 * acc);
           if (++stage == C::STAGES) { stage = 0; phase ^= 1; }
         }
@@ -559,8 +524,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
     for (int unit = unit0; unit < num_units; unit += unit_stride, ++it) {
       const int acc = it & 1;
       int mg, nt;
-      unit_to_tile(unit, num_units / tiles_n, tiles_n, pw, mg, nt);
-      const int m0 = (mg * CM + (int)cta_rank) * BLOCK_M;
+      unit_to_tile(unit, tiles_m, tiles_n, pw, mg, nt);
+      const int m0 = mg * BLOCK_M;
       const int n0 = nt * BLOCK_N;
       mbar_wait(tmem_full_bar + 8 * acc, (it >> 1) & 1);
       tc_fence_after();
@@ -589,7 +554,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant_
 
   tc_fence_before();
   __syncthreads();
-  if (CM > 1) cluster_sync_all();   // no CTA may exit while a peer can still multicast into it / arrive on its barriers
   if (warp == 1) {
     tc_fence_after();
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(C::TMEM_COLS) : "memory");
@@ -624,10 +588,9 @@ __device__ __forceinline__ void tma_load_2d_pair_hint(uint32_t dst, const CUtens
       "l"(reinterpret_cast<uint64_t>(map)), "r"(leader_bar), "r"(c0), "r"(c1), "l"(policy)
       : "memory");
 }
-__device__ __forceinline__ uint64_t l2_policy(int kind) {   // 0 normal, 1 evict_last, 2 evict_first
+__device__ __forceinline__ uint64_t l2_policy(bool evict_last) {   // evict_last, or evict_normal
   uint64_t p;
-  if (kind == 1) asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
-  else if (kind == 2) asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
+  if (evict_last) asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
   else asm volatile("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(p));
   return p;
 }
@@ -735,8 +698,8 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_cons
     // ===================== TMA producer (both CTAs) =====================
     if (lane == 0) {
       const uint32_t leader_full = mapa_shared(full_bar, 0);
-      const bool hinted = (flags & (L2_W_LAST | L2_A_FIRST)) != 0;
-      const uint64_t pol_w = l2_policy((flags & L2_W_LAST) ? 1 : 0), pol_a = l2_policy((flags & L2_A_FIRST) ? 2 : 0);
+      const bool hinted = (flags & L2_W_LAST) != 0;
+      const uint64_t pol_w = l2_policy(hinted), pol_a = l2_policy(false);
       int stage = 0;
       uint32_t phase = 0;
       for (int unit = unit0; unit < num_units; unit += unit_stride) {
@@ -746,17 +709,13 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_cons
         const int n0 = nt * BLOCK_N + (int)cta_rank * C::HALF_N;
         for (int kb = 0; kb < num_kb; ++kb) {
           mbar_wait(empty_bar + 8 * stage, phase ^ 1);
-          if (flags & DBG_NO_TMA) {
-            if (leader) mbar_arrive(full_bar + 8 * stage);
+          if (leader) mbar_expect_tx(full_bar + 8 * stage, 2 * C::STAGE_BYTES);
+          if (hinted) {
+            tma_load_2d_pair_hint(smem_a + stage * A_STAGE_BYTES, &tma_a, leader_full + 8 * stage, kb * O::KB, m0, pol_a);
+            tma_load_2d_pair_hint(smem_b + stage * C::B_STAGE_BYTES, &tma_b, leader_full + 8 * stage, kb * O::KB, n0, pol_w);
           } else {
-            if (leader) mbar_expect_tx(full_bar + 8 * stage, 2 * C::STAGE_BYTES);
-            if (hinted) {
-              tma_load_2d_pair_hint(smem_a + stage * A_STAGE_BYTES, &tma_a, leader_full + 8 * stage, kb * O::KB, m0, pol_a);
-              tma_load_2d_pair_hint(smem_b + stage * C::B_STAGE_BYTES, &tma_b, leader_full + 8 * stage, kb * O::KB, n0, pol_w);
-            } else {
-              tma_load_2d_pair(smem_a + stage * A_STAGE_BYTES, &tma_a, leader_full + 8 * stage, kb * O::KB, m0);
-              tma_load_2d_pair(smem_b + stage * C::B_STAGE_BYTES, &tma_b, leader_full + 8 * stage, kb * O::KB, n0);
-            }
+            tma_load_2d_pair(smem_a + stage * A_STAGE_BYTES, &tma_a, leader_full + 8 * stage, kb * O::KB, m0);
+            tma_load_2d_pair(smem_b + stage * C::B_STAGE_BYTES, &tma_b, leader_full + 8 * stage, kb * O::KB, n0);
           }
           if (++stage == C::STAGES) { stage = 0; phase ^= 1; }
         }
@@ -781,22 +740,13 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_cons
           const int ksteps = k_left >= O::KB ? O::KB / O::UK : (k_left + O::UK - 1) / O::UK;
           const uint32_t a_addr = smem_a + stage * A_STAGE_BYTES;
           const uint32_t b_addr = smem_b + stage * C::B_STAGE_BYTES;
-          if (flags & DBG_NO_MMA) {
-            mbar_arrive_remote(mapa_shared(empty_bar + 8 * stage, 0));
-            mbar_arrive_remote(mapa_shared(empty_bar + 8 * stage, 1));
-            if (kb == num_kb - 1) {
-              mbar_arrive_remote(mapa_shared(tmem_full_bar + 8 * acc, 0));
-              mbar_arrive_remote(mapa_shared(tmem_full_bar + 8 * acc, 1));
-            }
-          } else {
-            for (int k = 0; k < ksteps; ++k) {
-              const uint64_t ad = umma_smem_desc(a_addr + k * O::UK * O::ESZ), bd = umma_smem_desc(b_addr + k * O::UK * O::ESZ);
-              if constexpr (F8) umma_e4m3_pair(tmem_d, ad, bd, idesc, (kb | k) != 0 ? 1u : 0u);
-              else umma_bf16_pair(tmem_d, ad, bd, idesc, (kb | k) != 0 ? 1u : 0u);
-            }
-            umma_commit_pair(empty_bar + 8 * stage);
-            if (kb == num_kb - 1) umma_commit_pair(tmem_full_bar + 8 * acc);
+          for (int k = 0; k < ksteps; ++k) {
+            const uint64_t ad = umma_smem_desc(a_addr + k * O::UK * O::ESZ), bd = umma_smem_desc(b_addr + k * O::UK * O::ESZ);
+            if constexpr (F8) umma_e4m3_pair(tmem_d, ad, bd, idesc, (kb | k) != 0 ? 1u : 0u);
+            else umma_bf16_pair(tmem_d, ad, bd, idesc, (kb | k) != 0 ? 1u : 0u);
           }
+          umma_commit_pair(empty_bar + 8 * stage);
+          if (kb == num_kb - 1) umma_commit_pair(tmem_full_bar + 8 * acc);
           if (++stage == C::STAGES) { stage = 0; phase ^= 1; }
         }
       }
@@ -826,217 +776,45 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_cons
       }
       float ssq = 0.f;
       const int pos = ep.rope_cols > 0 ? m % ep.rope_L : 0;
-      if (!(flags & DBG_NO_EPI)) {
-        if (TMA_OUT) {
-          // this warp: accumulator columns [n0 + 64 chunk0, + 64) of rows [m0 + 32 quarter, + 32)
-          const int c_first = 2 * chunk0;
-          if (n0 + c_first * 32 < Nacc) {                       // warp-uniform
-            if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");   // the previous store has read the staging tile
-            __syncwarp();
+      if (TMA_OUT) {
+        // this warp: accumulator columns [n0 + 64 chunk0, + 64) of rows [m0 + 32 quarter, + 32)
+        const int c_first = 2 * chunk0;
+        if (n0 + c_first * 32 < Nacc) {                       // warp-uniform
+          if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");   // the previous store has read the staging tile
+          __syncwarp();
 #pragma unroll 1
-            for (int hh = 0; hh < 2; ++hh) {
-              const int c = c_first + hh;
-              if (n0 + c * 32 >= Nacc) break;
-              uint32_t r[32];
-              tmem_ld32(tmem_base + ((uint32_t)(quarter * 32) << 16) + acc * BLOCK_N + c * 32, r);
-              if constexpr (F8) scale_cols(r, ep.col_scale, n0 + c * 32, Nacc);
-              epilogue_chunk(ep, m, pos, n0 + c * 32, r, rs, flags, ssq, stage_row, hh, lane);
-            }
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            __syncwarp();
-            if (lane == 0) {
-              const int col_acc = n0 + c_first * 32;
-              tma_store_2d(&tma_o, my_stage, swiglu ? col_acc >> 1 : col_acc, m0 + quarter * 32);
-              asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-            }
-          }
-        } else {
-#pragma unroll 1
-          for (int c = chunk0; c < BLOCK_N / 32; c += NUM_EPI_WARPS / 4) {
-            if (n0 + c * 32 >= Nacc) break;   // warp-uniform
+          for (int hh = 0; hh < 2; ++hh) {
+            const int c = c_first + hh;
+            if (n0 + c * 32 >= Nacc) break;
             uint32_t r[32];
             tmem_ld32(tmem_base + ((uint32_t)(quarter * 32) << 16) + acc * BLOCK_N + c * 32, r);
             if constexpr (F8) scale_cols(r, ep.col_scale, n0 + c * 32, Nacc);
-            epilogue_chunk(ep, m, pos, n0 + c * 32, r, rs, flags, ssq);
+            epilogue_chunk(ep, m, pos, n0 + c * 32, r, rs, flags, ssq, stage_row, hh, lane);
+          }
+          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+          __syncwarp();
+          if (lane == 0) {
+            const int col_acc = n0 + c_first * 32;
+            tma_store_2d(&tma_o, my_stage, swiglu ? col_acc >> 1 : col_acc, m0 + quarter * 32);
+            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
           }
         }
-        if (ep.sumsq_out && m < M) sumsq_add(ep.sumsq_out + remap_row(ep.remap_gi, ep.remap_go, ep.remap_off, m), ssq);
-        if ((flags & DBG_NO_STORE) && ssq == 123456.789f) reinterpret_cast<float*>(ep.out)[0] = ssq;   // keeps the ablated math alive
-      }
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive_remote(leader_tmem_empty + 8 * acc);
-    }
-    if (TMA_OUT && lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");     // stores complete before the CTA retires
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  if (warp == 1) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(C::TMEM_COLS) : "memory");
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// Quad variant: a 4-CTA cluster = TWO CTA pairs on vertically adjacent 256-row tiles that share the W tile.  Each CTA stages its
-// own 128 rows of A and ONE QUARTER (64 rows) of the W tile, which TMA multicasts into the same-rank CTA of the other pair, so an
-// SM fetches 24 KB per k-block from L2 instead of 32 KB (the L2 -> SM path is the largest data-movement energy term of the
-// power-capped mainloop).  A stage is released only when BOTH pairs' MMAs have read it (empty barriers count 2, commits are
-// multicast to all four CTAs); everything else is the pair kernel.
-// ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void tma_load_2d_pair_mc(uint32_t dst, const CUtensorMap* map, uint32_t leader_bar, int c0, int c1, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;" ::"r"(dst),
-      "l"(reinterpret_cast<uint64_t>(map)), "r"(leader_bar), "r"(c0), "r"(c1), "h"(mask)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit_pair_mask(uint32_t bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar), "h"(mask)
-               : "memory");
-}
-constexpr uint32_t PEER_BIT_MASK = 0xFEFFFFFFu;   // shared::cta address with the CTA-in-pair bit cleared = the pair leader's copy
-
-template <int BLOCK_N>
-__global__ void __launch_bounds__(NUM_THREADS, 1)
-gemm_tc_quad_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b, EpilogueParams ep,
-                    int M, int Nacc, int K, int flags) {
-  using C = PairCfg<BLOCK_N>;
-  constexpr int PAIR_M = 2 * BLOCK_M, QUAD_M = 4 * BLOCK_M, QUARTER_N = BLOCK_N / 4;
-  const uint32_t rank4 = cluster_ctarank();
-  const uint32_t pr = rank4 >> 1, r = rank4 & 1;     // pair within the cluster, rank within the pair
-  const bool leader = r == 0;
-  extern __shared__ uint8_t smem_raw[];
-  const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  const uint32_t smem_a = smem_base;
-  const uint32_t smem_b = smem_base + C::STAGES * A_STAGE_BYTES;
-  const uint32_t bars = smem_base + C::STAGES * C::STAGE_BYTES;
-  const uint32_t full_bar = bars;
-  const uint32_t empty_bar = bars + 8 * C::STAGES;
-  const uint32_t tmem_full_bar = bars + 16 * C::STAGES;
-  const uint32_t tmem_empty_bar = tmem_full_bar + 16;
-  const uint32_t tmem_slot = tmem_empty_bar + 16;
-  uint32_t* tmem_slot_ptr = reinterpret_cast<uint32_t*>(smem_raw + (tmem_slot - smem_u32(smem_raw)));
-
-  const int warp = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
-  const int tiles_n = (Nacc + BLOCK_N - 1) / BLOCK_N;
-  const int tiles_m = (M + QUAD_M - 1) / QUAD_M;
-  const int num_units = tiles_m * tiles_n;
-  const int unit0 = blockIdx.x >> 2, unit_stride = gridDim.x >> 2;
-  const int num_kb = (K + BLOCK_K - 1) / BLOCK_K;
-  const int pw = (flags >> PANEL_SHIFT) > 0 ? (flags >> PANEL_SHIFT) : tiles_n;   // n-tiles per L2-resident panel of W
-  const uint16_t pair_mask = (uint16_t)(3u << (2 * pr));        // both CTAs of my pair
-  const uint16_t col_mask = (uint16_t)((1u << r) | (4u << r));   // the CTAs of both pairs that hold W half r
-
-  if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tma_a)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tma_b)) : "memory");
-    for (int s = 0; s < C::STAGES; ++s) {
-      mbar_init(full_bar + 8 * s, 1);
-      mbar_init(empty_bar + 8 * s, 2);        // one commit from each pair's MMA thread
-    }
-    for (int s = 0; s < 2; ++s) {
-      mbar_init(tmem_full_bar + 8 * s, 1);
-      mbar_init(tmem_empty_bar + 8 * s, 2 * NUM_EPI_WARPS);
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(C::TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot_ptr;
-
-  if (warp == 0) {
-    // ===================== TMA producer (all four CTAs) =====================
-    if (lane == 0) {
-      const uint32_t leader_full = full_bar & PEER_BIT_MASK;
-      int stage = 0;
-      uint32_t phase = 0;
-      for (int unit = unit0; unit < num_units; unit += unit_stride) {
-        int mg, nt;
-        unit_to_tile(unit, tiles_m, tiles_n, pw, mg, nt);
-        const int m0 = mg * QUAD_M + (int)pr * PAIR_M + (int)r * BLOCK_M;
-        const int n0 = nt * BLOCK_N + (int)r * C::HALF_N + (int)pr * QUARTER_N;   // my quarter of the W tile
-        for (int kb = 0; kb < num_kb; ++kb) {
-          mbar_wait(empty_bar + 8 * stage, phase ^ 1);
-          if (leader) mbar_expect_tx(full_bar + 8 * stage, 2 * C::STAGE_BYTES);
-          tma_load_2d_pair(smem_a + stage * A_STAGE_BYTES, &tma_a, leader_full + 8 * stage, kb * BLOCK_K, m0);
-          tma_load_2d_pair_mc(smem_b + stage * C::B_STAGE_BYTES + pr * (QUARTER_N * BLOCK_K * 2), &tma_b, leader_full + 8 * stage, kb * BLOCK_K, n0,
-                              col_mask);
-          if (++stage == C::STAGES) { stage = 0; phase ^= 1; }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ===================== MMA issuer (the leader CTA of each pair) =====================
-    if (leader && lane == 0) {
-      constexpr uint32_t idesc = umma_idesc(PAIR_M, BLOCK_N);
-      int stage = 0;
-      uint32_t phase = 0;
-      int it = 0;
-      for (int unit = unit0; unit < num_units; unit += unit_stride, ++it) {
-        const int acc = it & 1;
-        mbar_wait(tmem_empty_bar + 8 * acc, ((it >> 1) & 1) ^ 1);
-        tc_fence_after();
-        const uint32_t tmem_d = tmem_base + acc * BLOCK_N;
-        for (int kb = 0; kb < num_kb; ++kb) {
-          mbar_wait(full_bar + 8 * stage, phase);
-          tc_fence_after();
-          const int k_left = K - kb * BLOCK_K;
-          const int ksteps = k_left >= BLOCK_K ? BLOCK_K / UMMA_K : (k_left + UMMA_K - 1) / UMMA_K;
-          const uint32_t a_addr = smem_a + stage * A_STAGE_BYTES;
-          const uint32_t b_addr = smem_b + stage * C::B_STAGE_BYTES;
-          for (int k = 0; k < ksteps; ++k) {
-            umma_bf16_pair(tmem_d, umma_smem_desc(a_addr + k * UMMA_K * 2), umma_smem_desc(b_addr + k * UMMA_K * 2), idesc,
-                           (kb | k) != 0 ? 1u : 0u);
-          }
-          umma_commit_pair_mask(empty_bar + 8 * stage, (uint16_t)0xF);       // the stage is also written by the other pair's producers
-          if (kb == num_kb - 1) umma_commit_pair_mask(tmem_full_bar + 8 * acc, pair_mask);
-          if (++stage == C::STAGES) { stage = 0; phase ^= 1; }
-        }
-      }
-    }
-  } else {
-    // ===================== epilogue (warps 2.., every CTA drains its own 128 rows) =====================
-    const int quarter = warp & 3;
-    const int chunk0 = (warp - 2) >> 2;
-    const uint32_t leader_tmem_empty = mapa_shared(tmem_empty_bar, 2 * pr);
-    int it = 0;
-    for (int unit = unit0; unit < num_units; unit += unit_stride, ++it) {
-      const int acc = it & 1;
-      int mg, nt;
-      unit_to_tile(unit, tiles_m, tiles_n, pw, mg, nt);
-      const int m0 = mg * QUAD_M + (int)pr * PAIR_M + (int)r * BLOCK_M;
-      const int n0 = nt * BLOCK_N;
-      mbar_wait(tmem_full_bar + 8 * acc, (it >> 1) & 1);
-      tc_fence_after();
-      const int m = m0 + quarter * 32 + lane;
-      float rs = 1.f;
-      if (m < M) {
-        if (ep.row_scale) rs = __ldg(ep.row_scale + m);
-        else if (ep.row_sumsq) rs = sumsq_rstd(ep.row_sumsq + m, ep.ss_inv, ep.ss_eps);
-      }
-      float ssq = 0.f;
-      const int pos = ep.rope_cols > 0 ? m % ep.rope_L : 0;
+      } else {
 #pragma unroll 1
-      for (int c = chunk0; c < BLOCK_N / 32; c += NUM_EPI_WARPS / 4) {
-        if (n0 + c * 32 >= Nacc) break;   // warp-uniform
-        uint32_t rr[32];
-        tmem_ld32(tmem_base + ((uint32_t)(quarter * 32) << 16) + acc * BLOCK_N + c * 32, rr);
-        epilogue_chunk(ep, m, pos, n0 + c * 32, rr, rs, flags, ssq);
+        for (int c = chunk0; c < BLOCK_N / 32; c += NUM_EPI_WARPS / 4) {
+          if (n0 + c * 32 >= Nacc) break;   // warp-uniform
+          uint32_t r[32];
+          tmem_ld32(tmem_base + ((uint32_t)(quarter * 32) << 16) + acc * BLOCK_N + c * 32, r);
+          if constexpr (F8) scale_cols(r, ep.col_scale, n0 + c * 32, Nacc);
+          epilogue_chunk(ep, m, pos, n0 + c * 32, r, rs, flags, ssq);
+        }
       }
       if (ep.sumsq_out && m < M) sumsq_add(ep.sumsq_out + remap_row(ep.remap_gi, ep.remap_go, ep.remap_off, m), ssq);
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive_remote(leader_tmem_empty + 8 * acc);
     }
+    if (TMA_OUT && lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");     // stores complete before the CTA retires
   }
 
   tc_fence_before();
@@ -1121,8 +899,8 @@ gemm_tc_wide_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_cons
     // ===================== TMA producer (both CTAs) =====================
     if (lane == 0) {
       const uint32_t leader_full = mapa_shared(full_bar, 0);
-      const bool hinted = (flags & (L2_W_LAST | L2_A_FIRST)) != 0;
-      const uint64_t pol_w = l2_policy((flags & L2_W_LAST) ? 1 : 0), pol_a = l2_policy((flags & L2_A_FIRST) ? 2 : 0);
+      const bool hinted = (flags & L2_W_LAST) != 0;
+      const uint64_t pol_w = l2_policy(hinted), pol_a = l2_policy(false);
       int stage = 0;
       uint32_t phase = 0;
       for (int unit = unit0; unit < num_units; unit += unit_stride) {
@@ -1284,18 +1062,6 @@ static int make_map(CUtensorMap* map, const void* base, int rows, int cols, int 
   return TCAVP_OK;
 }
 
-// TCAVP_GEMM_CLUSTER (A/B testing): 1 = no clusters, 2 = 2-CTA clusters with TMA multicast of W, 3 = CTA pairs (cta_group::2, default),
-// 4 = two CTA pairs per 4-CTA cluster sharing the W tile through TMA multicast
-static int cluster_pref() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("TCAVP_GEMM_CLUSTER");
-    v = e ? atoi(e) : 3;
-    if (v < 1 || v > 4) v = 3;
-  }
-  return v;
-}
-
 // Vector-path switches of the epilogue: 256-bit output / residual accesses need 32-byte aligned rows, the bias loads 16-byte alignment.
 static int epilogue_flags(const EpilogueParams& ep) {
   const size_t osz = ep.out_dtype == TCAVP_BF16 ? 2 : 4, rsz = ep.res_dtype == TCAVP_BF16 ? 2 : 4;
@@ -1307,27 +1073,21 @@ static int epilogue_flags(const EpilogueParams& ep) {
 }
 
 // Panel width (n-tiles) of the persistent tile order + L2 hints, packed into the kernel's flags (see unit_to_tile).
-// A panel of W is sized to stay in L2 (TCAVP_GEMM_PANEL_MB, default 40 of the 126 MB; loaded evict_last) while A streams past it.
+// A panel of W is sized to stay in L2 (40 of the 126 MB; loaded evict_last) while A streams past it.
 // Modelled DRAM reads: W + A x panels with panels, A + (W rows one wave of resident units touches) x waves without (ncu: without
-// evict_last even a 33 MB W is re-streamed by most waves) - the smaller one decides.  TCAVP_GEMM_L2HINT: 0 none, 1 W evict_last,
-// 2 also A evict_first, 3 (default) W evict_last + streaming (evict_first) output stores.
+// evict_last even a 33 MB W is re-streamed by most waves) - the smaller one decides.  The hints (pair and wide kernels): W evict_last,
+// and streaming (evict_first) stores for outputs larger than 256 MB.
 static int panel_flags(long long M, long long N, long long K, int unit_m, int tile_n, int resident_units, bool can_hint) {
-  static long long budget = -1;
-  static int hint = -1, force = 0;
-  if (budget < 0) {
-    const char* e = getenv("TCAVP_GEMM_L2HINT");
-    hint = e ? atoi(e) : 3;
-    e = getenv("TCAVP_GEMM_PANEL_FORCE");      // test hook: this many n-tiles per panel whatever the problem size
-    force = e ? atoi(e) : 0;
-    e = getenv("TCAVP_GEMM_PANEL_MB");
-    budget = (e ? atoll(e) : 40) << 20;
-  }
-  if (force > 0 && force <= 0x7fff) return (force << PANEL_SHIFT) | (can_hint && hint > 0 ? L2_W_LAST : 0);
+  constexpr long long budget = 40ll << 20;
+  static const int force = [] {      // test hook: this many n-tiles per panel whatever the problem size
+    const char* e = getenv("TCAVP_GEMM_PANEL_FORCE");
+    return e ? atoi(e) : 0;
+  }();
+  if (force > 0 && force <= 0x7fff) return (force << PANEL_SHIFT) | (can_hint ? L2_W_LAST : 0);
   const long long w_bytes = N * K * 2, a_bytes = M * K * 2;
   // streaming stores only for outputs the next kernel cannot find in L2 anyway (> 2 x L2 of bf16)
   const int out_first = M * N * 2 > (256ll << 20) ? L2_OUT_FIRST : 0;
-  const int hint_flags = !can_hint || hint <= 0 ? 0 : (hint == 2 ? (L2_W_LAST | L2_A_FIRST) : hint >= 3 ? (L2_W_LAST | out_first) : L2_W_LAST);
-  if (budget <= 0) return 0;
+  const int hint_flags = can_hint ? (L2_W_LAST | out_first) : 0;
   if (w_bytes <= budget) return w_bytes * 4 > budget ? hint_flags : 0;     // whole W is one resident panel (tiny W: nothing to protect)
   const long long tiles_n = (N + tile_n - 1) / tile_n, tiles_m = (M + unit_m - 1) / unit_m;
   long long pw = budget / ((long long)tile_n * K * 2);
@@ -1342,25 +1102,26 @@ static int panel_flags(long long M, long long N, long long K, int unit_m, int ti
   return ((int)pw << PANEL_SHIFT) | hint_flags;
 }
 
-// tcavp_last_kernel() names of the e4m3 forms (the bf16 launches keep their plain kernel names)
-template <int BLOCK_N> constexpr const char* e4m3_name() {
-  return BLOCK_N == 32 ? "gemm_tc_kernel<32,e4m3>" : BLOCK_N == 64 ? "gemm_tc_kernel<64,e4m3>" : BLOCK_N == 128 ? "gemm_tc_kernel<128,e4m3>"
-                                                                                                             : "gemm_tc_kernel<256,e4m3>";
+// tcavp_last_kernel() name of a single-CTA form: the template shape, and the operand type for e4m3
+template <int BLOCK_N, bool F8> constexpr const char* tc_name() {
+  if (F8) return BLOCK_N == 32 ? "gemm_tc_kernel<32,e4m3>" : BLOCK_N == 64 ? "gemm_tc_kernel<64,e4m3>" : BLOCK_N == 128 ? "gemm_tc_kernel<128,e4m3>"
+                                                                                                                     : "gemm_tc_kernel<256,e4m3>";
+  return BLOCK_N == 32 ? "gemm_tc_kernel<32>" : BLOCK_N == 64 ? "gemm_tc_kernel<64>" : BLOCK_N == 128 ? "gemm_tc_kernel<128>" : "gemm_tc_kernel<256>";
 }
 
-template <int BLOCK_N, int CM, bool F8 = false>
+template <int BLOCK_N, bool F8 = false>
 static int launch_tc(const tcavp_gemm_args& a, const EpilogueParams& ep, cudaStream_t stream) {
   using C = Cfg<BLOCK_N>;
   CUtensorMap ma, mb;
   int rc = make_map(&ma, a.A, a.M, a.K, a.lda, BLOCK_M, F8);
   if (rc) return rc;
-  rc = make_map(&mb, a.W, a.N, a.K, a.ldw, BLOCK_N / CM, F8);
+  rc = make_map(&mb, a.W, a.N, a.K, a.ldw, BLOCK_N, F8);
   if (rc) return rc;
-  TCAVP_CUDA(cudaFuncSetAttribute(gemm_tc_kernel<BLOCK_N, CM, F8>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
+  TCAVP_CUDA(cudaFuncSetAttribute(gemm_tc_kernel<BLOCK_N, F8>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
   const int tiles_m = (a.M + BLOCK_M - 1) / BLOCK_M, tiles_n = (a.N + BLOCK_N - 1) / BLOCK_N;
-  const int units = ((tiles_m + CM - 1) / CM) * tiles_n;
-  const int max_clusters = sm_count() / CM;
-  const int grid = (units < max_clusters ? units : max_clusters) * CM;
+  const int units = tiles_m * tiles_n;
+  const int max_ctas = sm_count();
+  const int grid = units < max_ctas ? units : max_ctas;
   int flags = epilogue_flags(ep);
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(grid);
@@ -1369,26 +1130,14 @@ static int launch_tc(const tcavp_gemm_args& a, const EpilogueParams& ep, cudaStr
   cfg.stream = stream;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CM;
+  attr[0].val.clusterDim.x = 1;
   attr[0].val.clusterDim.y = 1;
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  flags |= panel_flags(a.M, a.N, a.K, BLOCK_M * CM, BLOCK_N, max_clusters, false);
-  TCAVP_CUDA(cudaLaunchKernelEx(&cfg, gemm_tc_kernel<BLOCK_N, CM, F8>, ma, mb, ep, a.M, a.N, a.K, flags));
-  return check_launch(F8 ? e4m3_name<BLOCK_N>() : "gemm_tc_kernel");
-}
-
-// TCAVP_GEMM_TMASTORE: 1 (default) = bf16 outputs leave through shared memory + TMA stores (pair kernel), 0 = 256-bit global stores.
-// Measured A/B on B200 (profiles/gemm_tmastore_ab_r02.txt): within +-1 % of each other on the K = 768 shapes — the kernel runs at the
-// 1 kW cap either way; the TMA form is kept as the default because it frees the epilogue warps' LSU work and writes whole lines.
-static int tma_store_pref() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("TCAVP_GEMM_TMASTORE");
-    v = e ? atoi(e) : 1;
-  }
-  return v;
+  flags |= panel_flags(a.M, a.N, a.K, BLOCK_M, BLOCK_N, max_ctas, false);
+  TCAVP_CUDA(cudaLaunchKernelEx(&cfg, gemm_tc_kernel<BLOCK_N, F8>, ma, mb, ep, a.M, a.N, a.K, flags));
+  return check_launch(tc_name<BLOCK_N, F8>());
 }
 
 // [rows, cols] bf16 output view for the TMA-store epilogue: box = 32 rows x box_cols (64: SWIZZLE_128B, 32: SWIZZLE_64B)
@@ -1414,8 +1163,10 @@ static int make_out_map(CUtensorMap* map, void* base, int rows, int cols, int ld
 
 template <int BLOCK_N, bool F8 = false>
 static int launch_tc_pair(const tcavp_gemm_args& a, const EpilogueParams& ep, cudaStream_t stream) {
-  // TMA-store epilogue: bf16 output rows in place (no row remap), 16-byte aligned rows, not the SwiGLU-backward form
-  const bool tma_out = tma_store_pref() && ep.out_dtype == TCAVP_BF16 && ep.remap_gi == 0 && ep.act != TCAVP_ACT_SWIGLU_BWD &&
+  // TMA-store epilogue: bf16 output rows in place (no row remap), 16-byte aligned rows, not the SwiGLU-backward form.  Measured on
+  // B200 (profiles/gemm_tmastore_ab_r02.txt) within +-1 % of the 256-bit global stores on the K = 768 shapes; it frees the epilogue
+  // warps' LSU work and writes whole lines.
+  const bool tma_out = ep.out_dtype == TCAVP_BF16 && ep.remap_gi == 0 && ep.act != TCAVP_ACT_SWIGLU_BWD &&
                        (ep.ldo % 8) == 0 && reinterpret_cast<uintptr_t>(ep.out) % 16 == 0;
   CUtensorMap ma, mb, mo;
   int rc = make_map(&ma, a.A, a.M, a.K, a.lda, BLOCK_M, F8);
@@ -1437,7 +1188,6 @@ static int launch_tc_pair(const tcavp_gemm_args& a, const EpilogueParams& ep, cu
   const int grid = (units < max_pairs ? units : max_pairs) * 2;
   int flags = epilogue_flags(ep);
   if (tma_out) flags |= EPI_TMA_OUT;
-  if (const char* e = getenv("TCAVP_GEMM_DEBUG")) flags |= atoi(e) & (DBG_NO_TMA | DBG_NO_MMA | DBG_NO_EPI | DBG_NO_STORE);
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(grid);
   cfg.blockDim = dim3(NUM_THREADS);
@@ -1453,59 +1203,13 @@ static int launch_tc_pair(const tcavp_gemm_args& a, const EpilogueParams& ep, cu
   flags |= panel_flags(a.M, a.N, a.K, 2 * BLOCK_M, BLOCK_N, max_pairs, true);
   if (tma_out) TCAVP_CUDA(cudaLaunchKernelEx(&cfg, gemm_tc_pair_kernel<BLOCK_N, true, F8>, ma, mb, mo, ep, a.M, a.N, a.K, flags));
   else TCAVP_CUDA(cudaLaunchKernelEx(&cfg, gemm_tc_pair_kernel<BLOCK_N, false, F8>, ma, mb, mo, ep, a.M, a.N, a.K, flags));
-  return check_launch(F8 ? "gemm_tc_pair_kernel<256,e4m3>" : "gemm_tc_pair_kernel");
+  return check_launch(F8 ? "gemm_tc_pair_kernel<256,e4m3>" : "gemm_tc_pair_kernel<256>");
 }
 
-template <int BLOCK_N>
-static int launch_tc_quad(const tcavp_gemm_args& a, const EpilogueParams& ep, cudaStream_t stream) {
-  using C = PairCfg<BLOCK_N>;
-  CUtensorMap ma, mb;
-  int rc = make_map(&ma, a.A, a.M, a.K, a.lda, BLOCK_M);
-  if (rc) return rc;
-  rc = make_map(&mb, a.W, a.N, a.K, a.ldw, BLOCK_N / 4);
-  if (rc) return rc;
-  TCAVP_CUDA(cudaFuncSetAttribute(gemm_tc_quad_kernel<BLOCK_N>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
-  TCAVP_CUDA(cudaFuncSetAttribute(gemm_tc_quad_kernel<BLOCK_N>, cudaFuncAttributeNonPortableClusterSizeAllowed, 0));
-  const int tiles_m = (a.M + 4 * BLOCK_M - 1) / (4 * BLOCK_M), tiles_n = (a.N + BLOCK_N - 1) / BLOCK_N;
-  const int units = tiles_m * tiles_n;
-  cudaLaunchConfig_t cfg = {};
-  cfg.blockDim = dim3(NUM_THREADS);
-  cfg.dynamicSmemBytes = C::SMEM_BYTES;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 4;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  static int max_quads = 0;       // co-resident 4-CTA clusters (GPC boundaries may leave a few SMs unused)
-  if (max_quads == 0) {
-    cfg.gridDim = dim3(sm_count() / 4 * 4);
-    int n = 0;
-    if (cudaOccupancyMaxActiveClusters(&n, gemm_tc_quad_kernel<BLOCK_N>, &cfg) != cudaSuccess || n <= 0) n = sm_count() / 4 - 2;
-    max_quads = n;
-  }
-  const int grid = (units < max_quads ? units : max_quads) * 4;
-  cfg.gridDim = dim3(grid);
-  int flags = epilogue_flags(ep);
-  flags |= panel_flags(a.M, a.N, a.K, 4 * BLOCK_M, BLOCK_N, max_quads, false);
-  TCAVP_CUDA(cudaLaunchKernelEx(&cfg, gemm_tc_quad_kernel<BLOCK_N>, ma, mb, ep, a.M, a.N, a.K, flags));
-  return check_launch("gemm_tc_quad_kernel");
-}
-
-// TCAVP_GEMM_WIDE_SPLIT: k-blocks at the head and tail of a tile that the wide kernel issues half-major (1 = plain k-major order).
+// k-blocks at the head and tail of a tile that the wide kernel issues half-major (1 would be plain k-major order).
 // Measured on B200 (profiles/wide_split_ab_r02v.txt, same box, A-B-A-B): K = 3072 down_proj 775 -> 766 us, 7B o_proj 1263 -> 1258 us with 4;
 // on K = 768 the wide tile gains 13 % from it (gate/up 844 -> 954 TF/s) but the double-buffered pair kernel stays ahead (1041 TF/s).
-static int wide_split() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("TCAVP_GEMM_WIDE_SPLIT");
-    v = e ? atoi(e) : 4;
-    if (v < 1) v = 1;
-  }
-  return v;
-}
+constexpr int WIDE_SPLIT = 4;
 
 static int launch_tc_wide(const tcavp_gemm_args& a, const EpilogueParams& ep, cudaStream_t stream) {
   using C = WideCfg;
@@ -1533,7 +1237,7 @@ static int launch_tc_wide(const tcavp_gemm_args& a, const EpilogueParams& ep, cu
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   flags |= panel_flags(a.M, a.N, a.K, 4 * BLOCK_M, C::BLOCK_N, max_pairs, true);
-  TCAVP_CUDA(cudaLaunchKernelEx(&cfg, gemm_tc_wide_kernel, ma, mb, ep, a.M, a.N, a.K, flags, wide_split()));
+  TCAVP_CUDA(cudaLaunchKernelEx(&cfg, gemm_tc_wide_kernel, ma, mb, ep, a.M, a.N, a.K, flags, WIDE_SPLIT));
   return check_launch("gemm_tc_wide_kernel");
 }
 
@@ -1776,18 +1480,17 @@ extern "C" int tcavp_gemm(const tcavp_gemm_args* a, tcavp_stream_t stream_) {
   if (a->in_dtype == TCAVP_BF16) {
     TCAVP_REQUIRE(a->K % 8 == 0 && a->lda % 8 == 0 && a->ldw % 8 == 0, "tcavp_gemm(bf16): K, lda, ldw must be multiples of 8 (K=%d lda=%d ldw=%d)", a->K, a->lda, a->ldw);
     TCAVP_REQUIRE(reinterpret_cast<uintptr_t>(a->A) % 16 == 0 && reinterpret_cast<uintptr_t>(a->W) % 16 == 0, "tcavp_gemm(bf16): A and W must be 16-byte aligned");
-    if (a->N <= 32) return tc::launch_tc<32, 1>(*a, ep, stream);
-    if (a->N <= 64) return tc::launch_tc<64, 1>(*a, ep, stream);
-    if (a->N <= 128) return tc::launch_tc<128, 1>(*a, ep, stream);
-    // large problems: CTA pairs (one 256 x 256 tile per TPC), or 2-CTA clusters sharing the W tile through TMA multicast
-    // wide tile: long contraction AND at least ~4 waves of 512 x 256 tiles (coarser tiles quantise worse on mid-size problems)
-    if (tc::cluster_pref() >= 3 && tc::wide_min_k() > 0 && a->K >= tc::wide_min_k() && a->M >= 64 * tc::BLOCK_M &&
+    if (a->N <= 32) return tc::launch_tc<32>(*a, ep, stream);
+    if (a->N <= 64) return tc::launch_tc<64>(*a, ep, stream);
+    if (a->N <= 128) return tc::launch_tc<128>(*a, ep, stream);
+    // large problems: CTA pairs (one 256 x 256 tile per TPC)
+    // wide tile: long contraction AND at least ~4 waves of 512 x 256 tiles (coarser tiles quantise worse on mid-size problems).
+    // ops.py's _long_k_gemm mirrors this condition to autotune the wide-vs-pair choice before the first such GEMM.
+    if (tc::wide_min_k() > 0 && a->K >= tc::wide_min_k() && a->M >= 64 * tc::BLOCK_M &&
         (long long)((a->M + 511) / 512) * ((a->N + 255) / 256) >= 4LL * (sm_count() / 2))
       return tc::launch_tc_wide(*a, ep, stream);
-    if (tc::cluster_pref() == 4 && a->M >= 32 * tc::BLOCK_M) return tc::launch_tc_quad<256>(*a, ep, stream);
-    if (tc::cluster_pref() >= 3 && a->M >= 16 * tc::BLOCK_M) return tc::launch_tc_pair<256>(*a, ep, stream);
-    if (tc::cluster_pref() == 2 && a->M >= 16 * tc::BLOCK_M) return tc::launch_tc<256, 2>(*a, ep, stream);
-    return tc::launch_tc<256, 1>(*a, ep, stream);
+    if (a->M >= 16 * tc::BLOCK_M) return tc::launch_tc_pair<256>(*a, ep, stream);
+    return tc::launch_tc<256>(*a, ep, stream);
   }
   if (a->in_dtype == TCAVP_E4M3) {
     TCAVP_REQUIRE(a->col_scale && reinterpret_cast<uintptr_t>(a->col_scale) % 16 == 0, "tcavp_gemm(e4m3): needs a 16-byte aligned col_scale");
@@ -1796,11 +1499,11 @@ extern "C" int tcavp_gemm(const tcavp_gemm_args* a, tcavp_stream_t stream_) {
     TCAVP_REQUIRE(reinterpret_cast<uintptr_t>(a->A) % 16 == 0 && reinterpret_cast<uintptr_t>(a->W) % 16 == 0, "tcavp_gemm(e4m3): A and W must be 16-byte aligned");
     TCAVP_REQUIRE(!a->row_sumsq && !a->sumsq_out && !a->aux_out && a->act != TCAVP_ACT_SWIGLU_BWD,
                   "tcavp_gemm(e4m3): row_sumsq, sumsq_out, aux_out and SWIGLU_BWD are bf16-only epilogues");
-    if (a->N <= 32) return tc::launch_tc<32, 1, true>(*a, ep, stream);
-    if (a->N <= 64) return tc::launch_tc<64, 1, true>(*a, ep, stream);
-    if (a->N <= 128) return tc::launch_tc<128, 1, true>(*a, ep, stream);
-    if (tc::cluster_pref() >= 3 && a->M >= 16 * tc::BLOCK_M) return tc::launch_tc_pair<256, true>(*a, ep, stream);
-    return tc::launch_tc<256, 1, true>(*a, ep, stream);
+    if (a->N <= 32) return tc::launch_tc<32, true>(*a, ep, stream);
+    if (a->N <= 64) return tc::launch_tc<64, true>(*a, ep, stream);
+    if (a->N <= 128) return tc::launch_tc<128, true>(*a, ep, stream);
+    if (a->M >= 16 * tc::BLOCK_M) return tc::launch_tc_pair<256, true>(*a, ep, stream);
+    return tc::launch_tc<256, true>(*a, ep, stream);
   }
   if (a->in_dtype == TCAVP_F32) {
     const long long t64 = (long long)((a->N + 63) / 64) * ((a->M + 63) / 64);

@@ -113,6 +113,8 @@ class LaunchProfiler:
 
 
 class _Timed:
+    """Records one launch with the active LaunchProfiler.  `kernel` is the label, or, for entry points where the library picks the
+    kernel, a function of last_kernel() that returns (label, nbytes), called only while a profiler is active; None records nothing."""
     __slots__ = ("kernel", "flops", "nbytes", "e0")
 
     def __init__(self, kernel, flops=0.0, nbytes=0.0):
@@ -125,10 +127,11 @@ class _Timed:
         return self
 
     def __exit__(self, *a):
-        if _PROF is not None:
+        if _PROF is not None and self.kernel is not None:
             e1 = torch.cuda.Event(enable_timing=True)
             e1.record()
-            _PROF.add(self.kernel, self.flops, self.nbytes, self.e0, e1)
+            kernel, nbytes = (self.kernel, self.nbytes) if isinstance(self.kernel, str) else self.kernel(last_kernel())
+            _PROF.add(kernel, self.flops, nbytes, self.e0, e1)
 
 
 def _nb(*ts):
@@ -161,6 +164,13 @@ def _need_cuda(*ts):
 # wide is 6-15 % ahead on some B200s, the pair tile 6-12 % ahead on others of the same pool and power cap (profiles/wide_vs_pair_r02y.txt).
 # So the first long-K GEMM of a process times both for ~0.1 s each on this GPU and keeps the faster (TCAVP_GEMM_WIDE_K pins it instead).
 _ROUTE = {"wide_k": None, "tuned": None}
+
+
+def _long_k_gemm(M, N, K):
+    """True for the bf16 problems tcavp_gemm sends to the wide kernel when the threshold allows it: a long contraction and at least
+    four waves of 512 x 256 tiles on 148 SMs.  Must match the condition in tcavp_gemm (gemm.cu): it is the only routing decision
+    this module repeats, to run autotune_gemm_route() before the first such GEMM."""
+    return N > 128 and K >= 2048 and M >= 8192 and ((M + 511) // 512) * ((N + 255) // 256) >= 4 * 74
 
 
 def autotune_gemm_route(budget_ms=120.0):
@@ -262,26 +272,19 @@ def gemm(a, w, out, *, M=None, N=None, K=None, lda=None, ldw=None, ldo=None, bia
         if col_scale.dtype != torch.float32:
             raise TypeError("gemm: col_scale must be fp32")
         g.col_scale = col_scale.data_ptr()
-    if g.in_dtype == E4M3:   # mirrors tcavp_gemm's e4m3 dispatch (no wide / quad forms)
-        if g.N > 128 and g.M >= 2048:
-            kern = "gemm_tc_pair_kernel<256,e4m3>[%sN%d,K%d]" % ("M%d," % g.M if g.M < 32768 else "", g.N, g.K)
-        else:
-            kern = "gemm_tc_kernel<%d,e4m3>[N%d,K%d]" % (32 if g.N <= 32 else 64 if g.N <= 64 else 128 if g.N <= 128 else 256, g.N, g.K)
-    elif g.in_dtype == BF16:
-        long_k = g.N > 128 and g.K >= 2048 and g.M >= 8192 and ((g.M + 511) // 512) * ((g.N + 255) // 256) >= 4 * 74
-        if long_k and _ROUTE["wide_k"] is None:
-            autotune_gemm_route()
-        if long_k and _ROUTE["wide_k"] and g.K >= _ROUTE["wide_k"]:
-            kern = "gemm_tc_wide_kernel[N%d,K%d]" % (g.N, g.K)     # mirrors tcavp_gemm's dispatch (long contraction, >= 4 waves of tiles)
-        elif g.N > 128 and g.M >= 2048:    # CTA-pair (cta_group::2) kernel for the large problems
-            # small-M launches (the Q-Former's 16 query rows per scene) are reported apart from the token-stream launches of the same [N, K]
-            kern = "gemm_tc_pair_kernel<256>[%sN%d,K%d]" % ("M%d," % g.M if g.M < 32768 else "", g.N, g.K)
-        else:
-            kern = "gemm_tc_kernel<%d>[N%d,K%d]" % (32 if g.N <= 32 else 64 if g.N <= 64 else 128 if g.N <= 128 else 256, g.N, g.K)
-    else:
-        kern = "gemm_simt_kernel"
+    if g.in_dtype == BF16 and _ROUTE["wide_k"] is None and _long_k_gemm(g.M, g.N, g.K):
+        autotune_gemm_route()
     esz = a.element_size()
-    with _Timed(kern, 2.0 * g.M * g.N * g.K, float(g.M * g.K * esz + g.N * g.K * esz + g.M * g.N * out.element_size())):
+    nbytes = float(g.M * g.K * esz + g.N * g.K * esz + g.M * g.N * out.element_size())
+
+    def label(kern):
+        if kern == "gemm_simt_kernel":
+            return kern, nbytes
+        # small-M pair launches (the Q-Former's 16 query rows per scene) are reported apart from the token-stream launches of the same [N, K]
+        m = "M%d," % g.M if kern.startswith("gemm_tc_pair_kernel") and g.M < 32768 else ""
+        return "%s[%sN%d,K%d]" % (kern, m, g.N, g.K), nbytes
+
+    with _Timed(label if g.M > 0 else None, 2.0 * g.M * g.N * g.K):      # M = 0: tcavp_gemm checks the arguments and launches nothing
         _lib.check(_lib.load().tcavp_gemm(byref(g), _stream()), "tcavp_gemm")
     return out
 
@@ -302,27 +305,16 @@ def attention(q, k, v, out, *, B, H, Hkv, Tq, Tk, dh, q_strides, k_strides, v_st
             raise TypeError("attention: key_mask must be int32")
         a.key_mask = key_mask.data_ptr()
     _set_drop(a, drop)
-    shared_kv = False
-    if (a.dtype == BF16 and causal and dh in (64, 128) and Tq == Tk and 128 <= Tq <= 256 and not a.drop_thresh and q_strides[0] == Tq * q_strides[1]
-            and k_strides[0] == Tk * k_strides[1] and v_strides[0] == Tk * v_strides[1] and _os.environ.get("TCAVP_ATTN_TCGEN05", "1") != "0"):
-        kern = f"attn_tm_kernel[dh{dh},L{Tq}]"          # tcgen05 / TMEM / TMA (attention_tm.cu)
-    elif (a.dtype == BF16 and H == 2 and Hkv == 1 and k.data_ptr() == v.data_ptr() and tuple(k_strides) == tuple(v_strides) and not causal
-          and key_mask is None and not a.drop_thresh and Tq <= 64 and Tk <= 256 and dh % 128 == 0 and q_strides[0] == Tq * q_strides[1]
-          and k_strides[0] == Tk * k_strides[1] and _os.environ.get("TCAVP_ATTNX_TCGEN05", "1") != "0"):
-        kern = f"attn_xt_kernel[dh{dh},q{Tq},k{Tk}]"      # tcgen05: two heads on one shared K = V head (attention_xt.cu)
-        shared_kv = True
-    elif a.dtype == BF16 and dh in (16, 32, 64, 96, 128) and max(Tq, Tk) <= 256:
-        kern = f"attn_flash_kernel[dh{dh},q{Tq},k{Tk}]"
-    elif a.dtype == BF16 and dh > 128 and dh % 64 == 0 and Tq <= 64 and Tk <= 256 and not causal:
-        kern = "attn_x_kernel"
-    elif dh in (16, 32) and Tk <= 128:
-        kern = f"attn_row_kernel[dh{dh},q{Tq},k{Tk}]"
-    else:
-        kern = f"attn_warp_kernel[dh{dh},q{Tq},k{Tk}]"
     fl = 4.0 * B * H * Tq * Tk * dh * (0.5 if causal else 1.0)
-    # algorithmic bytes: q read + out written + k and v read once (ONE pass when the keys are the values)
-    nbytes = q.element_size() * B * dh * (2.0 * H * Tq + (1.0 if shared_kv else 2.0) * Hkv * Tk)
-    with _Timed(kern, fl, nbytes):
+
+    def label(kern):
+        # algorithmic bytes: q read + out written + k and v read once (ONE pass when the keys are the values: attn_xt_kernel)
+        nbytes = q.element_size() * B * dh * (2.0 * H * Tq + (1.0 if kern == "attn_xt_kernel" else 2.0) * Hkv * Tk)
+        if kern == "attn_tm_kernel":
+            return f"{kern}[dh{dh},L{Tq}]", nbytes
+        return (kern if kern == "attn_x_kernel" else f"{kern}[dh{dh},q{Tq},k{Tk}]"), nbytes
+
+    with _Timed(label if B > 0 and Tq > 0 else None, fl):      # an empty problem launches nothing
         _lib.check(_lib.load().tcavp_attention(byref(a), _stream()), "tcavp_attention")
     return out
 
