@@ -420,6 +420,55 @@ int tcavp_dropout(const void* in, int ldi, int in_dtype, const void* residual, i
                   long long rows, int cols, const uint32_t* seed, uint32_t site, uint32_t thresh, float scale, int accumulate,
                   tcavp_stream_t stream);
 
+/* ---- text generation on the device (reference scripts/train.py:577-654 -> HF generate(do_sample=True, ...) with past_key_values) -------
+ * Every entry point below reads the decode position from device memory, position = offset + *counter, and tcavp_sample_next advances
+ * the counter itself: one decode iteration captured in a CUDA graph stays correct over any number of replays. */
+
+/* One step of HF's logits-processor chain and the draw, one CTA per sequence.  logits fp32 [B, V] (row stride ld); work fp32 [B, V]
+ * receives the processed logits (removed tokens -inf: what generate.py process_logits returns); hist int64 [B, ld_hist] holds the
+ * prompt ids followed by the generated ones, n = hist_offset + state[0] of them valid.  In order:
+ *   repetition penalty over hist[0, n) (once per distinct token: s < 0 ? s * penalty : s / penalty of the raw logit; 1 = off);
+ *   no-repeat-n-gram (0 = off); do_sample: temperature, top-k (0 or >= V = off; values below the k-th largest removed, ties kept),
+ *   top-p (outside (0, 1) = off; a token is kept when the mass strictly above it is < top_p, so a tie group at the boundary is kept
+ *   whole; the largest is always kept);
+ *   do_sample: inverse-CDF draw over the kept tokens in ascending token id with integer weights w_i = floor(exp(x_i - max) * 2^40):
+ *     key = mix(seed[0] ^ mix(seed[1] + 0x9E3779B9)),  u = mix(mix(key ^ step) ^ (row * 0x85EBCA6B + 0x632BE5AB))   (mix: tcavp_dropout)
+ *     r = floor(u * W / 2^32), W = sum w_i;  token = the first i with sum_{j <= i} w_j > r     (step = state[0], row = sequence index)
+ *   else argmax of the processed logits, lowest index on ties.
+ * eos_token_id >= 0: a row whose done[b] is set emits pad_token_id, a row that emits eos sets done[b].  The token goes to hist[b, n]
+ * (when n < ld_hist) and tokens_out[b].  int state[3] = {step, 0, first step count at which every row was done (0 = not yet)}: the last
+ * CTA increments state[0] and fills state[2]; state[1] is its arrival counter and must be 0 between launches. */
+int tcavp_sample_next(const float* logits, long long ld, int B, int V, float* work, long long* hist, int ld_hist, int hist_offset, int* state,
+                      const uint32_t* seed, int do_sample, float temperature, int top_k, float top_p, float repetition_penalty,
+                      int no_repeat_ngram_size, long long eos_token_id, long long pad_token_id, int* done, long long* tokens_out,
+                      tcavp_stream_t stream);
+
+/* One query row per (sequence, head) over a KV cache filled up to position p - 1, p = offset + *counter: the new key / value rows
+ * (k_new / v_new, the projection output of position p) are appended to the cache at p and the query attends over positions 0 .. p.
+ * GQA (Hkv divides H), head_dim 32 / 64 / 128, TCAVP_F32 or TCAVP_BF16.  Keys are split over CTAs in chunks of 128 and the partials merged
+ * by a second kernel (flash-decoding); fp32 SIMT arithmetic: a bandwidth-bound kernel, no tensor cores.  Strides in elements:
+ * q / k_new / v_new / out rows of sequence b at b * q_sb / b * new_sb / b * o_sb, cache rows at b * cache_sb + t * cache_st, head h at
+ * h * dh.  workspace: tcavp_decode_attention_workspace_bytes(B, H, dh, capacity) bytes of fp32 partials.  p >= capacity: no work. */
+typedef struct {
+  int B, H, Hkv, dh, capacity;
+  const void* q; long long q_sb;
+  const void* k_new; const void* v_new; long long new_sb;
+  void* k_cache; void* v_cache; long long cache_sb, cache_st;
+  void* out; long long o_sb;
+  int dtype; float scale;
+  const int* counter; int offset;
+  float* workspace; long long workspace_bytes;
+} tcavp_decode_attn_args;
+long long tcavp_decode_attention_workspace_bytes(int B, int H, int dh, int capacity);
+int tcavp_decode_attention(const tcavp_decode_attn_args* args, tcavp_stream_t stream);
+
+/* The position-dependent gathers of a decode step, p = offset + *counter: out[b, 0:H] = embed[tokens[b]] (+ wpe[p] when wpe != NULL:
+ * GPT-2) in `dtype` (row stride ldo), and, when rope_full != NULL, rope_out[0:dh] = row p of a tcavp_rope_table table of rope_L
+ * positions (layout 0 or 1), i.e. the one-position table of the GEMM's fused RoPE epilogue. */
+int tcavp_decode_embed(const long long* tokens, const void* embed, int vocab, const void* wpe, int n_pos, void* out, int ldo, int H, int dtype,
+                       const float* rope_full, int rope_L, int dh, int rope_layout, float* rope_out, const int* counter, int offset, int B,
+                       tcavp_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

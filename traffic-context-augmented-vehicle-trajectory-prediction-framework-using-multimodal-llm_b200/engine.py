@@ -172,7 +172,7 @@ class Engine:
         xs = torch.zeros(M, Kx, dtype=self.act, device=self.dev) if kx != m["n_lora"] else self._new(M, Kx)
         h = self._new(M, H)
         qkv, attn, mid = self._new(M, 3 * H), self._new(M, H), self._new(M, I)
-        for ly in m["layers"]:
+        for li, ly in enumerate(m["layers"]):
             if kx:      # ln_1(x) lands directly in the leading columns of the K-extended operand
                 ops.layernorm_strided(x, ly["ln1"][0], ly["ln1"][1], xs, rows=M, cols=H, eps=ly["ln1"][2], ldo=Kx)
                 ops.gemm(xs, ly["a_cat"], xs[:, H:], M=M, N=m["n_lora"], K=H, lda=Kx, ldo=Kx)
@@ -181,9 +181,8 @@ class Engine:
                 ops.layernorm(x, ly["ln1"][0], ly["ln1"][1], h, eps=ly["ln1"][2])
                 ops.gemm(h, ly["wqkv"], qkv, bias=ly["bqkv"])
             if kv_out is not None:       # prefill of a KV-cache decode: keys / values of every layer kept ([B, capacity, 2H])
-                cache = torch.empty(B, kv_out[1], 2 * H, dtype=self.act, device=self.dev)
+                cache = self._kv_cache(kv_out, li, B, 2 * H)
                 cache[:, :L].copy_(qkv.view(B, L, 3 * H)[:, :, H:])
-                kv_out[0].append(cache)
             ops.attention(qkv, qkv[:, H:], qkv[:, 2 * H:], attn, B=B, H=nh, Hkv=nh, Tq=L, Tk=L, dh=dh, q_strides=(L * 3 * H, 3 * H),
                           k_strides=(L * 3 * H, 3 * H), v_strides=(L * 3 * H, 3 * H), o_strides=(L * H, H), scale=dh ** -0.5, causal=True,
                           key_mask=mask)
@@ -197,13 +196,26 @@ class Engine:
         """llm_decode_step for a GPT-2-arch backbone: + wpe[t], the block sequence of _gpt2_forward on one row per sequence, the new key /
         value appended to the cache, one query over positions 0..t."""
         m = self.llm
-        H, nh, dh, I, kx = m["H"], m["nh"], m["dh"], m["I"], m["kx"]
-        B, Kx = x_new.shape[0], H + kx
+        H, nh, dh = m["H"], m["nh"], m["dh"]
+        B = x_new.shape[0]
         cap = caches[0].shape[1]
         if t >= cap or t >= m["wpe"].shape[0]:
             raise ops._lib.TcavpError(f"decode position {t} is past the cache capacity {cap} / n_positions {m['wpe'].shape[0]}")
         pos = ops.cast(m["wpe"][t:t + 1], self._new(B, H), rows=B, cols=H, in_row_mod=1)
         x = ops.axpby(x_new.reshape(B, H), self._new(B, H), rows=B, cols=H, b=pos)
+
+        def attend(qkv, cache, attn):
+            cache[:, t].copy_(qkv[:, H:])
+            ops.attention(qkv, cache, cache[:, :, H:], attn, B=B, H=nh, Hkv=nh, Tq=1, Tk=t + 1, dh=dh, q_strides=(3 * H, 3 * H),
+                          k_strides=(cap * 2 * H, 2 * H), v_strides=(cap * 2 * H, 2 * H), o_strides=(H, H), scale=dh ** -0.5)
+        return self._gpt2_decode_layers(x, B, caches, attend)
+
+    def _gpt2_decode_layers(self, x, B, caches, attend):
+        """The block sequence of one GPT-2 decode step on the rows `x` (B, H) = embedding + wpe of the new tokens; attend(qkv, cache, attn)
+        appends the new key / value and runs the one-row attention."""
+        m = self.llm
+        H, I, kx = m["H"], m["I"], m["kx"]
+        Kx = H + kx
         xs = torch.zeros(B, Kx, dtype=self.act, device=self.dev)
         h, qkv, attn, mid = self._new(B, H), self._new(B, 3 * H), self._new(B, H), self._new(B, I)
         for ly, cache in zip(m["layers"], caches):
@@ -214,9 +226,7 @@ class Engine:
             else:
                 ops.layernorm(x, ly["ln1"][0], ly["ln1"][1], h, eps=ly["ln1"][2])
                 ops.gemm(h, ly["wqkv"], qkv, bias=ly["bqkv"])
-            cache[:, t].copy_(qkv[:, H:])
-            ops.attention(qkv, cache, cache[:, :, H:], attn, B=B, H=nh, Hkv=nh, Tq=1, Tk=t + 1, dh=dh, q_strides=(3 * H, 3 * H),
-                          k_strides=(cap * 2 * H, 2 * H), v_strides=(cap * 2 * H, 2 * H), o_strides=(H, H), scale=dh ** -0.5)
+            attend(qkv, cache, attn)
             ops.gemm(attn, ly["proj"].w, x, bias=ly["proj"].b, residual=x)
             ops.layernorm(x, ly["ln2"][0], ly["ln2"][1], h, eps=ly["ln2"][2])
             ops.gemm(h, ly["fc"].w, mid, bias=ly["fc"].b, act=ops.ACT_GELU_TANH)
@@ -491,11 +501,24 @@ class Engine:
         else:   # zero decoder layers
             ops.add_rowvec(t, q["vis_mod"], fused, rows=B * Q, cols=Hq, remap=(Q, L_total, 0))
 
+    def _kv_cache(self, kv_out, li, B, width):
+        """Layer li's [B, capacity, width] cache of a prefill: the list's entry when the caller preallocated one per layer, else a new one
+        appended to the list."""
+        caches, cap = kv_out
+        if len(caches) == len(self.llm["layers"]):
+            c = caches[li]
+            if c.shape != (B, cap, width) or c.dtype != self.act or not c.is_contiguous():
+                raise ValueError(f"preallocated KV cache {li}: {tuple(c.shape)} {c.dtype}, expected ({B}, {cap}, {width}) {self.act}")
+            return c
+        caches.append(torch.empty(B, cap, width, dtype=self.act, device=self.dev))
+        return caches[-1]
+
     def llm_forward(self, fused, mask, B, L, kv_out=None):
         """HF:375-427 LlamaModel over inputs_embeds with LoRA on q/k/v (in place on `fused`); returns the
         post-final-norm hidden states (= hidden_states[-1], reference scripts/train.py:553).
         `kv_out` = (list, capacity): the prefill of a KV-cache decode — every layer's rotated keys and values are also stored in a
-        [B, capacity, 2 * n_kv * head_dim] cache appended to the list (generate.py; `llm_decode_step` continues from them)."""
+        [B, capacity, 2 * n_kv * head_dim] cache appended to the list (generate.py; `llm_decode_step` continues from them).  A list that
+        already holds one such cache per layer is filled in place (the static caches of a captured decode loop)."""
         m = self.llm
         if m.get("arch") == "gpt2":
             return self._gpt2_forward(fused, mask, B, L, kv_out)
@@ -538,9 +561,8 @@ class Engine:
             if rope is None:
                 ops.rope_(qkv, rows=M, L=L, ld=nqkv, n_q_heads=nh, n_k_heads=nkv, dh=dh, table=table)
             if kv_out is not None:
-                cache = torch.empty(B, kv_out[1], 2 * nkv * dh, dtype=self.act, device=self.dev)
+                cache = self._kv_cache(kv_out, li, B, 2 * nkv * dh)
                 cache[:, :L].copy_(qkv.view(B, L, nqkv)[:, :, nh * dh:])
-                kv_out[0].append(cache)
             ops.attention(qkv, qkv[:, nh * dh:], qkv[:, (nh + nkv) * dh:], attn, B=B, H=nh, Hkv=nkv, Tq=L, Tk=L, dh=dh,
                           q_strides=(L * nqkv, nqkv), k_strides=(L * nqkv, nqkv), v_strides=(L * nqkv, nqkv),
                           o_strides=(L * nh * dh, nh * dh), scale=dh ** -0.5, causal=True, key_mask=mask)
@@ -579,10 +601,23 @@ class Engine:
             self._rope[key] = ops.rope_table(cap, dh, m["theta"], self.dev, layout=lay)
         full = self._rope[key]
         table = (full[:, t:t + 1] if lay == 1 else full[t:t + 1]).contiguous()       # the one position this step needs (rope_L = 1)
+        xs = torch.zeros(B, H + kx, dtype=self.act, device=self.dev)
+        ops.cast(x_new.reshape(B, H), xs, rows=B, cols=H, ldi=H, ldo=H + kx)
+        nq, nk = nh * dh, nkv * dh
+
+        def attend(qkv, cache, attn):
+            cache[:, t].copy_(qkv[:, nq:])
+            ops.attention(qkv, cache, cache[:, :, nk:], attn, B=B, H=nh, Hkv=nkv, Tq=1, Tk=t + 1, dh=dh, q_strides=(qkv.shape[1], qkv.shape[1]),
+                          k_strides=(cap * 2 * nk, 2 * nk), v_strides=(cap * 2 * nk, 2 * nk), o_strides=(nq, nq), scale=dh ** -0.5)
+        return self._llama_decode_layers(xs, B, caches, table, attend)
+
+    def _llama_decode_layers(self, xs, B, caches, table, attend):
+        """The decoder stack of one Llama decode step on the K-extended rows `xs` (B, H + kx) holding the new tokens' embeddings; `table` =
+        the one-position RoPE table, attend(qkv, cache, attn) appends the new key / value and runs the one-row attention."""
+        m = self.llm
+        H, nh, nkv, dh, I, kx = m["H"], m["nh"], m["nkv"], m["dh"], m["I"], m["kx"]
         Kx, nq, nk = H + kx, nh * dh, nkv * dh
         nqkv = nq + 2 * nk
-        xs = torch.zeros(B, Kx, dtype=self.act, device=self.dev)
-        ops.cast(x_new.reshape(B, H), xs, rows=B, cols=H, ldi=H, ldo=Kx)
         x = xs[:, :H]
         rstd = torch.empty(B, dtype=torch.float32, device=self.dev)
         qkv, attn, mid = self._new(B, nqkv), self._new(B, nq), self._new(B, I)
@@ -597,9 +632,7 @@ class Engine:
                 ops.gemm(xs, ly["wqkv"], qkv, M=B, N=nqkv, K=Kx, lda=Kx, rope=rope, row_scale=rstd)
             if rope is None:
                 ops.rope_(qkv, rows=B, L=1, ld=nqkv, n_q_heads=nh, n_k_heads=nkv, dh=dh, table=table)
-            cache[:, t].copy_(qkv[:, nq:])
-            ops.attention(qkv, cache, cache[:, :, nk:], attn, B=B, H=nh, Hkv=nkv, Tq=1, Tk=t + 1, dh=dh, q_strides=(nqkv, nqkv),
-                          k_strides=(cap * 2 * nk, 2 * nk), v_strides=(cap * 2 * nk, 2 * nk), o_strides=(nq, nq), scale=dh ** -0.5)
+            attend(qkv, cache, attn)
             if self.fp8:
                 self._proj(ly, "wo", attn, x, residual=x)
                 self._proj(ly, "wgu", x, mid, rms=True, act=ops.ACT_SWIGLU)
@@ -610,6 +643,44 @@ class Engine:
             ops.gemm(xs, ly["wgu"], mid, M=B, K=H, lda=Kx, act=ops.ACT_SWIGLU, row_scale=rstd)
             ops.gemm(mid, ly["wdown"], x, ldo=Kx, residual=x, ldr=Kx)
         return ops.rmsnorm(xs, m["norm"], self._new(B, H), eps=m["eps"], rows=B, cols=H, ldi=Kx)
+
+    def decode_workspace(self, B, capacity):
+        """Device buffers of `llm_decode_step_device` for B sequences and a cache of `capacity` positions."""
+        m = self.llm
+        nkv = m["nh"] if m.get("arch") == "gpt2" else m["nkv"]
+        return dict(attn=ops.decode_attention_workspace(B, m["nh"], m["dh"], capacity, self.dev),
+                    rope=torch.empty(m["dh"], dtype=torch.float32, device=self.dev), nkv=nkv)
+
+    def llm_decode_step_device(self, tokens, caches, counter, offset, ws):
+        """`llm_decode_step` with the position on the device: the tokens (B,) int64 at position p = offset + counter[0] are embedded
+        (+ wpe[p] for GPT-2; RoPE row p for Llama) and decoded against `caches` filled up to p - 1; their keys / values are appended at p
+        (tcavp_decode_embed, tcavp_decode_attention).  No host-side position: a CUDA graph of this call stays correct when the counter
+        advances between replays.  `ws` = decode_workspace(B, capacity).  The caller keeps p below the cache capacity (and GPT-2's
+        n_positions); the kernels do no work past it."""
+        m = self.llm
+        H, nh, dh = m["H"], m["nh"], m["dh"]
+        B, cap = tokens.shape[0], caches[0].shape[1]
+        gpt2 = m.get("arch") == "gpt2"
+        nkv = ws["nkv"]
+        nq, nk = nh * dh, nkv * dh
+
+        def attend(qkv, cache, attn):
+            ld = qkv.shape[1]
+            ops.decode_attention(qkv, qkv[:, nq:], qkv[:, nq + nk:], cache, cache[:, :, nk:], attn, ws["attn"], counter, offset=offset, B=B, H=nh,
+                                 Hkv=nkv, dh=dh, capacity=cap, q_sb=ld, new_sb=ld, cache_sb=cap * 2 * nk, cache_st=2 * nk, o_sb=nq,
+                                 scale=dh ** -0.5)
+        if gpt2:
+            x = ops.decode_embed(tokens, m["embed"], self._new(B, H), counter, offset=offset, wpe=m["wpe"])
+            return self._gpt2_decode_layers(x, B, caches, attend)
+        kx = m["kx"]
+        lay = 1 if m["fuse_rope"] else 0
+        key = (cap, dh, lay)
+        if key not in self._rope:
+            self._rope[key] = ops.rope_table(cap, dh, m["theta"], self.dev, layout=lay)
+        xs = torch.zeros(B, H + kx, dtype=self.act, device=self.dev)
+        ops.decode_embed(tokens, m["embed"], xs, counter, offset=offset, ldo=H + kx, rope=(self._rope[key], cap, dh, lay, ws["rope"]))
+        table = ws["rope"].view(dh // 4, 1, 4) if lay == 1 else ws["rope"].view(1, dh // 2, 2)
+        return self._llama_decode_layers(xs, B, caches, table, attend)
 
     def ltsf_encode(self, x, B):
         """reference scripts/train.py:837-840 -> enc (B*T_in, C)."""

@@ -13,12 +13,21 @@ layer's rotated keys / values), then every new token is one `Engine.llm_decode_s
 query attends over the cached positions.  `kv_cache=False` recomputes the sequence so far at every step, which is also what the cached
 path is tested against.  The sampled tokens depend on torch's RNG, the logits do not.
 
+`seed=<int>` selects the device loop instead (KV cache only): after the eager prefill, one decode iteration — embed the sampled tokens,
+`Engine.llm_decode_step_device`, lm_head, `tcavp_sample_next` — is captured in a CUDA graph and replayed once per new token.  The
+position lives in device memory and the sampler advances it, so the loop makes no blocking host read; sampling is a pure function of
+(seed, row, step) (counter hash, include/tcavp.h) instead of torch's RNG, so a run is reproducible from its seed.  Same processors, same
+greedy tokens, different random draws than the default path.
+
 Deviation from the reference, on purpose: the reference's patched embedding returns `fused_embeds[:, :len(ids)]` on the first call, i.e.
 it silently drops the last 16 prompt positions and hands HF an attention mask that is 16 longer than the input (train.py:604-611,
 627-632).  This implementation generates after the FULL prefix (image tokens + whole prompt), which is what the surrounding code intends."""
 import torch
 
 from . import ops
+
+MAX_DECODE_LOOPS = 4     # captured decode loops kept per engine (least recently used dropped first)
+CAPTURES = 0             # decode-loop captures in this process
 
 
 @torch.no_grad()
@@ -65,8 +74,21 @@ def process_logits(logits, seq, temperature, top_k, top_p, repetition_penalty, n
 
 @torch.no_grad()
 def generate_ids(model, vision_embs, prompt_ids, max_new_tokens=128, temperature=0.9, top_k=40, top_p=0.9, do_sample=True,
-                 repetition_penalty=1.2, no_repeat_ngram_size=3, eos_token_id=None, pad_token_id=None, generator=None, kv_cache=True):
-    """-> (B, prompt + new) token ids: the prompt followed by the generated tokens (rows that hit `eos_token_id` are padded)."""
+                 repetition_penalty=1.2, no_repeat_ngram_size=3, eos_token_id=None, pad_token_id=None, generator=None, kv_cache=True, seed=None):
+    """-> (B, prompt + new) token ids: the prompt followed by the generated tokens (rows that hit `eos_token_id` are padded).
+    `seed` (int): the device loop (module docstring): sampling reproducible from the seed, no host synchronisation per token; needs
+    kv_cache=True and no `generator`."""
+    if seed is not None:
+        if isinstance(seed, bool) or not isinstance(seed, int):
+            raise ValueError(f"seed must be an int (got {type(seed).__name__})")
+        if not kv_cache:
+            raise ValueError("seed needs kv_cache=True: the device loop decodes from the KV cache")
+        if generator is not None:
+            raise ValueError("seed and generator are exclusive: with a seed the draws come from the counter hash, not from a torch generator")
+        return _generate_device(model, vision_embs, prompt_ids, int(max_new_tokens), seed, dict(
+            do_sample=bool(do_sample), temperature=float(temperature) if do_sample else 1.0, top_k=int(top_k or 0) if do_sample else 0,
+            top_p=(None if top_p is None else float(top_p)) if do_sample else None, repetition_penalty=float(repetition_penalty or 1.0),
+            no_repeat_ngram_size=int(no_repeat_ngram_size or 0), eos_token_id=eos_token_id, pad_token_id=pad_token_id))
     eng = model.engine()
     dev = eng.dev
     ids = prompt_ids.to(device=dev, dtype=torch.int64)
@@ -109,13 +131,15 @@ def generate_ids(model, vision_embs, prompt_ids, max_new_tokens=128, temperature
     return seq
 
 
-def generate_batch(model, vision_embs, prompt_ids, tokenizer, max_new_tokens=128, temperature=0.9, top_k=40, top_p=0.9, device="cuda"):
-    """Drop-in for `LlamaMultiModal.generate_batch` (train.py:577-654): list of decoded strings, cut after the reference's end marker."""
+def generate_batch(model, vision_embs, prompt_ids, tokenizer, max_new_tokens=128, temperature=0.9, top_k=40, top_p=0.9, device="cuda", seed=None):
+    """Drop-in for `LlamaMultiModal.generate_batch` (train.py:577-654): list of decoded strings, cut after the reference's end marker.
+    `seed`: the device loop of generate_ids."""
     was_training = model.training
     model.eval()
     try:
         out = generate_ids(model, vision_embs, prompt_ids, max_new_tokens=max_new_tokens, temperature=temperature, top_k=top_k, top_p=top_p,
-                           eos_token_id=getattr(tokenizer, "eos_token_id", None), pad_token_id=getattr(tokenizer, "pad_token_id", None))
+                           eos_token_id=getattr(tokenizer, "eos_token_id", None), pad_token_id=getattr(tokenizer, "pad_token_id", None),
+                           seed=seed)
     finally:
         model.train(was_training)
     texts = []
@@ -126,3 +150,108 @@ def generate_batch(model, vision_embs, prompt_ids, tokenizer, max_new_tokens=128
             text = text[: text.index(marker) + len(marker)]
         texts.append(text)
     return texts
+
+
+class DecodeLoop:
+    """The static buffers of one (B, prefix length, prompt length, new tokens, sampling parameters) on one engine and the CUDA graph of
+    one decode iteration over them: embed the tokens just sampled, `Engine.llm_decode_step_device` at position P - 1 + step, lm_head,
+    tcavp_sample_next (which appends the next token and advances the step).  `run` fills the caches with the eager prefill, samples the
+    first token and replays the graph for the others."""
+
+    def __init__(self, eng, B, P, Lp, n_new, sp):
+        global CAPTURES
+        m, dev = eng.llm, eng.dev
+        self.eng, self.B, self.P, self.Lp, self.n_new, self.sp = eng, B, P, Lp, n_new, sp
+        self.cap = P + n_new
+        width = 2 * (m["nh"] if m.get("arch") == "gpt2" else m["nkv"]) * m["dh"]
+        self.caches = [torch.zeros(B, self.cap, width, dtype=eng.act, device=dev) for _ in m["layers"]]
+        self.head = eng.lm_head()
+        V = self.head.shape[0]
+        self.logits = torch.zeros(B, V, dtype=torch.float32, device=dev)
+        self.work = torch.empty(B, V, dtype=torch.float32, device=dev)
+        self.hist = torch.zeros(B, Lp + n_new, dtype=torch.int64, device=dev)
+        self.tokens = torch.zeros(B, dtype=torch.int64, device=dev)
+        self.state = torch.zeros(3, dtype=torch.int32, device=dev)       # step, arrival counter, all-done step
+        self.done = torch.zeros(B, dtype=torch.int32, device=dev)
+        self.seed = torch.zeros(2, dtype=torch.int32, device=dev)
+        self.ws = eng.decode_workspace(B, self.cap)
+        self.flag = torch.zeros(1, dtype=torch.int32, pin_memory=True)
+        self.graph = None
+        if n_new > 1:
+            # one eager iteration on a side stream (RoPE table, allocator warm-up; the buffers it scribbles on are reset by run()), then capture
+            s = torch.cuda.Stream()
+            s.wait_stream(torch.cuda.current_stream())
+            with torch.cuda.stream(s):
+                self.iteration()
+            torch.cuda.current_stream().wait_stream(s)
+            self.graph = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(self.graph):
+                self.iteration()
+            CAPTURES += 1
+
+    def sample(self):
+        ops.sample_next(self.logits, self.work, self.hist, self.state, self.done, self.tokens, hist_offset=self.Lp, seed=self.seed, **self.sp)
+
+    def iteration(self):
+        h = self.eng.llm_decode_step_device(self.tokens, self.caches, self.state, self.P - 1, self.ws)
+        ops.gemm(h, self.head, self.logits)
+        self.sample()
+
+    def run(self, prefix, ids, seed):
+        """-> (B, Lp + generated) ids, trimmed as the eager loop trims them (at the first step after which every row is done)."""
+        eng, B, P, H = self.eng, self.B, self.P, prefix.shape[2]
+        s = int(seed) & 0xFFFFFFFFFFFFFFFF
+        words = [w - (1 << 32) if w >= (1 << 31) else w for w in (s & 0xFFFFFFFF, s >> 32)]
+        self.seed[0].fill_(words[0])
+        self.seed[1].fill_(words[1])
+        self.state.zero_()
+        self.done.zero_()
+        self.hist[:, :self.Lp].copy_(ids)
+        ones = torch.ones(B, P, dtype=torch.int32, device=eng.dev)
+        fh = eng.llm_forward(prefix.clone(), ones, B, P, kv_out=(self.caches, self.cap))
+        ops.gemm(fh.view(B, P, H)[:, P - 1].contiguous(), self.head, self.logits)
+        self.sample()
+        _device_loop(self, self.n_new - 1)
+        n = int(self.state[2]) or self.n_new          # after the loop: the one host read of the call
+        return self.hist[:, :self.Lp + n].clone()
+
+
+def _device_loop(loop, n):
+    """Replays the decode iteration up to n times.  When an EOS id is set, the all-done step is polled without blocking (a copy to pinned
+    memory behind an event that is only queried) and the loop stops once it is seen; the replays it may run past that point only append pad."""
+    poll = loop.sp["eos_token_id"] is not None
+    pending = None
+    for _ in range(n):
+        if pending is not None and pending.query():
+            if int(loop.flag[0]):
+                break
+            pending = None
+        loop.graph.replay()
+        if poll and pending is None:
+            loop.flag.copy_(loop.state[2:3], non_blocking=True)
+            pending = torch.cuda.Event()
+            pending.record()
+
+
+@torch.no_grad()
+def _generate_device(model, vision_embs, prompt_ids, max_new_tokens, seed, sp):
+    eng = model.engine()
+    ids = prompt_ids.to(device=eng.dev, dtype=torch.int64)
+    B, Lp = ids.shape
+    prefix = eng.prefix_embeds(vision_embs, ids)
+    P = prefix.shape[1]
+    if max_new_tokens <= 0:
+        return ids.clone()
+    m = eng.llm
+    if m.get("arch") == "gpt2" and P + max_new_tokens - 1 > m["wpe"].shape[0]:
+        raise ops._lib.TcavpError(f"decode position {P + max_new_tokens - 2} is past the cache capacity {P + max_new_tokens} / n_positions "
+                                  f"{m['wpe'].shape[0]}")
+    loops = eng.__dict__.setdefault("_decode_loops", {})
+    key = (B, P, Lp, max_new_tokens, tuple(sorted(sp.items())))
+    loop = loops.pop(key, None)
+    if loop is None:
+        loop = DecodeLoop(eng, B, P, Lp, max_new_tokens, sp)
+        while len(loops) >= MAX_DECODE_LOOPS:
+            loops.pop(next(iter(loops)))          # dicts keep insertion order: the first key is the least recently used
+    loops[key] = loop                             # (re-)inserted last = most recently used
+    return loop.run(prefix, ids, seed)

@@ -12,7 +12,7 @@ _ROOT = os.path.dirname(_HERE)
 CSRC = os.path.join(_HERE, "csrc")
 LIB_PATH = os.path.join(_HERE, "libtcavp.so")
 INCLUDE = os.path.join(_ROOT, "include")
-SOURCES = ["api.cu", "gemm.cu", "attention.cu", "attention_tc.cu", "attention_tm.cu", "attention_x.cu", "attention_xt.cu", "norm.cu", "elementwise.cu", "ltsf.cu", "backward.cu", "attention_bwd_tc.cu", "dw_tc.cu", "lora_drop.cu", "ffn_tm.cu", "ce.cu"]
+SOURCES = ["api.cu", "gemm.cu", "attention.cu", "attention_tc.cu", "attention_tm.cu", "attention_x.cu", "attention_xt.cu", "norm.cu", "elementwise.cu", "ltsf.cu", "backward.cu", "attention_bwd_tc.cu", "dw_tc.cu", "lora_drop.cu", "ffn_tm.cu", "ce.cu", "generate.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-I", INCLUDE]
 
@@ -30,6 +30,8 @@ EXPORTS = [
     "tcavp_clip_prologue", "tcavp_adamw_clipped", "tcavp_mark_nonfinite",
     # fp8 serving mode
     "tcavp_quant_e4m3_rows",
+    # text generation on the device
+    "tcavp_sample_next", "tcavp_decode_attention_workspace_bytes", "tcavp_decode_attention", "tcavp_decode_embed",
 ]
 
 
@@ -109,6 +111,7 @@ def load():
             lib.tcavp_last_error.restype = ctypes.c_char_p
             lib.tcavp_launch_count.restype = ctypes.c_longlong
             lib.tcavp_last_kernel.restype = ctypes.c_char_p
+            lib.tcavp_decode_attention_workspace_bytes.restype = ctypes.c_longlong
             for name in EXPORTS:
                 getattr(lib, name)   # AttributeError if a declared symbol is not exported
             _lib = lib

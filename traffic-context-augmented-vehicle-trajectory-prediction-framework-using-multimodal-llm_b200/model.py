@@ -341,15 +341,16 @@ class LlamaMultiModal(nn.Module):
         self.text_modality_embedding = nn.Parameter(torch.randn(1, 1, self.llama_hidden_size))
         self.tokenizer = None   # no hub access: callers pass input_ids / attention_mask (train.py:524 branch)
 
-    def generate_batch(self, vision_embs, prompt_ids, tokenizer, max_new_tokens=128, temperature=0.9, top_k=40, top_p=0.9, device="cuda"):
+    def generate_batch(self, vision_embs, prompt_ids, tokenizer, max_new_tokens=128, temperature=0.9, top_k=40, top_p=0.9, device="cuda", seed=None):
         """reference scripts/train.py:577-654 (the per-epoch sample generation of train.py:1231-1241): sampled continuation of the
-        prompt after the image-token prefix, decoded with `tokenizer`.  Runs on the owning model's engine — see generate.py."""
+        prompt after the image-token prefix, decoded with `tokenizer`.  Runs on the owning model's engine — see generate.py.  `seed` (int):
+        the CUDA-graph decode loop, sampling reproducible from the seed."""
         owner = self._owner() if getattr(self, "_owner", None) is not None else None
         if owner is None:
             raise RuntimeError("generate_batch needs the MultiModalTrajectoryModel that owns this module (its engine runs the decoder)")
         from .generate import generate_batch
         return generate_batch(owner, vision_embs, prompt_ids, tokenizer, max_new_tokens=max_new_tokens, temperature=temperature, top_k=top_k,
-                              top_p=top_p, device=device)
+                              top_p=top_p, device=device, seed=seed)
 
 
 class SelfAttentionBlock(nn.Module):

@@ -864,3 +864,91 @@ def mark_nonfinite_(loss, dst):
         raise ValueError("mark_nonfinite_: loss is one value, dst not empty")
     _call("tcavp_mark_nonfinite", "mark_nonfinite_kernel", _p(loss), _p(dst))
     return dst
+
+
+# --------------------------------------------------------------------------------------------------
+# text generation on the device (include/tcavp.h, "text generation on the device")
+# --------------------------------------------------------------------------------------------------
+class DecodeAttnArgs(Structure):
+    _fields_ = [("B", c_int), ("H", c_int), ("Hkv", c_int), ("dh", c_int), ("capacity", c_int),
+                ("q", c_void_p), ("q_sb", c_longlong),
+                ("k_new", c_void_p), ("v_new", c_void_p), ("new_sb", c_longlong),
+                ("k_cache", c_void_p), ("v_cache", c_void_p), ("cache_sb", c_longlong), ("cache_st", c_longlong),
+                ("out", c_void_p), ("o_sb", c_longlong),
+                ("dtype", c_int), ("scale", c_float),
+                ("counter", c_void_p), ("offset", c_int),
+                ("workspace", c_void_p), ("workspace_bytes", c_longlong)]
+
+
+def _need_i32_counter(counter):
+    if counter.dtype != torch.int32 or not counter.is_cuda:
+        raise TypeError("the decode position counter must be a CUDA int32 tensor")
+
+
+def sample_next(logits, work, hist, state, done, tokens, *, hist_offset, seed=None, do_sample=True, temperature=1.0, top_k=0, top_p=None,
+                repetition_penalty=1.0, no_repeat_ngram_size=0, eos_token_id=None, pad_token_id=None):
+    """One step of generate.py's process_logits + draw for every row of fp32 `logits` [B, V] (tcavp_sample_next): `work` [B, V] fp32
+    receives the processed logits, the token goes to `tokens` [B] int64 and hist[b, hist_offset + state[0]]; state int32[3]
+    (step, 0, all-done step) and done int32[B] are device state.  `seed`: CUDA int32[2] (low, high word), needed when do_sample."""
+    _need_cuda(logits, work, hist, state, done, tokens, seed)
+    B, V = logits.shape
+    if logits.dtype != torch.float32 or work.dtype != torch.float32 or logits.stride(1) != 1 or work.stride() != (V, 1):
+        raise TypeError("sample_next: logits / work must be fp32 with unit column stride (work contiguous [B, V])")
+    if hist.dtype != torch.int64 or tokens.dtype != torch.int64 or hist.stride(1) != 1:
+        raise TypeError("sample_next: hist / tokens must be int64")
+    if state.dtype != torch.int32 or done.dtype != torch.int32 or state.numel() < 3 or done.numel() < B:
+        raise TypeError("sample_next: state int32[3], done int32[B]")
+    if seed is not None and (seed.dtype != torch.int32 or seed.numel() != 2):
+        raise TypeError("sample_next: seed must be int32[2]")
+    eos = -1 if eos_token_id is None else int(eos_token_id)
+    pad = eos if pad_token_id is None else int(pad_token_id)
+    p = 0.0 if top_p is None else float(top_p)
+    with _Timed("sample_next_kernel", 0.0, float(B * V * 8)):
+        _lib.check(_lib.load().tcavp_sample_next(_p(logits), _ll(logits.stride(0)), B, V, _p(work), _p(hist), hist.stride(0), hist_offset,
+                                                 _p(state), _p(seed), int(bool(do_sample)), c_float(temperature), int(top_k or 0), c_float(p),
+                                                 c_float(repetition_penalty or 1.0), int(no_repeat_ngram_size or 0), _ll(eos),
+                                                 _ll(0 if pad < 0 else pad), _p(done), _p(tokens), _stream()), "tcavp_sample_next")
+    return tokens
+
+
+def decode_attention_workspace(B, H, dh, capacity, device):
+    n = int(_lib.load().tcavp_decode_attention_workspace_bytes(B, H, dh, capacity))
+    return torch.empty(n // 4, dtype=torch.float32, device=device)
+
+
+def decode_attention(q, k_new, v_new, k_cache, v_cache, out, workspace, counter, *, offset, B, H, Hkv, dh, capacity, q_sb, new_sb,
+                     cache_sb, cache_st, o_sb, scale):
+    """tcavp_decode_attention: one query row per (sequence, head) at position p = offset + counter[0]; appends k_new / v_new to the
+    cache at p and attends over positions 0 .. p.  Strides in elements (see include/tcavp.h)."""
+    _need_cuda(q, k_new, v_new, k_cache, v_cache, out, workspace, counter)
+    _need_i32_counter(counter)
+    a = DecodeAttnArgs()
+    a.B, a.H, a.Hkv, a.dh, a.capacity = B, H, Hkv, dh, capacity
+    a.q, a.q_sb = q.data_ptr(), q_sb
+    a.k_new, a.v_new, a.new_sb = k_new.data_ptr(), v_new.data_ptr(), new_sb
+    a.k_cache, a.v_cache, a.cache_sb, a.cache_st = k_cache.data_ptr(), v_cache.data_ptr(), cache_sb, cache_st
+    a.out, a.o_sb = out.data_ptr(), o_sb
+    a.dtype, a.scale = dt(q), scale
+    a.counter, a.offset = counter.data_ptr(), offset
+    a.workspace, a.workspace_bytes = workspace.data_ptr(), workspace.numel() * workspace.element_size()
+    # algorithmic bytes at the largest position the cache holds (the live length is on the device)
+    nbytes = q.element_size() * B * dh * (2.0 * H + 2.0 * Hkv * capacity)
+    with _Timed("decode_attention[dh%d]" % dh, 4.0 * B * H * capacity * dh, nbytes):
+        _lib.check(_lib.load().tcavp_decode_attention(byref(a), _stream()), "tcavp_decode_attention")
+    return out
+
+
+def decode_embed(tokens, embed, out, counter, *, offset, ldo=None, wpe=None, rope=None):
+    """tcavp_decode_embed: out[b, :H] = embed[tokens[b]] (+ wpe[p]) and, with rope = (full table, L, dh, layout, one-row out), the
+    RoPE table row of p = offset + counter[0]."""
+    _need_cuda(tokens, embed, out, counter, wpe)
+    _need_i32_counter(counter)
+    if tokens.dtype != torch.int64 or embed.dtype != out.dtype or (wpe is not None and wpe.dtype != embed.dtype):
+        raise TypeError("decode_embed: int64 tokens, embed / wpe / out of one dtype")
+    B, H = tokens.shape[0], embed.shape[1]
+    full, L, dh, layout, row = rope if rope is not None else (None, 0, 0, 0, None)
+    with _Timed("decode_embed_kernel", 0.0, float(B * H * 2 * out.element_size())):
+        _lib.check(_lib.load().tcavp_decode_embed(_p(tokens), _p(embed), embed.shape[0], _p(wpe), 0 if wpe is None else wpe.shape[0], _p(out),
+                                                  H if ldo is None else ldo, H, dt(out), _p(full), L, dh, layout, _p(row), _p(counter), offset, B,
+                                                  _stream()), "tcavp_decode_embed")
+    return out
