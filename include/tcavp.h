@@ -143,8 +143,9 @@ int tcavp_split_bf16x3(const float* x, int ldx, void* out, int ldo, long long ro
  *   key_mask    optional int32 [B, Tk], 1 = attend, 0 = masked (key padding).  Rows whose keys are all
  *               masked produce zeros (the reference discards such rows, train.py:378-380).
  * Softmax statistics and accumulation are fp32 for both dtypes.  `dtype` applies to q, k, v and out.
- * bf16 with dh in {16,32,64,96,128} and Tq,Tk <= 256 (flash kernel) or with few queries against a wide head
- * (Tq <= 32, dh % 64 == 0: LTSF cross-attention) runs on tensor cores; everything else on the SIMT kernel.
+ * bf16 with dh in {16,32,64,96,128} and Tq,Tk <= 256 (flash kernel), causal self-attention with dh 64 / 128 and Tq == Tk >= 128 at
+ * any length (tcgen05 kernels), or few queries against a wide head (Tq <= 32, dh % 64 == 0: LTSF cross-attention) runs on tensor cores;
+ * everything else on the SIMT kernel.
  */
 typedef struct tcavp_attn_args {
   int B, H, Hkv, Tq, Tk, dh;
@@ -160,6 +161,10 @@ typedef struct tcavp_attn_args {
    * layers of train.py:358, 402-405): P_drop = keep(b, h, i, j) ? P / (1 - p) : 0, applied after the softmax (row sums on the undropped
    * P).  drop_thresh == 0 disables it.  See tcavp_dropout for the mask function; element index = ((b*H + h)*Tq + i)*Tk + j. */
   const uint32_t* drop_seed; uint32_t drop_site; uint32_t drop_thresh; float drop_scale;
+  /* optional fp32 [B, H, Tq] output (element (b, h, i) at lse[b*lse_sb + h*Tq + i]): the natural-log logsumexp of the scaled scores over
+   * the keys row i may see, -inf for a row with no visible key.  Written by the self-attention routes (head_dim <= 128 bf16 and every
+   * fp32 shape); the backward of tcavp_attention_bwd_owned recomputes the probabilities from it.  NULL writes nothing. */
+  float* lse; long long lse_sb;
 } tcavp_attn_args;
 
 int tcavp_attention(const tcavp_attn_args* args, tcavp_stream_t stream);
@@ -363,10 +368,13 @@ int tcavp_dw(const void* dY, int lddy, int dy_dtype, const void* X, int ldx, int
 int tcavp_attention_bwd(const tcavp_attn_args* args, const void* dout, long long do_sb, long long do_st, void* dq, long long dq_sb,
                         long long dq_st, float* dk, long long dk_sb, long long dk_st, float* dv, long long dv_sb, long long dv_st,
                         tcavp_stream_t stream);
-/* Tensor-core-only form of tcavp_attention_bwd for H == Hkv: one CTA owns every key row of its (batch, head), so dk / dv are
- * plain stores in `dkv_dtype` (TCAVP_BF16: straight into the packed d(qkv) activation buffer — no fp32 staging, no zero-fill,
- * no cast) with the same stride convention as k / v.  args->out must hold the forward output.  Fails (TCAVP_ERR_ARG) on shapes the
- * tensor-core kernel does not cover; callers then use tcavp_attention_bwd. */
+/* Tensor-core-only form of tcavp_attention_bwd: the CTAs that own a key range sum its gradient over every query (and every query head
+ * of a GQA group), so dk / dv are plain stores in `dkv_dtype` (TCAVP_BF16: straight into the packed d(qkv) activation buffer — no
+ * fp32 staging, no zero-fill, no cast) with the same stride convention as k / v; no atomics, repeated calls give the same bits.
+ * args->out must hold the forward output.  With args->lse holding the forward's logsumexp (tcavp_attention with lse set), bf16,
+ * head_dim 64 / 128 and no dropout, any length and any H % Hkv == 0 is covered (key-blocked kernels; MHA at <= 256 positions keeps the
+ * one-CTA-per-head kernel); without it H == Hkv and Tq, Tk <= 256.  Fails (TCAVP_ERR_ARG) on shapes the tensor-core kernels do not
+ * cover; callers then use tcavp_attention_bwd. */
 int tcavp_attention_bwd_owned(const tcavp_attn_args* args, const void* dout, long long do_sb, long long do_st, void* dq, long long dq_sb,
                               long long dq_st, void* dk, long long dk_sb, long long dk_st, void* dv, long long dv_sb, long long dv_st,
                               int dkv_dtype, tcavp_stream_t stream);

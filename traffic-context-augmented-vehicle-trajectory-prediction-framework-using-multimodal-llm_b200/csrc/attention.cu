@@ -99,6 +99,7 @@ __global__ void __launch_bounds__(128) attn_warp_kernel(tcavp_attn_args a) {
     m = mn;
   }
   const float inv = l > 0.f ? 1.f / l : 0.f;
+  if (a.lse && lane == 0) a.lse[(size_t)b * a.lse_sb + (size_t)h * a.Tq + i] = m + logf(l);   // -inf when no key is visible
   T* o = reinterpret_cast<T*>(a.out) + (size_t)b * a.o_sb + (size_t)i * a.o_st + (size_t)h * a.dh;
 #pragma unroll
   for (int e = 0; e < NE; ++e) {
@@ -170,6 +171,7 @@ __global__ void __launch_bounds__(128) attn_row_kernel(tcavp_attn_args a) {
       m = mn;
     }
     const float inv = l > 0.f ? 1.f / l : 0.f;
+    if (a.lse) a.lse[(size_t)b * a.lse_sb + (size_t)h * a.Tq + i] = m + logf(l);
     T* o = reinterpret_cast<T*>(a.out) + (size_t)b * a.o_sb + (size_t)i * a.o_st + (size_t)h * DH;
 #pragma unroll
     for (int d = 0; d < DH; ++d) o[d] = Cvt<T>::from_f(acc[d] * inv);
@@ -214,8 +216,10 @@ extern "C" int tcavp_attention(const tcavp_attn_args* a, tcavp_stream_t stream_)
   TCAVP_REQUIRE(!a->causal || a->Tq == a->Tk, "tcavp_attention: causal needs Tq == Tk");
   TCAVP_REQUIRE(a->dtype == TCAVP_F32 || a->dtype == TCAVP_BF16, "tcavp_attention: bad dtype");
   TCAVP_REQUIRE(a->drop_thresh == 0 || (a->drop_seed != nullptr && a->drop_scale > 0.f), "tcavp_attention: dropout needs a device seed and a scale");
+  TCAVP_REQUIRE(!a->lse || a->dtype == TCAVP_F32 || a->dh <= 128, "tcavp_attention: lse needs head_dim <= 128 in bf16");
   if (a->dtype == TCAVP_BF16) {
-    int rc = attention_xt_launch(*a, stream);       // two heads on one shared K = V head (checks its own shape conditions first)
+    // two heads on one shared K = V head (checks its own shape conditions first; writes no lse)
+    int rc = a->lse ? 1 : attention_xt_launch(*a, stream);
     if (rc > 0) rc = a->dh > 128 ? attention_x_launch(*a, stream) : attention_tm_launch(*a, stream);
     if (rc > 0 && a->dh <= 128) rc = attention_tc_launch(*a, stream);
     if (rc <= 0) return rc;

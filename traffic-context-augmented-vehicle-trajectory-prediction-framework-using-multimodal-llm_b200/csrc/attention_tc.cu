@@ -234,6 +234,11 @@ __global__ void __launch_bounds__(MAXT, MINB) attn_flash_kernel(tcavp_attn_args 
   l_hi += __shfl_xor_sync(0xffffffffu, l_hi, 1);
   l_hi += __shfl_xor_sync(0xffffffffu, l_hi, 2);
   const float i_lo = l_lo > 0.f ? 1.f / l_lo : 0.f, i_hi = l_hi > 0.f ? 1.f / l_hi : 0.f;
+  if (a.lse && t4 == 0) {        // natural log of the row sum at the base-2 reference max; -inf for a row with no visible key
+    float* lse = a.lse + (size_t)b * a.lse_sb + (size_t)h * a.Tq;
+    if (r_lo < a.Tq) lse[r_lo] = (m_lo + log2f(l_lo)) * 0.6931471805599453f;
+    if (r_hi < a.Tq) lse[r_hi] = (m_hi + log2f(l_hi)) * 0.6931471805599453f;
+  }
 #pragma unroll
   for (int n = 0; n < NT; ++n) {
     const int c = n * 8 + t4 * 2;

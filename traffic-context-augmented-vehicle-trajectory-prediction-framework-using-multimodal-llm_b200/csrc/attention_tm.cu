@@ -1,5 +1,7 @@
 // tcgen05 flash attention for the LLM self-attention (HF:251-289 with the causal + key-padding mask of HF:399; GQA):
-// bf16, causal, head_dim 64 / 128, 128 <= L <= 256 (the fused sequence is 16 image + 128 text tokens = 144).
+// bf16, causal, head_dim 64 / 128, L >= 128.  attn_tm_kernel below covers 128 <= L <= 256 (the fused sequence is 16 image + 128 text
+// tokens = 144) with whole-row tiles; attn_tml_kernel (further down) covers L > 256 with 128-key blocks and an online softmax.
+// Both optionally write the row logsumexp (tcavp_attn_args::lse) that the key-blocked backward rebuilds the probabilities from.
 //
 // Persistent, warp-specialised, one CTA per SM looping over (scene, head) items:
 //   warp 0      TMA producer: Q, K, V tiles of the item ([L16 rows] x 64-column boxes, 128-byte swizzle) straight out of the packed
@@ -130,6 +132,7 @@ struct Geo {
   float sl2;                          // softmax scale * log2(e)
   const int32_t* key_mask;
   __nv_bfloat16* out; long long o_sb, o_st;
+  float* lse; long long lse_sb;       // optional [B, H, L] logsumexp output
 };
 
 // Valid-key bits of the 16 score columns [16u, 16u + 16) for query row q: key-padding bits AND the causal bound j <= q.
@@ -145,9 +148,9 @@ __device__ __forceinline__ uint32_t unit_bits(const uint32_t* s_mask, int u, int
 // (211 us against 202 us on the 768-class shape).  The bf16 probabilities overwrite the score columns (P aliases S).  A
 // 16-column unit whose keys are all attendable for every row of the warp (the common case left of the causal diagonal) takes a
 // select-free path.  `q`: query index of the row, `ncols`: key columns of the tile, `warp_kmax`: largest key any row of the warp sees.
-// Returns the row sum.
+// Returns (row sum, base-2 reference max the probabilities were taken against).
 // (__noinline__: tile A and tile B share one copy — ten warps in different places of a 60 KB kernel thrash the instruction caches)
-__device__ __noinline__ float softmax_rows(const Geo& g, uint32_t srow, int q, int ncols, int warp_kmax, const uint32_t* s_mask) {
+__device__ __noinline__ float2 softmax_rows(const Geo& g, uint32_t srow, int q, int ncols, int warp_kmax, const uint32_t* s_mask) {
   const int nu = min(ncols, (warp_kmax + 16) & ~15) >> 4;
   const int nu_all = ncols >> 4;
   float m = -INFINITY;
@@ -199,7 +202,12 @@ __device__ __noinline__ float softmax_rows(const Geo& g, uint32_t srow, int q, i
   }
   tmem_st_wait();
   tc_fence_before();
-  return l;
+  return make_float2(l, mref);
+}
+
+// lse[b, h, q] = ln(sum_j exp(scale * s_qj)) from the row sum l taken against the base-2 reference mref (-inf when l == 0)
+__device__ __forceinline__ void store_lse(float* lse, long long lse_sb, int H, int L, int b, int h, int q, float l, float mref) {
+  if (lse && q < L) lse[(size_t)b * lse_sb + (size_t)h * L + q] = (mref + log2f(l)) * 0.6931471805599453f;
 }
 
 // Drains one output row per thread: O / row sum -> bf16 -> global (128 or 256 contiguous bytes per row).
@@ -400,14 +408,18 @@ attn_tm_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constant_
       const int qb = wq * 32 + lane;                    // tile B row = query index
       if (has_b) {
         // rows >= NB of tile B are not part of the problem: their query index is pushed past L so nothing is stored for them
-        l_b = softmax_rows(g, lane_base + g.sb_col, qb < g.NB ? qb : g.L + qb, g.NB, min(wq * 32 + 31, g.NB - 1), s_mask[st]);
+        const float2 r = softmax_rows(g, lane_base + g.sb_col, qb < g.NB ? qb : g.L + qb, g.NB, min(wq * 32 + 31, g.NB - 1), s_mask[st]);
+        l_b = r.x;
         __syncwarp();
         if (lane == 0) mbar_arrive(sbar + SL_PB);
+        store_lse(g.lse, g.lse_sb, g.H, g.L, b, h, qb < g.NB ? qb : g.L + qb, r.x, r.y);
       }
       const int qa = qa0 + wq * 32 + lane;
-      const float l_a = softmax_rows(g, lane_base, qa, g.L16, qa0 + wq * 32 + 31, s_mask[st]);
+      const float2 ra = softmax_rows(g, lane_base, qa, g.L16, qa0 + wq * 32 + 31, s_mask[st]);
+      const float l_a = ra.x;
       __syncwarp();
       if (lane == 0) mbar_arrive(sbar + SL_PA);
+      store_lse(g.lse, g.lse_sb, g.H, g.L, b, h, qa, ra.x, ra.y);
       if (has_b) {
         mbar_wait(sbar + SL_OBFULL, ph);
         tc_fence_after();
@@ -424,6 +436,330 @@ attn_tm_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constant_
         b += step_b; h += step_h;
         if (h >= g.H) { h -= g.H; ++b; }
       }
+    }
+  }
+
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 1) {
+    tc_fence_after();
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
+  }
+}
+
+
+// ------------------------------------------------------------------------------------------------
+// Key-blocked form for L > 256 (attn_tml_kernel): one work item = (scene, head, 128-row query tile t), which iterates over the
+// 128-key blocks 0 .. t (causal: block t is the diagonal one, the only block that needs the causal mask).  Same roles as above:
+//   warp 0      TMA producer: the item's Q tile into a 2-deep Q ring, then K and V of every key block into a stage ring, plus the
+//               block's four key-valid words (ballots over key_mask, so the mask costs no shared memory that grows with L)
+//   warp 1      one thread issues S(g) = Q K_g^T into one of two S buffers, ONE BLOCK AHEAD of O += P(g-1) V(g-1) (A = P from TMEM,
+//               B = V MN-major), so the softmax of block g overlaps the score product of block g + 1
+//   warps 4-7   online softmax, one thread per query row: running reference max and row sum in registers, P written over S
+// TMEM: S0 [0, 128), S1 [128, 256), O [256, 256 + dh).  O accumulates across the key blocks of an item.
+//
+// Rescaling O: a row's probabilities are taken against a reference max that is only raised when the block max exceeds it by more
+// than RESCALE_LOG2 (2^8 in probability): every probability stays <= 256, exact enough in bf16 and far from fp32 overflow, and
+// the final normalisation divides by the row sum taken against the same stale reference, so the result does not depend on when the
+// reference moved.  When it does move, the row's thread tcgen05.ld's its O row, scales it and tcgen05.st's it back after the
+// previous P.V has retired and before it releases P of this block.  Random and trained scores raise it in the first block or two
+// only, so almost every block skips the O round trip.
+// Items are ordered longest first (query tile NT-1 of every (scene, head) before tile NT-2, ...) and dealt round-robin to the
+// persistent CTAs, so the uneven causal work of the tiles evens out across the grid.
+constexpr int L_THREADS = 256;           // 8 warps: 0 TMA, 1 MMA (+ TMEM owner), 2-3 idle, 4-7 softmax
+constexpr int L_MAX_STAGES = 4;
+constexpr float RESCALE_LOG2 = 8.f;
+
+struct GeoL {
+  int B, H, Hkv, L, NT;                  // NT = 128-row query tiles per (scene, head)
+  int stages;
+  uint32_t q_bytes, stage_bytes;         // one Q tile; K + V of one key block
+  float sl2;
+  const int32_t* key_mask;
+  __nv_bfloat16* out; long long o_sb, o_st;
+  float* lse; long long lse_sb;
+};
+
+// barriers (8 bytes each): q_full[2], q_empty[2], kv_full[S], kv_empty[S], mask[S], s_full[2], p_ready, pv_done, o_free, TMEM slot
+constexpr uint32_t LB_QFULL = 0, LB_QEMPTY = 16, LB_KVFULL = 32, LB_KVEMPTY = LB_KVFULL + 8 * L_MAX_STAGES,
+                   LB_MASK = LB_KVEMPTY + 8 * L_MAX_STAGES, LB_SFULL = LB_MASK + 8 * L_MAX_STAGES, LB_PREADY = LB_SFULL + 16,
+                   LB_PVDONE = LB_PREADY + 8, LB_OFREE = LB_PVDONE + 8, LB_TMEM = LB_OFREE + 8, LB_BYTES = LB_TMEM + 8;
+
+__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&r)[16]) {
+  asm volatile(
+      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};" ::"r"(taddr),
+      "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]), "r"(r[10]), "r"(r[11]),
+      "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
+      : "memory");
+}
+
+// item -> (scene, head, query tile), longest tiles first
+__device__ __forceinline__ void item_coords(const GeoL& g, int it, int& b, int& h, int& t) {
+  const int bh = g.B * g.H;
+  t = g.NT - 1 - it / bh;
+  const int r = it % bh;
+  b = r / g.H;
+  h = r % g.H;
+}
+
+template <int DH>
+__global__ void __launch_bounds__(L_THREADS, 1)
+attn_tml_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constant__ CUtensorMap tma_k, const __grid_constant__ CUtensorMap tma_v, GeoL g) {
+  constexpr int NBOX = DH / BOXC;
+  constexpr uint32_t BOX = 128u * 128u;                        // one [128 rows x 64 columns] bf16 box
+  extern __shared__ uint8_t smem_raw[];
+  __shared__ uint32_t s_mask[L_MAX_STAGES][4];                 // per stage: key-valid bits of the block's 128 keys
+  const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
+  const uint32_t sq0 = smem_base, skv0 = smem_base + 2u * g.q_bytes;
+  const uint32_t bars = skv0 + (uint32_t)g.stages * g.stage_bytes;
+  uint32_t* tmem_slot_ptr = reinterpret_cast<uint32_t*>(smem_raw + (bars + LB_TMEM - smem_u32(smem_raw)));
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int n_items = g.B * g.H * g.NT;
+  const int my_items = blockIdx.x < n_items ? (n_items - 1 - (int)blockIdx.x) / (int)gridDim.x + 1 : 0;
+  const int hrep = g.H / g.Hkv;
+
+  if (warp == 0 && lane == 0) {
+    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tma_q)) : "memory");
+    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tma_k)) : "memory");
+    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tma_v)) : "memory");
+    for (int i = 0; i < 2; ++i) {
+      mbar_init(bars + LB_QFULL + 8 * i, 1);
+      mbar_init(bars + LB_QEMPTY + 8 * i, 1);
+      mbar_init(bars + LB_SFULL + 8 * i, 1);
+    }
+    for (int s = 0; s < L_MAX_STAGES; ++s) {
+      mbar_init(bars + LB_KVFULL + 8 * s, 1);
+      mbar_init(bars + LB_KVEMPTY + 8 * s, 1);
+      mbar_init(bars + LB_MASK + 8 * s, 1);
+    }
+    mbar_init(bars + LB_PREADY, 4);
+    mbar_init(bars + LB_PVDONE, 1);
+    mbar_init(bars + LB_OFREE, 4);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  if (warp == 1) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(bars + LB_TMEM), "r"(512) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *tmem_slot_ptr;
+
+  if (warp == 0) {
+    // ===================== TMA producer =====================
+    uint32_t gblk = 0;                                            // running key-block counter of this CTA
+    for (int n = 0; n < my_items; ++n) {
+      int b, h, t;
+      item_coords(g, (int)blockIdx.x + n * (int)gridDim.x, b, h, t);
+      const int hk = h / hrep;
+      if (lane == 0) {
+        const uint32_t qf = bars + LB_QFULL + 8 * (n & 1);
+        mbar_wait(bars + LB_QEMPTY + 8 * (n & 1), (((uint32_t)n >> 1) & 1u) ^ 1u);
+        mbar_expect_tx(qf, g.q_bytes);
+#pragma unroll
+        for (int c = 0; c < NBOX; ++c) tma_load_2d(sq0 + (n & 1) * g.q_bytes + c * BOX, &tma_q, qf, h * DH + c * BOXC, b * g.L + t * 128);
+      }
+      for (int j = 0; j <= t; ++j, ++gblk) {
+        const int s = (int)(gblk % (uint32_t)g.stages);
+        const uint32_t use = gblk / (uint32_t)g.stages;
+        int kv[4];
+#pragma unroll
+        for (int w = 0; w < 4; ++w) {                             // HF:399: padding keys are masked for every query
+          const int key = j * 128 + w * 32 + lane;
+          kv[w] = key < g.L ? (g.key_mask ? __ldg(g.key_mask + (size_t)b * g.L + key) : 1) : 0;
+        }
+        if (lane == 0) {
+          mbar_wait(bars + LB_KVEMPTY + 8 * s, (use & 1u) ^ 1u);   // also frees the stage's mask words (read before P is ready)
+          const uint32_t full = bars + LB_KVFULL + 8 * s;
+          mbar_expect_tx(full, g.stage_bytes);
+          const uint32_t st = skv0 + (uint32_t)s * g.stage_bytes;
+#pragma unroll
+          for (int c = 0; c < NBOX; ++c) {
+            tma_load_2d(st + c * BOX, &tma_k, full, hk * DH + c * BOXC, b * g.L + j * 128);
+            tma_load_2d(st + (NBOX + c) * BOX, &tma_v, full, hk * DH + c * BOXC, b * g.L + j * 128);
+          }
+        }
+        __syncwarp();
+#pragma unroll
+        for (int w = 0; w < 4; ++w) {
+          const uint32_t bits = __ballot_sync(0xffffffffu, kv[w] != 0);
+          if (lane == 0) s_mask[s][w] = bits;
+        }
+        if (lane == 0) mbar_arrive(bars + LB_MASK + 8 * s);
+        __syncwarp();
+      }
+    }
+  } else if (warp == 1) {
+    // ===================== MMA issuer: S one key block ahead of P.V =====================
+    if (lane == 0) {
+      const uint32_t id_s = idesc_f16(128, 128, 0), id_pv = idesc_f16(128, DH, 1);
+      const uint32_t tO = tmem_base + 256;
+      // S cursor: (item sn, block sj, global block sg); the P.V cursor trails it by one block
+      int sn = 0, sj = 0, st_ = 0;
+      uint32_t sg = 0;
+      auto issue_s = [&]() {
+        if (sn >= my_items) return;
+        int b, h, t;
+        item_coords(g, (int)blockIdx.x + sn * (int)gridDim.x, b, h, t);
+        (void)b; (void)h;
+        st_ = t;
+        if (sj == 0) mbar_wait(bars + LB_QFULL + 8 * (sn & 1), ((uint32_t)sn >> 1) & 1u);
+        const int s = (int)(sg % (uint32_t)g.stages);
+        mbar_wait(bars + LB_KVFULL + 8 * s, (sg / (uint32_t)g.stages) & 1u);
+        tc_fence_after();
+        const uint32_t sq = sq0 + (sn & 1) * g.q_bytes, sk = skv0 + (uint32_t)s * g.stage_bytes;
+        const uint32_t tS = tmem_base + (sg & 1u) * 128u;
+#pragma unroll
+        for (int kk = 0; kk < DH / 16; ++kk) {
+          const uint32_t boff = (uint32_t)(kk >> 2) * BOX + (uint32_t)(kk & 3) * 32u;
+          umma_ss(tS, desc_kmajor(sq + boff), desc_kmajor(sk + boff), id_s, kk != 0);
+        }
+        umma_commit(bars + LB_SFULL + 8 * (sg & 1u));
+        if (sj == st_) {                                          // last score product of the item: its Q buffer may be refilled
+          umma_commit(bars + LB_QEMPTY + 8 * (sn & 1));
+          ++sn; sj = 0;
+        } else {
+          ++sj;
+        }
+        ++sg;
+      };
+      issue_s();
+      uint32_t pg = 0;
+      for (int n = 0; n < my_items; ++n) {
+        int b, h, t;
+        item_coords(g, (int)blockIdx.x + n * (int)gridDim.x, b, h, t);
+        for (int j = 0; j <= t; ++j, ++pg) {
+          issue_s();                                              // S(pg + 1) overwrites P(pg - 1): its P.V was issued earlier
+          if (j == 0) mbar_wait(bars + LB_OFREE, ((uint32_t)n & 1u) ^ 1u);   // the previous item's O has been drained
+          mbar_wait(bars + LB_PREADY, pg & 1u);
+          tc_fence_after();
+          const int s = (int)(pg % (uint32_t)g.stages);
+          const uint32_t sv = skv0 + (uint32_t)s * g.stage_bytes + NBOX * BOX;
+          const uint32_t tP = tmem_base + (pg & 1u) * 128u;
+#pragma unroll
+          for (int kk = 0; kk < 8; ++kk)
+            umma_ts(tO, tP + kk * 8, desc_mnmajor(sv + (uint32_t)kk * 2048u, BOX), id_pv, (j > 0 || kk != 0) ? 1u : 0u);
+          umma_commit(bars + LB_PVDONE);
+          umma_commit(bars + LB_KVEMPTY + 8 * s);                 // every MMA that reads this stage has retired when this arrives
+        }
+      }
+    }
+  } else if (warp >= 4) {
+    // ===================== softmax / output warps: TMEM lane quarter wq, one query row per thread =====================
+    const int wq = warp & 3;
+    const int row = wq * 32 + lane;
+    const uint32_t lane_off = (uint32_t)(wq * 32) << 16;
+    const uint32_t orow = tmem_base + lane_off + 256;
+    uint32_t gblk = 0;
+    for (int n = 0; n < my_items; ++n) {
+      int b, h, t;
+      item_coords(g, (int)blockIdx.x + n * (int)gridDim.x, b, h, t);
+      const int q = t * 128 + row;
+      float ref = -INFINITY, l = 0.f;                             // base-2 reference max, row sum against it
+      for (int j = 0; j <= t; ++j, ++gblk) {
+        const int st = (int)(gblk % (uint32_t)g.stages);
+        mbar_wait(bars + LB_MASK + 8 * st, (gblk / (uint32_t)g.stages) & 1u);
+        mbar_wait(bars + LB_SFULL + 8 * (gblk & 1u), (gblk >> 1) & 1u);
+        tc_fence_after();
+        const uint32_t srow = tmem_base + lane_off + (gblk & 1u) * 128u;
+        const bool diag = j == t;
+        // units past the causal bound of every row of this warp are not read (their P is stored as zeros)
+        const int nu = diag ? min(8, (wq * 32 + 31) / 16 + 1) : 8;
+        auto bits = [&](int u) {
+          const uint32_t key16 = (s_mask[st][u >> 1] >> ((u & 1) * 16)) & 0xFFFFu;
+          if (!diag) return key16;
+          const int n_ok = row - u * 16 + 1;
+          return key16 & (n_ok >= 16 ? 0xFFFFu : (n_ok <= 0 ? 0u : ((1u << n_ok) - 1u)));
+        };
+        float m = -INFINITY;
+        for (int u = 0; u < nu; ++u) {
+          uint32_t r[16];
+          tmem_ld16_issue(srow + u * 16, r);
+          tmem_ld_wait();
+          tmem_ld_fence(r);
+          const uint32_t vb = bits(u);
+#pragma unroll
+          for (int c = 0; c < 16; ++c) m = fmaxf(m, ((vb >> c) & 1u) ? __uint_as_float(r[c]) : -INFINITY);
+        }
+        const float mb = m == -INFINITY ? -INFINITY : m * g.sl2;
+        // raise the reference only when the block max clears it by RESCALE_LOG2; a row with no visible key so far has O = 0, l = 0
+        const bool raise = ref == -INFINITY ? mb != -INFINITY : mb > ref + RESCALE_LOG2;
+        const float corr = (raise && ref != -INFINITY) ? ex2(ref - mb) : 1.f;
+        if (raise) ref = mb;
+        l *= corr;
+        const float mref = ref == -INFINITY ? 0.f : ref;
+        for (int u = 0; u < nu; ++u) {
+          uint32_t r[16];
+          tmem_ld16_issue(srow + u * 16, r);
+          tmem_ld_wait();
+          tmem_ld_fence(r);                                       // the unit's scores are in registers: P may overwrite them
+          const uint32_t vb = bits(u);
+          uint32_t pk[8];
+#pragma unroll
+          for (int c = 0; c < 16; c += 2) {
+            const float p0 = ((vb >> c) & 1u) ? ex2(fmaf(__uint_as_float(r[c]), g.sl2, -mref)) : 0.f;
+            const float p1 = ((vb >> (c + 1)) & 1u) ? ex2(fmaf(__uint_as_float(r[c + 1]), g.sl2, -mref)) : 0.f;
+            l += p0 + p1;
+            pk[c >> 1] = pack2(p0, p1);
+          }
+          tmem_st8(srow + u * 8, pk);
+        }
+        {
+          const uint32_t z[8] = {0u, 0u, 0u, 0u, 0u, 0u, 0u, 0u};
+          for (int u = nu; u < 8; ++u) tmem_st8(srow + u * 8, z);
+        }
+        if (j > 0) {
+          mbar_wait(bars + LB_PVDONE, (gblk - 1) & 1u);           // O holds every earlier block of the item
+          tc_fence_after();
+          if (__any_sync(0xffffffffu, corr != 1.f)) {
+#pragma unroll
+            for (int c0 = 0; c0 < DH; c0 += 64) {
+              uint32_t r[4][16];
+#pragma unroll
+              for (int i = 0; i < 4; ++i) tmem_ld16_issue(orow + c0 + i * 16, r[i]);
+              tmem_ld_wait();
+#pragma unroll
+              for (int i = 0; i < 4; ++i) {
+                tmem_ld_fence(r[i]);
+#pragma unroll
+                for (int e = 0; e < 16; ++e) r[i][e] = __float_as_uint(__uint_as_float(r[i][e]) * corr);
+                tmem_st16(orow + c0 + i * 16, r[i]);
+              }
+            }
+          }
+        }
+        tmem_st_wait();
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(bars + LB_PREADY);
+      }
+      // ---- drain: O / l -> bf16 -> global, lse ----
+      mbar_wait(bars + LB_PVDONE, (gblk - 1) & 1u);
+      tc_fence_after();
+      const float inv = l > 0.f ? 1.f / l : 0.f;
+      __nv_bfloat16* op = g.out + (size_t)b * g.o_sb + (size_t)q * g.o_st + (size_t)h * DH;
+      const bool live = q < g.L;
+#pragma unroll
+      for (int c0 = 0; c0 < DH; c0 += 64) {
+        uint32_t r[4][16];
+#pragma unroll
+        for (int i = 0; i < 4; ++i) tmem_ld16_issue(orow + c0 + i * 16, r[i]);
+        tmem_ld_wait();
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+          tmem_ld_fence(r[i]);
+          uint32_t w[8];
+#pragma unroll
+          for (int e = 0; e < 8; ++e) w[e] = pack2(__uint_as_float(r[i][2 * e]) * inv, __uint_as_float(r[i][2 * e + 1]) * inv);
+          if (live) stg256(op + c0 + i * 16, w);
+        }
+      }
+      store_lse(g.lse, g.lse_sb, g.H, g.L, b, h, q, l, ref == -INFINITY ? 0.f : ref);
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(bars + LB_OFREE);
     }
   }
 
@@ -467,6 +803,40 @@ static int make_map(CUtensorMap* map, const void* base, long long rows, int cols
 
 }  // namespace tm
 
+// Key-blocked launch (L > 256).  Same operand conditions as the tile form; returns 1 when the shape is not covered.
+static int attention_tml_launch(const tcavp_attn_args& a, cudaStream_t stream) {
+  using namespace tm;
+  const int L = a.Tq;
+  GeoL g;
+  g.B = a.B; g.H = a.H; g.Hkv = a.Hkv; g.L = L; g.NT = (L + 127) / 128;
+  g.q_bytes = (uint32_t)(a.dh / BOXC) * 128u * 128u;
+  g.stage_bytes = 2u * g.q_bytes;
+  int stages = (int)((225u * 1024u - 2u * g.q_bytes - LB_BYTES - 1024u) / g.stage_bytes);
+  if (stages < 2) return 1;
+  g.stages = stages > L_MAX_STAGES ? L_MAX_STAGES : stages;
+  g.sl2 = a.scale * 1.4426950408889634f;
+  g.key_mask = a.key_mask;
+  g.out = reinterpret_cast<__nv_bfloat16*>(a.out); g.o_sb = a.o_sb; g.o_st = a.o_st;
+  g.lse = a.lse; g.lse_sb = a.lse_sb;
+  if ((long long)a.B * a.H * g.NT > 0x7fffffffLL || (long long)a.B * L > 0x7fffffffLL) return 1;
+  CUtensorMap mq, mk, mv;
+  const long long rows = (long long)a.B * L;
+  if (make_map(&mq, a.q, rows, a.H * a.dh, a.q_st, 128) || make_map(&mk, a.k, rows, a.Hkv * a.dh, a.k_st, 128) ||
+      make_map(&mv, a.v, rows, a.Hkv * a.dh, a.v_st, 128))
+    return 1;
+  const size_t smem = (size_t)2 * g.q_bytes + (size_t)g.stages * g.stage_bytes + LB_BYTES + 1024;   // > 118 KB: one CTA per SM
+  const int items = a.B * a.H * g.NT;
+  const int grid = items < sm_count() ? items : sm_count();
+  if (a.dh == 64) {
+    TCAVP_CUDA(cudaFuncSetAttribute(attn_tml_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    attn_tml_kernel<64><<<grid, L_THREADS, smem, stream>>>(mq, mk, mv, g);
+  } else {
+    TCAVP_CUDA(cudaFuncSetAttribute(attn_tml_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    attn_tml_kernel<128><<<grid, L_THREADS, smem, stream>>>(mq, mk, mv, g);
+  }
+  return check_launch("attn_tml_kernel");
+}
+
 // Returns 1 when the shape is not covered (caller falls back to the mma.sync flash kernel), <= 0 otherwise.
 int attention_tm_launch(const tcavp_attn_args& a, cudaStream_t stream) {
   using namespace tm;
@@ -477,7 +847,7 @@ int attention_tm_launch(const tcavp_attn_args& a, cudaStream_t stream) {
   }
   if (!enabled) return 1;
   if (a.dtype != TCAVP_BF16 || !a.causal || a.Tq != a.Tk || a.drop_thresh != 0) return 1;
-  if (!(a.dh == 64 || a.dh == 128) || a.Tq < 128 || a.Tq > 256 || a.B < 1) return 1;
+  if (!(a.dh == 64 || a.dh == 128) || a.Tq < 128 || a.B < 1) return 1;
   const int L = a.Tq, L16 = (L + 15) / 16 * 16, NB = L16 - 128;
   // rows of consecutive scenes must be contiguous (one 2-D tensor map per operand) and TMA-addressable
   if (a.q_sb != (long long)L * a.q_st || a.k_sb != (long long)L * a.k_st || a.v_sb != (long long)L * a.v_st) return 1;
@@ -485,6 +855,7 @@ int attention_tm_launch(const tcavp_attn_args& a, cudaStream_t stream) {
   if (!al16(a.q) || !al16(a.k) || !al16(a.v) || reinterpret_cast<uintptr_t>(a.out) % 32 || a.q_st % 8 || a.k_st % 8 || a.v_st % 8 || a.o_st % 16 ||
       a.o_sb % 16)
     return 1;
+  if (L > 256) return attention_tml_launch(a, stream);
   Geo g;
   g.B = a.B; g.H = a.H; g.Hkv = a.Hkv; g.L = L; g.L16 = L16; g.NB = NB;
   g.box_bytes = (uint32_t)L16 * 128u;
@@ -503,6 +874,7 @@ int attention_tm_launch(const tcavp_attn_args& a, cudaStream_t stream) {
   g.sl2 = a.scale * 1.4426950408889634f;
   g.key_mask = a.key_mask;
   g.out = reinterpret_cast<__nv_bfloat16*>(a.out); g.o_sb = a.o_sb; g.o_st = a.o_st;
+  g.lse = a.lse; g.lse_sb = a.lse_sb;
   CUtensorMap mq, mk, mv;
   const long long rows = (long long)a.B * L;
   if (make_map(&mq, a.q, rows, a.H * a.dh, a.q_st, L16) || make_map(&mk, a.k, rows, a.Hkv * a.dh, a.k_st, L16) ||

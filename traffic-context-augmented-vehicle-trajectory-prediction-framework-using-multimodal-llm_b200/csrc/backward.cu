@@ -1030,6 +1030,9 @@ int dw_tc_launch(const void* Y, int ldy, const void* X, int ldx, const float* sc
 int attention_bwd_tc_launch(const tcavp_attn_args& a, const void* dout, long long do_sb, long long do_st, void* dq, long long dq_sb,
                             long long dq_st, void* dk, long long dk_sb, long long dk_st, void* dv, long long dv_sb, long long dv_st,
                             int dkv_dtype, cudaStream_t stream);   // attention_bwd_tc.cu
+int attention_bwd_blk_launch(const tcavp_attn_args& a, const void* dout, long long do_sb, long long do_st, void* dq, long long dq_sb,
+                             long long dq_st, void* dk, long long dk_sb, long long dk_st, void* dv, long long dv_sb, long long dv_st,
+                             int dkv_dtype, cudaStream_t stream);  // attention_bwd_tc.cu (key-blocked, from the forward's logsumexp)
 
 // ------------------------------------------------------------------------------------------------
 // AdamW (torch.optim.AdamW semantics, reference scripts/im_kim_train_GRN.py:1008): decoupled weight decay,
@@ -1504,18 +1507,21 @@ extern "C" int tcavp_attention_bwd_owned(const tcavp_attn_args* a, const void* d
                                          long long dq_st, void* dk, long long dk_sb, long long dk_st, void* dv, long long dv_sb, long long dv_st,
                                          int dkv_dtype, tcavp_stream_t stream) {
   TCAVP_REQUIRE(a != nullptr, "tcavp_attention_bwd_owned: null args");
-  TCAVP_REQUIRE(a->B >= 0 && a->H > 0 && a->H == a->Hkv && a->Tq > 0 && a->Tk > 0, "tcavp_attention_bwd_owned: bad shape (needs H == Hkv)");
+  TCAVP_REQUIRE(a->B >= 0 && a->H > 0 && a->Hkv > 0 && a->H % a->Hkv == 0 && a->Tq > 0 && a->Tk > 0, "tcavp_attention_bwd_owned: bad shape");
   TCAVP_REQUIRE(!a->causal || a->Tq == a->Tk, "tcavp_attention_bwd_owned: causal needs Tq == Tk");
   if (a->B == 0) return TCAVP_OK;
   TCAVP_REQUIRE(a->q && a->k && a->v && dout && dq && dk && dv && DT_OK(dkv_dtype), "tcavp_attention_bwd_owned: bad pointer/dtype");
   TCAVP_REQUIRE(a->drop_thresh == 0 || (a->drop_seed != nullptr && a->drop_scale > 0.f), "tcavp_attention_bwd_owned: dropout needs a device seed and a scale");
-  int rc = 1;
-  if (a->out) rc = attention_bwd_tc_launch(*a, dout, do_sb, do_st, dq, dq_sb, dq_st, dk, dk_sb, dk_st, dv, dv_sb, dv_st, dkv_dtype, STREAM(stream));
-  if (rc > 0)   // few queries against wide heads (LTSF cross-attention): head_dim % 64 == 0, Tq <= 64, no causal mask
+  // longer than 256 positions or GQA, with the forward's logsumexp: key-blocked kernels (bf16, head_dim 64 / 128, no dropout)
+  int rc = attention_bwd_blk_launch(*a, dout, do_sb, do_st, dq, dq_sb, dq_st, dk, dk_sb, dk_st, dv, dv_sb, dv_st, dkv_dtype, STREAM(stream));
+  if (rc > 0 && a->out && a->H == a->Hkv)
+    rc = attention_bwd_tc_launch(*a, dout, do_sb, do_st, dq, dq_sb, dq_st, dk, dk_sb, dk_st, dv, dv_sb, dv_st, dkv_dtype, STREAM(stream));
+  if (rc > 0 && a->H == a->Hkv)   // few queries against wide heads (LTSF cross-attention): head_dim % 64 == 0, Tq <= 64, no causal mask
     rc = attention_x_bwd_launch(*a, dout, do_sb, do_st, dq, dq_sb, dq_st, dk, dk_sb, dk_st, dv, dv_sb, dv_st, dkv_dtype, STREAM(stream));
   if (rc > 0)
-    return fail_arg("tcavp_attention_bwd_owned: shape not covered (bf16 and either head_dim 16/32/64/96/128 with Tq, Tk <= 256 and the forward "
-                    "output in args->out, or head_dim %% 64 == 0 with Tq <= 64, Tk <= 256, not causal)");
+    return fail_arg("tcavp_attention_bwd_owned: shape not covered (bf16 and either head_dim 64/128 with the forward output in args->out and its "
+                    "logsumexp in args->lse, no dropout; or H == Hkv, head_dim 16/32/64/96/128 with Tq, Tk <= 256 and the forward output; or "
+                    "H == Hkv, head_dim %% 64 == 0 with Tq <= 64, Tk <= 256, not causal)");
   return rc;
 }
 

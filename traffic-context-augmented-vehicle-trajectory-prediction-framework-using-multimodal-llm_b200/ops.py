@@ -39,7 +39,8 @@ class AttnArgs(Structure):
                 ("v", c_void_p), ("v_sb", c_longlong), ("v_st", c_longlong),
                 ("out", c_void_p), ("o_sb", c_longlong), ("o_st", c_longlong),
                 ("dtype", c_int), ("scale", c_float), ("causal", c_int), ("key_mask", c_void_p),
-                ("drop_seed", c_void_p), ("drop_site", c_uint32), ("drop_thresh", c_uint32), ("drop_scale", c_float)]
+                ("drop_seed", c_void_p), ("drop_site", c_uint32), ("drop_thresh", c_uint32), ("drop_scale", c_float),
+                ("lse", c_void_p), ("lse_sb", c_longlong)]
 
 
 class Drop:
@@ -65,6 +66,13 @@ def drop_threshold(p):
 def _set_drop(a, drop):
     if drop is not None and drop.thresh:
         a.drop_seed, a.drop_site, a.drop_thresh, a.drop_scale = drop.seed.data_ptr(), drop.site, drop.thresh, drop.scale
+
+
+def _set_lse(a, lse, B, H, Tq):
+    if lse is not None:
+        if lse.dtype != torch.float32 or not lse.is_contiguous() or lse.numel() != B * H * Tq:
+            raise TypeError("lse must be a contiguous fp32 [B, H, Tq] tensor")
+        a.lse, a.lse_sb = lse.data_ptr(), H * Tq
 
 
 _PROF = None
@@ -290,9 +298,11 @@ def gemm(a, w, out, *, M=None, N=None, K=None, lda=None, ldw=None, ldo=None, bia
 
 
 def attention(q, k, v, out, *, B, H, Hkv, Tq, Tk, dh, q_strides, k_strides, v_strides, o_strides, scale, causal=False,
-              key_mask=None, drop=None):
-    """q/k/v/out are tensors whose data_ptr() is element (0,0,0,0); *_strides = (batch stride, time stride) in elements."""
-    _need_cuda(q, k, v, out, key_mask)
+              key_mask=None, drop=None, lse=None):
+    """q/k/v/out are tensors whose data_ptr() is element (0,0,0,0); *_strides = (batch stride, time stride) in elements.
+    lse: optional contiguous fp32 [B, H, Tq] output, the natural-log logsumexp of each row's scaled scores (-inf for a row with no
+    visible key); attention_bwd_owned recomputes the probabilities from it."""
+    _need_cuda(q, k, v, out, key_mask, lse)
     a = AttnArgs()
     a.B, a.H, a.Hkv, a.Tq, a.Tk, a.dh = B, H, Hkv, Tq, Tk, dh
     a.q, (a.q_sb, a.q_st) = q.data_ptr(), q_strides
@@ -305,12 +315,13 @@ def attention(q, k, v, out, *, B, H, Hkv, Tq, Tk, dh, q_strides, k_strides, v_st
             raise TypeError("attention: key_mask must be int32")
         a.key_mask = key_mask.data_ptr()
     _set_drop(a, drop)
+    _set_lse(a, lse, B, H, Tq)
     fl = 4.0 * B * H * Tq * Tk * dh * (0.5 if causal else 1.0)
 
     def label(kern):
         # algorithmic bytes: q read + out written + k and v read once (ONE pass when the keys are the values: attn_xt_kernel)
         nbytes = q.element_size() * B * dh * (2.0 * H * Tq + (1.0 if kern == "attn_xt_kernel" else 2.0) * Hkv * Tk)
-        if kern == "attn_tm_kernel":
+        if kern in ("attn_tm_kernel", "attn_tml_kernel"):
             return f"{kern}[dh{dh},L{Tq}]", nbytes
         return (kern if kern == "attn_x_kernel" else f"{kern}[dh{dh},q{Tq},k{Tk}]"), nbytes
 
@@ -771,8 +782,20 @@ def attention_bwd(q, k, v, dout, dq, dk, dv, *, B, H, Hkv, Tq, Tk, dh, q_strides
                                                    _ll(dv_strides[0]), _ll(dv_strides[1]), _stream()), "tcavp_attention_bwd")
 
 
-def attention_bwd_owned_ok(q, *, H, Hkv, Tq, Tk, dh, o, causal=False):
-    """True when tcavp_attention_bwd_owned (tensor-core kernel, dk / dv stored directly in the activation dtype) covers the shape."""
+def attention_lse_bwd_ok(q, *, H, Hkv, Tq, Tk, dh, drop=None):
+    """True when tcavp_attention_bwd_owned runs the key-blocked kernels for this shape once given the forward's logsumexp: bf16, head_dim
+    64 / 128, no dropout, and longer than 256 positions or GQA.  The train forwards ask ops.attention for `lse` exactly then."""
+    return (q.dtype == torch.bfloat16 and dh in (64, 128) and (drop is None or not drop.thresh) and H % Hkv == 0
+            and (max(Tq, Tk) > 256 or H != Hkv))
+
+
+def attention_bwd_owned_ok(q, *, H, Hkv, Tq, Tk, dh, o, causal=False, lse=None, drop=None, strides=()):
+    """True when tcavp_attention_bwd_owned (tensor-core kernel, dk / dv stored directly in the activation dtype) covers the shape.
+    The key-blocked kernels (lse given) also need 16-byte aligned q / o and, in `strides`, every q / k / v / dO / O batch and time stride
+    a multiple of 8 elements (as the packed activations of the engines are); the predicate checks the ones it is given."""
+    if (o is not None and lse is not None and attention_lse_bwd_ok(q, H=H, Hkv=Hkv, Tq=Tq, Tk=Tk, dh=dh, drop=drop)
+            and q.data_ptr() % 16 == 0 and o.data_ptr() % 16 == 0 and all(int(s) % 8 == 0 for s in strides)):
+        return True
     if q.dtype != torch.bfloat16 or H != Hkv:
         return False
     if o is not None and dh in (16, 32, 64, 96, 128) and max(Tq, Tk) <= 256:
@@ -781,13 +804,15 @@ def attention_bwd_owned_ok(q, *, H, Hkv, Tq, Tk, dh, o, causal=False):
 
 
 def attention_bwd_owned(q, k, v, dout, dq, dk, dv, *, B, H, Tq, Tk, dh, q_strides, k_strides, v_strides, do_strides, dq_strides,
-                        dk_strides, dv_strides, scale, causal=False, key_mask=None, o=None, o_strides=None, drop=None):
-    """dk / dv are written (not accumulated) in their own dtype, e.g. straight into the packed d(qkv) buffer."""
-    _need_cuda(q, k, v, dout, dq, dk, dv, key_mask, o)
+                        dk_strides, dv_strides, scale, causal=False, key_mask=None, o=None, o_strides=None, drop=None, Hkv=None, lse=None):
+    """dk / dv are written (not accumulated) in their own dtype, e.g. straight into the packed d(qkv) buffer.  lse: the forward's
+    logsumexp (ops.attention(lse=...)); with it, sequences past 256 positions and GQA (Hkv < H) run on the key-blocked kernels."""
+    _need_cuda(q, k, v, dout, dq, dk, dv, key_mask, o, lse)
     if dk.dtype != dv.dtype:
         raise TypeError("attention_bwd_owned: dk / dv dtypes differ")
+    Hkv = H if Hkv is None else Hkv
     a = AttnArgs()
-    a.B, a.H, a.Hkv, a.Tq, a.Tk, a.dh = B, H, H, Tq, Tk, dh
+    a.B, a.H, a.Hkv, a.Tq, a.Tk, a.dh = B, H, Hkv, Tq, Tk, dh
     a.q, (a.q_sb, a.q_st) = q.data_ptr(), q_strides
     a.k, (a.k_sb, a.k_st) = k.data_ptr(), k_strides
     a.v, (a.v_sb, a.v_st) = v.data_ptr(), v_strides
@@ -797,9 +822,14 @@ def attention_bwd_owned(q, k, v, dout, dq, dk, dv, *, B, H, Tq, Tk, dh, q_stride
     if key_mask is not None:
         a.key_mask = key_mask.data_ptr()
     _set_drop(a, drop)
+    _set_lse(a, lse, B, H, Tq)
     fl = 10.0 * B * H * Tq * Tk * dh * (0.5 if causal else 1.0)
-    small = o is not None and dh in (16, 32, 64, 96, 128) and max(Tq, Tk) <= 256
-    with _Timed(f"attn_{'bwd_tc' if small else 'x_bwd'}_kernel[dh{dh},q{Tq},k{Tk}]", fl, 0.0):
+
+    def label(kern):
+        # the key-blocked form is two launches (dK / dV, then dQ): one record under the pair's name
+        return f"{'attn_bwd_kv_q_kernels' if kern == 'attn_bwd_q_kernel' else kern}[dh{dh},q{Tq},k{Tk}]", 0.0
+
+    with _Timed(label if B > 0 else None, fl):
         _lib.check(_lib.load().tcavp_attention_bwd_owned(byref(a), _p(dout), _ll(do_strides[0]), _ll(do_strides[1]), _p(dq), _ll(dq_strides[0]),
                                                          _ll(dq_strides[1]), _p(dk), _ll(dk_strides[0]), _ll(dk_strides[1]), _p(dv),
                                                          _ll(dv_strides[0]), _ll(dv_strides[1]), dt(dk), _stream()), "tcavp_attention_bwd_owned")

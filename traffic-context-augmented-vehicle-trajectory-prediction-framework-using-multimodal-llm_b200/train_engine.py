@@ -338,15 +338,23 @@ class TrainEngine(Engine):
         return ops.layernorm_bwd(dy, x, ln[0], residual=residual, eps=ln[2], dx=dx, dw=dw, db=db)
 
     # ---- attention backward into packed gradient buffers ------------------------------------------------
+    def _attn_lse(self, act, B, H, Hkv, L, dh, drop=None):
+        """fp32 [B, H, L] logsumexp buffer for a causal self-attention forward whose backward recomputes the probabilities from it
+        (ops.attention_lse_bwd_ok: past 256 positions or GQA); None otherwise."""
+        if not ops.attention_lse_bwd_ok(act, H=H, Hkv=Hkv, Tq=L, Tk=L, dh=dh, drop=drop):
+            return None
+        return torch.empty(B * H * L, dtype=torch.float32, device=self.dev)
+
     def _attn_bwd(self, q, k, v, do, *, B, H, Hkv, Tq, Tk, dh, qs, ks, vs, dos, dq, dqs, dk_out, dv_out, ld_kv, scale, causal=False,
-                  key_mask=None, o=None, drop=None):
+                  key_mask=None, o=None, drop=None, lse=None):
         """dq is written in place (strides dqs); dk / dv are accumulated in fp32 and cast into dk_out / dv_out (row stride ld_kv)."""
-        if ops.attention_bwd_owned_ok(q, H=H, Hkv=Hkv, Tq=Tq, Tk=Tk, dh=dh, o=o, causal=causal):
-            # one CTA owns all key rows of a head: dk / dv land directly in the packed gradient buffer (no fp32 staging, no casts)
+        if ops.attention_bwd_owned_ok(q, H=H, Hkv=Hkv, Tq=Tq, Tk=Tk, dh=dh, o=o, causal=causal, lse=lse, drop=drop, strides=(*qs, *ks, *vs, *dos)):
+            # the CTAs that own a key block sum its gradient over every query (and GQA head): dk / dv land directly in the packed
+            # gradient buffer (no fp32 staging, no casts)
             kvs = (Tk * ld_kv, ld_kv)
             ops.attention_bwd_owned(q, k, v, do, dq, dk_out, dv_out, B=B, H=H, Tq=Tq, Tk=Tk, dh=dh, q_strides=qs, k_strides=ks, v_strides=vs,
                                     do_strides=dos, dq_strides=dqs, dk_strides=kvs, dv_strides=kvs, scale=scale, causal=causal,
-                                    key_mask=key_mask, o=o, o_strides=dos, drop=drop)
+                                    key_mask=key_mask, o=o, o_strides=dos, drop=drop, Hkv=Hkv, lse=lse)
             return
         wk = Hkv * dh
         dk = torch.zeros(B * Tk, wk, dtype=torch.float32, device=self.dev)
@@ -598,14 +606,15 @@ class TrainEngine(Engine):
                 xs = ops.layernorm(x, ly["ln1"][0], ly["ln1"][1], self._new(M, H), eps=ly["ln1"][2])
                 qkv = ops.gemm(xs, ly["wqkv"], self._new(M, 3 * H), bias=ly["bqkv"])
             attn = self._new(M, H)
+            lse = self._attn_lse(qkv, B, nh, nh, L, dh, self.drop("llm", li, "attn"))
             ops.attention(qkv, qkv[:, H:], qkv[:, 2 * H:], attn, B=B, H=nh, Hkv=nh, Tq=L, Tk=L, dh=dh, q_strides=sq, k_strides=sq, v_strides=sq,
-                          o_strides=(L * H, H), scale=dh ** -0.5, causal=True, key_mask=mask, drop=self.drop("llm", li, "attn"))
+                          o_strides=(L * H, H), scale=dh ** -0.5, causal=True, key_mask=mask, drop=self.drop("llm", li, "attn"), lse=lse)
             x_mid = self._sub_out(attn, ly["proj"], x, self.drop("llm", li, "resid1"))                  # x + resid_dropout(c_proj(a))
             h2 = ops.layernorm(x_mid, ly["ln2"][0], ly["ln2"][1], self._new(M, H), eps=ly["ln2"][2])
             pre = ops.gemm(h2, ly["fc"].w, self._new(M, I), bias=ly["fc"].b)
             mid = ops.gelu_tanh(pre, self._new(M, I), rows=M, cols=I)
             x_out = self._sub_out(mid, ly["mproj"], x_mid, self.drop("llm", li, "resid2"))              # x + dropout(mlp.c_proj(.))
-            ctxs.append((x, xs, qkv, attn, x_mid, pre))
+            ctxs.append((x, xs, qkv, attn, x_mid, pre, lse))
             x = x_out
         fh = ops.layernorm(x, m["norm"][0], m["norm"][1], self._new(M, H), eps=m["norm"][2])
         return fh, (ctxs, x, mask, None, B, L)
@@ -623,7 +632,7 @@ class TrainEngine(Engine):
         dx = lnb(dfh, x_last, m["norm"])
         xm = None
         for i in reversed(range(len(ctxs))):
-            x_in, xs, qkv, attn, x_mid, pre = ctxs[i]
+            x_in, xs, qkv, attn, x_mid, pre, lse = ctxs[i]
             ly = m["layers"][i]
             dmid = self._lin_bwd(self._drop_grad(dx, self.drop("llm", i, "resid2")), None, ly["mproj"], None, None, train=False)
             dpre = ops.gelu_tanh_bwd(dmid, pre, dmid, rows=M, cols=I)
@@ -633,7 +642,7 @@ class TrainEngine(Engine):
             dqkv = self._new(M, 3 * H)
             self._attn_bwd(qkv, qkv[:, H:], qkv[:, 2 * H:], dattn, B=B, H=nh, Hkv=nh, Tq=L, Tk=L, dh=dh, qs=sq, ks=sq, vs=sq, dos=(L * H, H),
                            dq=dqkv, dqs=sq, dk_out=dqkv[:, H:], dv_out=dqkv[:, 2 * H:], ld_kv=3 * H, scale=dh ** -0.5, causal=True, key_mask=mask,
-                           o=attn, drop=self.drop("llm", i, "attn"))
+                           o=attn, drop=self.drop("llm", i, "attn"), lse=lse)
             dh1 = ops.gemm(dqkv, ly["wqkvT"][:H], self._new(M, H))
             if kx:
                 du = ops.gemm(dqkv, ly["wqkvT"][H:], self._new(M, kx))               # gradient w.r.t. the LoRA side columns (dropout(h) A^T)
@@ -704,9 +713,10 @@ class TrainEngine(Engine):
                 ops.gemm(xs, ly["a_cat"], xs[:, H:], M=M, N=m["n_lora"], K=H, lda=Kx, ldo=Kx)
             qkv = ops.gemm(xs, ly["wqkv"], self._new(M, nqkv), M=M, N=nqkv, K=Kx, lda=Kx, rope=rope, row_scale=rstd1)
             attn = self._new(M, nq)
+            lse = self._attn_lse(qkv, B, nh, nkv, L, dh)
             ops.attention(qkv, qkv[:, nq:], qkv[:, nq + nk:], attn, B=B, H=nh, Hkv=nkv, Tq=L, Tk=L, dh=dh, q_strides=(L * nqkv, nqkv),
                           k_strides=(L * nqkv, nqkv), v_strides=(L * nqkv, nqkv), o_strides=(L * nq, nq), scale=dh ** -0.5, causal=True,
-                          key_mask=mask)
+                          key_mask=mask, lse=lse)
             xs2 = self._new_xs(M)
             ops.gemm(attn, ly["wo"], xs2, ldo=Kx, residual=xs, ldr=Kx)
             rstd2 = ops.row_rstd(xs2, torch.empty(M, dtype=torch.float32, device=self.dev), rows=M, cols=H, ldx=Kx, eps=m["eps"])
@@ -719,7 +729,7 @@ class TrainEngine(Engine):
                 mid = ops.swiglu(gu, self._new(M, I), rows=M, I=I)
             xs3 = self._new_xs(M)
             ops.gemm(mid, ly["wdown"], xs3, ldo=Kx, residual=xs2, ldr=Kx)
-            ctxs.append((xs, rstd1, qkv, attn, xs2, rstd2, gu, mid))
+            ctxs.append((xs, rstd1, qkv, attn, xs2, rstd2, gu, mid, lse))
             xs = xs3
         fh = ops.rmsnorm(xs, m["norm"], self._new(M, H), eps=m["eps"], rows=M, cols=H, ldi=Kx)
         return fh, (ctxs, xs, mask, table, B, L)
@@ -741,7 +751,7 @@ class TrainEngine(Engine):
             m["qk_inv_perm"] = torch.argsort(m["qk_perm"])
         inv_perm = m["qk_inv_perm"] if m["fuse_rope"] else None
         for i in reversed(range(len(ctxs))):
-            xs, rstd1, qkv, attn, xs2, rstd2, gu, mid = ctxs[i]
+            xs, rstd1, qkv, attn, xs2, rstd2, gu, mid, lse = ctxs[i]
             ly = m["layers"][i]
             if self.act == torch.bfloat16 and I % 32 == 0:
                 # d(mid) never leaves the tile: the down_proj^T GEMM's epilogue reads the stashed (gate, up) pairs and writes (d gate, d up)
@@ -755,7 +765,7 @@ class TrainEngine(Engine):
             dqkv = self._new(M, nqkv)
             self._attn_bwd(qkv, qkv[:, nq:], qkv[:, nq + nk:], dattn, B=B, H=nh, Hkv=nkv, Tq=L, Tk=L, dh=dh, qs=sq, ks=sq, vs=sq, dos=(L * nq, nq),
                            dq=dqkv, dqs=sq, dk_out=dqkv[:, nq:], dv_out=dqkv[:, nq + nk:], ld_kv=nqkv, scale=dh ** -0.5, causal=True, key_mask=mask,
-                           o=attn)
+                           o=attn, lse=lse)
             ops.rope_adjacent_(dqkv, rows=M, L=L, ld=nqkv, cols=nq + nk, dh=dh, table=table, inverse=True)
             dxs = ops.gemm(dqkv, ly["wqkvT"], self._new(M, Kx))            # [dn1 | dTn]
             drops = self._lora_drops(i)
